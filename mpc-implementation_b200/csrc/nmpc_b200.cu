@@ -330,7 +330,7 @@ int nmpc_create(const nmpc_spec* spec, int device, nmpc_handle** out) {
   h->ric_stride = RIC_N * h->pr.N;
   CKH(cudaMalloc(&h->d_ric, sizeof(double) * (size_t)h->ric_stride * h->max_blocks * h->warps_per_block));   // L2-resident Riccati scratch
   CKH(cudaMalloc(&h->d_cold, sizeof(double) * (size_t)h->cold_stride * h->max_blocks * h->warps_per_block));   // rare paths: restoration, watchdog
-  CKH(cudaMalloc(&h->d_ricmap, sizeof(unsigned) * 32 * 16));
+  CKH(cudaMalloc(&h->d_ricmap, sizeof(unsigned) * 32 * RIC_MAP_WORDS));
   {
     const int rc = h->inst->ricmap(h->d_ricmap, 0);
     if (rc != 0) { nmpc_destroy(h); return fail(std::string("nmpc_create: map kernel failed: ") + cudaGetErrorString((cudaError_t)rc)); }

@@ -69,7 +69,7 @@ constexpr int RIC_K2 = 81;    // 6 : kappa of the SOC right-hand side
 constexpr int RIC_N = 88;
 constexpr int FILT_CAP = 24;
 constexpr int ALG_N = 48;     // per-warp algorithm state kept in shared memory
-constexpr int STG_N = 356;    // Riccati staging area (nmpc_riccati.cuh)
+constexpr int STG_N = 282;    // Riccati staging area (nmpc_riccati.cuh)
 
 // scalar results returned by the phases through shared memory
 enum Res { R_F = 0, R_DU, R_PR, R_SUMY, R_SUMZ, R_VIOL, R_PMAX, R_PMIN, R_APR, R_ADU, R_GBD, R_THETA, R_TINY,

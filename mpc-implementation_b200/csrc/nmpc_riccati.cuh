@@ -24,12 +24,14 @@ extern __shared__ double smem_all[];
 
 // staging area layout (doubles, relative to Lay::STG0); every base is even (16-byte aligned)
 constexpr int SG_PP = 0;      // [9][9]  rows 0..7 = P+ (symmetric), row 8 = p+
-constexpr int SG_Z = 82;      // [3][16] the non-trivial rows 0..2 of Z = [B | A] (columns 0, 9, 10); the rest is 0 / T / identity
-constexpr int SG_Y = 130;     // [3][8]  Y_c = P+ z_c of the three special columns c = 0, 9, 10
-constexpr int SG_H = 154;     // [120]   packed lower triangle of the 15 x 15 stage matrix [H | h]
-constexpr int SG_W = 274;     // [9][6]  W = [Psi | psi]^T L^-T  (rows: 8 states + rhs)
-constexpr int SG_L = 328;     // [28]    L (21, packed lower) and the six 1/L[j][j]
-static_assert(SG_L + 28 <= STG_N, "staging area too small");
+constexpr int SG_Y = 82;      // [3][8]  Y_c = P+ z_c of the three special columns c = 0, 9, 10
+constexpr int SG_H = 106;     // [120]   packed lower triangle of the 15 x 15 stage matrix [H | h]
+constexpr int SG_W = 226;     // [9][6]  W = [Psi | psi]^T L^-T  (rows: 8 states + rhs)
+constexpr int SG_X = 280;     // [1]     where the lanes without a second trailing entry store theirs
+static_assert(SG_X + 1 <= STG_N, "staging area too small");
+// lane 0 owns two corrected entries of the stage matrix (e = 0 and e = 64); this lane computes the second one for it
+constexpr int RIC_CB_LANE = 24;
+static_assert(RIC_L % 2 == 0 && RIC_N % 2 == 0, "riccati_factor stores L with 16-byte stores");
 
 // state-Hessian entry Q_k[i][j] (+ delta_w part), used for the terminal stage only
 template <class L>
@@ -46,22 +48,26 @@ __device__ __forceinline__ double q_entry(int k, int i, int j, double dw) {
 // ---- per-lane ownership maps of the factorisation -------------------------------------------------------------
 // They depend on the lane and the layout only, so they are computed once per (N, n_obs) instantiation by
 // ric_map_kernel (at nmpc_create) into a global table of RIC_MAP_WORDS x 32 words, [word][lane], and loaded by
-// riccati_factor (15 coalesced L1-resident loads instead of ~800 instructions of index arithmetic per call).
+// riccati_factor (18 coalesced L1-resident loads instead of ~800 instructions of index arithmetic per call).
 // All entries are shared-memory indices relative to the warp's slice, packed two per word:
-//   w0..1 o0[4]   w2..3 o1[4]   w4..5 o2[4]   w6..7 ymain[4]   w8 cz|cy   w9 ch|th0   w10 th1|twa0   w11 twb0|twa1
-//   w12 twb1|tp0[0]   w13 tp1[0]|tp0[1]   w14 tp1[1]|codes,  codes = cmain code (2 bits: 0, 1, T, T^2) x 4 | c3 flag x 4 << 8
-constexpr int RIC_MAP_WORDS = 15;
+//   w0..1 o0[4]   w2..3 o1[4]   w4..5 o2[4]   w6..7 ymain[4]   w8 zy0|zy1   w9 zy2|zc0   w10 zc1|zc2   w11 cy|th0
+//   w12 th1|twa0   w13 twb0|twa1   w14 twb1|tp0[0]   w15 tp1[0]|tp0[1]   w16 tp1[1]|(unused)
+//   w17 codes = cmain code (2 bits: 0, 1, T, T^2) x 4 | c3 flag x 4 << 8 | correction A x 4 << 12 | correction B << 16
+constexpr int RIC_MAP_WORDS = 18;
 
 template <class L>
 __device__ void ric_map_build(int lane, unsigned* __restrict__ out /* [RIC_MAP_WORDS][32] */) {
   constexpr int S = L::S;
-  constexpr int PP = L::STG0 + SG_PP, ZS = L::STG0 + SG_Z, YS = L::STG0 + SG_Y, HS = L::STG0 + SG_H, WS = L::STG0 + SG_W;
+  constexpr int PP = L::STG0 + SG_PP, YS = L::STG0 + SG_Y, HS = L::STG0 + SG_H, WS = L::STG0 + SG_W;
   constexpr int LQ0 = L::LQ0;
   // Column c of Z = [B | A] is T e_{c+2} (c = 1..5) or e_{c-6} (c >= 6), plus stage-dependent entries in rows 0..2
   // for the "special" columns c = 0 (v: no unit part), 9 (theta), 10 (psi).
   auto spec = [](int c) { return c == 0 || c == 9 || c == 10; };
   auto sid = [](int c) { return c >= 6 ? c - 6 : c + 2; };                 // row of the unit entry (c >= 1)
   auto spj = [](int c) { return c == 0 ? 0 : c - 8; };                     // special column -> 0, 1, 2
+  // rows 0..2 of special column j, read at stage k from LQ0 + zoff + k: T * d (j = 0; riccati_factor applies the T),
+  // the first / last two entries of T E (j = 1 / 2), and 0 for Z[2][10]
+  auto zoff = [](int j, int s) { return LQ0 + S * (j == 0 ? LQ_DD + s : (j == 1 ? LQ_EE + s : (s < 2 ? LQ_EE + 3 + s : LQ_ZERO))); };
   auto row_of = [](int e) { int a = 0; while ((a + 1) * (a + 2) / 2 <= e) ++a; return a; };
   // ---- BUILDING the stage matrix: entry e = lane + 32 m of the packed lower triangle,
   //      ent = cmain * smem[ymain] + lq[o0] + mu * lq[o1] + dw * (lq[o2] + c3)
@@ -100,30 +106,40 @@ __device__ void ric_map_build(int lane, unsigned* __restrict__ out /* [RIC_MAP_W
     o0[m] = LQ0 + p0 * S; o1[m] = LQ0 + p1 * S; o2[m] = LQ0 + p2 * S;
     ymain[m] = ym; codes |= (unsigned)cm << (2 * m); codes |= (unsigned)cc << (8 + m);
   }
-  // ---- the nine entries whose z_a AND z_b (or p+) are special get  sum_s Z[s][za] * Yv[s]  on top (lanes 0..8)
-  int cz = ZS, cy = PP, ch = HS;
-  if (lane < 9) {
+  // ---- Y_j = P+ z_j, j = lane / 8 (stored by lanes 0..23)
+  const int yj = lane < 24 ? lane >> 3 : 0;
+  // ---- the nine entries whose z_a AND z_b (or p+) are special get  sum_s Z[s][za] * Yv[s]  on top, added by the lane
+  //      that builds the entry (bit m of correction A); lane 0 builds two of them and takes the second (e = 64, m = 2:
+  //      correction B) from lane RIC_CB_LANE, which builds none
+  int zc = 0, cy = PP;
+  for (int q = 0; q < 9; ++q) {
     const int ca_[9] = {0, 9, 10, 9, 10, 10, 14, 14, 14}, cb_[9] = {0, 0, 0, 9, 9, 10, 0, 9, 10};
-    const int a = ca_[lane], b = cb_[lane];
-    cz = ZS + (a == 14 ? b : a);
-    cy = a == 14 ? PP + 72 : YS + spj(b) * 8;
-    ch = HS + a * (a + 1) / 2 + b;
+    const int a = ca_[q], b = cb_[q], e = a * (a + 1) / 2 + b;
+    const bool second = e == 64;
+    if ((e & 31) == lane && !second) codes |= 1u << (12 + e / 32);
+    if (lane == 0 && second) codes |= 1u << 16;
+    if (second ? lane == RIC_CB_LANE : (e & 31) == lane) {
+      zc = spj(a == 14 ? b : a);
+      cy = a == 14 ? PP + 72 : YS + spj(b) * 8;
+    }
   }
-  // ---- TRAILING update: t = lane + 32 r over the packed lower triangle of the 9 x 9 block (0xffff: no entry)
+  // ---- TRAILING update: t = lane + 32 r over the packed lower triangle of the 9 x 9 block (t >= 44: no entry, the
+  //      lane computes H[6][6] - W_0 . W_0 again and stores it to SG_X)
   int th[2], twa[2], twb[2], tp0[2], tp1[2];
   for (int r = 0; r < 2; ++r) {
     const int t = lane + 32 * r;
     const int a = row_of(t), b = t - a * (a + 1) / 2;
     const bool valid = t < 44;                        // t == 44 is (rhs, rhs)
-    th[r] = valid ? HS + (a + 6) * (a + 7) / 2 + (b + 6) : 0xffff;
+    th[r] = HS + (valid ? (a + 6) * (a + 7) / 2 + (b + 6) : 27);
     twa[r] = WS + (valid ? a : 0) * 6; twb[r] = WS + (valid ? b : 0) * 6;
-    tp0[r] = !valid ? PP : (a == 8 ? PP + 72 + b : PP + a * 9 + b);
-    tp1[r] = !valid ? PP : (a == 8 ? PP + 72 + b : PP + b * 9 + a);
+    tp0[r] = !valid ? L::STG0 + SG_X : (a == 8 ? PP + 72 + b : PP + a * 9 + b);
+    tp1[r] = !valid ? L::STG0 + SG_X : (a == 8 ? PP + 72 + b : PP + b * 9 + a);
   }
   auto pk = [](int lo, int hi) { return (unsigned)lo | ((unsigned)hi << 16); };
   unsigned w[RIC_MAP_WORDS] = {pk(o0[0], o0[1]), pk(o0[2], o0[3]), pk(o1[0], o1[1]), pk(o1[2], o1[3]), pk(o2[0], o2[1]), pk(o2[2], o2[3]),
-                               pk(ymain[0], ymain[1]), pk(ymain[2], ymain[3]), pk(cz, cy), pk(ch, th[0]), pk(th[1], twa[0]),
-                               pk(twb[0], twa[1]), pk(twb[1], tp0[0]), pk(tp1[0], tp0[1]), pk(tp1[1], (int)codes)};
+                               pk(ymain[0], ymain[1]), pk(ymain[2], ymain[3]), pk(zoff(yj, 0), zoff(yj, 1)), pk(zoff(yj, 2), zoff(zc, 0)),
+                               pk(zoff(zc, 1), zoff(zc, 2)), pk(cy, th[0]), pk(th[1], twa[0]), pk(twb[0], twa[1]), pk(twb[1], tp0[0]),
+                               pk(tp1[0], tp0[1]), pk(tp1[1], 0), codes};
   for (int i = 0; i < RIC_MAP_WORDS; ++i) out[i * 32 + lane] = w[i];
 }
 template <class L>
@@ -132,7 +148,7 @@ __global__ void ric_map_kernel(unsigned* out) { ric_map_build<L>(threadIdx.x & 3
 template <class L>
 __device__ __noinline__ bool riccati_factor(double T, double* __restrict__ ric, const unsigned* __restrict__ map, double mu, double dw, int lane) {
   constexpr int S = L::S, N = L::N;
-  constexpr int PP = L::STG0 + SG_PP, ZS = L::STG0 + SG_Z, YS = L::STG0 + SG_Y, HS = L::STG0 + SG_H, WS = L::STG0 + SG_W, LS = L::STG0 + SG_L;
+  constexpr int PP = L::STG0 + SG_PP, YS = L::STG0 + SG_Y, HS = L::STG0 + SG_H, WS = L::STG0 + SG_W;
   constexpr int LQ0 = L::LQ0;
   unsigned w[RIC_MAP_WORDS];
 #pragma unroll
@@ -141,11 +157,12 @@ __device__ __noinline__ bool riccati_factor(double T, double* __restrict__ ric, 
   auto hi16 = [](unsigned v) { return (int)(v >> 16); };
   const int o0[4] = {lo16(w[0]), hi16(w[0]), lo16(w[1]), hi16(w[1])}, o1[4] = {lo16(w[2]), hi16(w[2]), lo16(w[3]), hi16(w[3])};
   const int o2[4] = {lo16(w[4]), hi16(w[4]), lo16(w[5]), hi16(w[5])}, ymain[4] = {lo16(w[6]), hi16(w[6]), lo16(w[7]), hi16(w[7])};
-  const int cz = lo16(w[8]), cy = hi16(w[8]), ch = lo16(w[9]);
-  const int th[2] = {hi16(w[9]) == 0xffff ? -1 : hi16(w[9]), lo16(w[10]) == 0xffff ? -1 : lo16(w[10])};
-  const int twa[2] = {hi16(w[10]), hi16(w[11])}, twb[2] = {lo16(w[11]), lo16(w[12])};
-  const int tp0[2] = {hi16(w[12]), hi16(w[13])}, tp1[2] = {lo16(w[13]), lo16(w[14])};
-  const unsigned codes = w[14] >> 16;
+  const int zy[3] = {lo16(w[8]), hi16(w[8]), lo16(w[9])}, zc[3] = {hi16(w[9]), lo16(w[10]), hi16(w[10])};
+  const int cy = lo16(w[11]);
+  const int th[2] = {hi16(w[11]), lo16(w[12])};
+  const int twa[2] = {hi16(w[12]), hi16(w[13])}, twb[2] = {lo16(w[13]), lo16(w[14])};
+  const int tp0[2] = {hi16(w[14]), hi16(w[15])}, tp1[2] = {lo16(w[15]), lo16(w[16])};
+  const unsigned codes = w[17];
   double c3[4], cmain[4];
 #pragma unroll
   for (int m = 0; m < 4; ++m) {
@@ -153,8 +170,12 @@ __device__ __noinline__ bool riccati_factor(double T, double* __restrict__ ric, 
     cmain[m] = cm == 0 ? 0.0 : (cm == 1 ? 1.0 : (cm == 2 ? T : T * T));
     c3[m] = ((codes >> (8 + m)) & 1u) ? 1.0 : 0.0;
   }
-#pragma unroll 1
-  for (int o = lane; o < 48; o += 32) smem[ZS + o] = 0.0;
+  // Z entries of column 0 are T * d; the others are read as they are (x 1.0 is exact)
+  const double fy = zy[0] == LQ0 + LQ_DD * S ? T : 1.0, fc = zc[0] == LQ0 + LQ_DD * S ? T : 1.0;
+  const int yi = lane & 7, yj = lane < 24 ? lane >> 3 : 0;
+  // lane c < 9 owns row c of W and column c of K; lanes 9..31 compute row 8 again and store the same values to the same
+  // addresses as lane 8, so that no store needs a branch
+  const int wc = lane < 9 ? lane : 8, wr = HS + (wc + 6) * (wc + 7) / 2;
   // ---- terminal stage: P_N = Q_N, p_N = q_N
 #pragma unroll 1
   for (int o = lane; o < 72; o += 32) {
@@ -164,78 +185,74 @@ __device__ __noinline__ bool riccati_factor(double T, double* __restrict__ ric, 
                                             : smem[LQ0 + (LQ_QA + j) * S + N] + mu * smem[LQ0 + (LQ_QB + j) * S + N] + dw * smem[LQ0 + (LQ_QD + j) * S + N]);
   }
   __syncwarp();
+  // Per stage: Y -> sync -> [H | h] -> sync -> Cholesky, W -> sync -> trailing update, K, L -> sync.  Every value is
+  // computed by the same operations in the same order as when Z, the nine corrections and L were staged through
+  // shared memory with a sync each; the intrinsics pin the contractions that staging used to force.
 #pragma unroll 1
   for (int k = N - 1; k >= 0; --k) {
-    // stage-dependent entries of Z
-    if (lane < 8) {
-      const int t = lane;
-      const int dst = t < 3 ? t * 16 : (t < 6 ? (t - 3) * 16 + 9 : (t - 6) * 16 + 10);   // [row 0..2][16 columns]
-      smem[ZS + dst] = t < 3 ? T * smem[LQ0 + (LQ_DD + t) * S + k] : smem[LQ0 + (LQ_EE + (t - 3)) * S + k];
-    }
-    __syncwarp();
+    double zyv[3], zcv[3];
+#pragma unroll
+    for (int s = 0; s < 3; ++s) { zyv[s] = __dmul_rn(fy, smem[zy[s] + k]); zcv[s] = __dmul_rn(fc, smem[zc[s] + k]); }
     // Y_c = P+ z_c for the special columns c = 0, 9, 10 (lanes 0..23)
-    if (lane < 24) {
-      const int j = lane >> 3, i = lane & 7, c = j == 0 ? 0 : 8 + j;
-      double acc = smem[ZS + c] * smem[PP + i * 9] + smem[ZS + 16 + c] * smem[PP + i * 9 + 1] + smem[ZS + 32 + c] * smem[PP + i * 9 + 2];
-      if (j > 0) acc += smem[PP + i * 9 + 2 + j];
-      smem[YS + lane] = acc;
+    {
+      double acc = __fma_rn(zyv[2], smem[PP + yi * 9 + 2], __fma_rn(zyv[0], smem[PP + yi * 9], __dmul_rn(zyv[1], smem[PP + yi * 9 + 1])));
+      if (yj > 0) acc = __dadd_rn(acc, smem[PP + yi * 9 + 2 + yj]);
+      if (lane < 24) smem[YS + lane] = acc;
     }
     __syncwarp();
-    // [H | h] -> staging
+    // [H | h] -> staging, with the corrections of the nine entries whose z_a and z_b (or p+) are both special
+    const double ca = __fma_rn(zcv[2], smem[cy + 2], __fma_rn(zcv[0], smem[cy], __dmul_rn(zcv[1], smem[cy + 1])));
+    const double cb = __shfl_sync(FULL, ca, RIC_CB_LANE);
 #pragma unroll
     for (int m = 0; m < 4; ++m) {
-      const double v = cmain[m] * smem[ymain[m]] + smem[o0[m] + k] + mu * smem[o1[m] + k] + dw * (smem[o2[m] + k] + c3[m]);
+      double v = cmain[m] * smem[ymain[m]] + smem[o0[m] + k] + mu * smem[o1[m] + k] + dw * (smem[o2[m] + k] + c3[m]);
+      if ((codes >> (12 + m)) & 1u) v = __dadd_rn(v, ca);
+      if (m == 2 && ((codes >> 16) & 1u)) v = __dadd_rn(v, cb);
       if (m < 3 || lane < 24) smem[HS + lane + 32 * m] = v;
     }
-    __syncwarp();
-    if (lane < 9) smem[ch] += smem[cz] * smem[cy] + smem[cz + 16] * smem[cy + 1] + smem[cz + 32] * smem[cy + 2];
     __syncwarp();
     // Cholesky of the 6 x 6 control block, redundantly in every lane's registers (uniform inertia verdict)
     double Lf[21], idg[6];
 #pragma unroll
     for (int e = 0; e < 21; ++e) Lf[e] = smem[HS + e];
     if (!chol6(Lf, idg)) return false;
-    if (lane == 0) {
+    // row wc of W = [Psi | psi]^T L^-T
+    double wv[6];
 #pragma unroll
-      for (int e = 0; e < 21; ++e) smem[LS + e] = Lf[e];
+    for (int j = 0; j < 6; ++j) {
+      double s_ = smem[wr + j];
 #pragma unroll
-      for (int e = 0; e < 6; ++e) smem[LS + 21 + e] = idg[e];
-    }
-    // lane c < 9: row c of W = [Psi | psi]^T L^-T, then column c of K = L^-T W^T
-    double* rk = ric + k * RIC_N;
-    if (lane < 9) {
-      double w[6];
-      const int row = HS + (lane + 6) * (lane + 7) / 2;
-#pragma unroll
-      for (int j = 0; j < 6; ++j) {
-        double s_ = smem[row + j];
-#pragma unroll
-        for (int m = 0; m < j; ++m) s_ -= w[m] * Lf[tri(j, m)];
-        w[j] = s_ * idg[j];
-        smem[WS + lane * 6 + j] = w[j];
-      }
-#pragma unroll
-      for (int i = 5; i >= 0; --i) {
-        double s_ = w[i];
-#pragma unroll
-        for (int m = i + 1; m < 6; ++m) s_ -= Lf[tri(m, i)] * w[m];
-        w[i] = s_ * idg[i];
-      }
-#pragma unroll
-      for (int r = 0; r < 6; ++r) rk[RIC_K + r * 9 + lane] = w[r];
+      for (int m = 0; m < j; ++m) s_ -= wv[m] * Lf[tri(j, m)];
+      wv[j] = s_ * idg[j];
+      smem[WS + wc * 6 + j] = wv[j];
     }
     __syncwarp();
-    if (lane < 27) rk[RIC_L + lane] = smem[LS + lane];   // L and 1/diag for the SOC re-solves
     // trailing block -> P_k, p_k for the next stage
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
-      if (th[r] >= 0) {
-        double acc = smem[th[r]];
+      double acc = smem[th[r]];
 #pragma unroll
-        for (int j = 0; j < 6; ++j) acc -= smem[twa[r] + j] * smem[twb[r] + j];
-        smem[tp0[r]] = acc; smem[tp1[r]] = acc;
-      }
+      for (int j = 0; j < 6; ++j) acc -= smem[twa[r] + j] * smem[twb[r] + j];
+      smem[tp0[r]] = acc; smem[tp1[r]] = acc;
     }
+    // column wc of K = L^-T W^T, and L with 1/diag for the SOC re-solves (every lane holds the same L and stores it):
+    // read only after the recursion, so they are computed here, next to the trailing update, and not at all for the
+    // stages of a failed factorisation
+    double* rk = ric + k * RIC_N;
+#pragma unroll
+    for (int i = 5; i >= 0; --i) {
+      double s_ = wv[i];
+#pragma unroll
+      for (int m = i + 1; m < 6; ++m) s_ -= Lf[tri(m, i)] * wv[m];
+      wv[i] = s_ * idg[i];
+    }
+#pragma unroll
+    for (int r = 0; r < 6; ++r) rk[RIC_K + r * 9 + wc] = wv[r];
+    double2* dl = reinterpret_cast<double2*>(rk + RIC_L);
+#pragma unroll
+    for (int e = 0; e < 10; ++e) dl[e] = make_double2(Lf[2 * e], Lf[2 * e + 1]);
+    dl[10] = make_double2(Lf[20], idg[0]); dl[11] = make_double2(idg[1], idg[2]); dl[12] = make_double2(idg[3], idg[4]);
+    rk[RIC_L + 26] = idg[5];
     __syncwarp();
   }
   return true;
