@@ -203,6 +203,7 @@ typedef struct nmpc_stats {
   int64_t watchdog_starts;
   int64_t soft_resto_steps;    /* steps accepted by the soft restoration phase's primal-dual error test */
   int64_t filter_resets;
+  int64_t trial_passes;        /* trial-point evaluations: ls_trials - trial_passes trials came from a paired pass's second point */
 } nmpc_stats;
 int nmpc_get_stats(nmpc_handle* h, nmpc_stats* out);   /* synchronises the handle's last stream */
 

@@ -37,7 +37,8 @@ class NmpcWarmOpts(C.Structure):
 class NmpcStats(C.Structure):
     _fields_ = [("kernel_launches", C.c_int64), ("factorizations", C.c_int64),
                 ("ls_trials", C.c_int64), ("soc_accepted", C.c_int64), ("resto_calls", C.c_int64), ("resto_iters", C.c_int64),
-                ("watchdog_starts", C.c_int64), ("soft_resto_steps", C.c_int64), ("filter_resets", C.c_int64)]
+                ("watchdog_starts", C.c_int64), ("soft_resto_steps", C.c_int64), ("filter_resets", C.c_int64),
+                ("trial_passes", C.c_int64)]
 
 
 EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_step",

@@ -265,7 +265,7 @@ struct nmpc_handle {
   cudaStream_t own_stream, last_stream;
   int64_t launches;
   double* dbg; int dbg_rows;
-  int align_group, align_mid, fill;
+  int align_group, align_mid, fill, pair_trials;
 };
 
 extern "C" {
@@ -323,6 +323,8 @@ int nmpc_create(const nmpc_spec* spec, int device, nmpc_handle** out) {
   h->align_mid = 1;           // point 1 (after the inertia-correction retries) on, point 2 (after the line search) off
   if (const char* e = getenv("NMPC_B200_ALIGN_MID")) h->align_mid = atoi(e) & 3;      // tuning knob: mid-iteration alignment points
   if (h->align_group == 0 || 3 * (h->warps_per_block / h->align_group) > 15) h->align_mid = 0;   // 16 named barriers per block
+  h->pair_trials = 1;         // N <= 15: a trial pass of the line search also evaluates the next trial point (bit-identical)
+  if (const char* e = getenv("NMPC_B200_PAIR_TRIALS")) h->pair_trials = atoi(e) != 0;      // tuning knob: 0 = one trial point per pass
   h->fill = spec->fill > 1 ? spec->fill : 1;
   if (const char* e = getenv("NMPC_B200_FILL")) { const int f = atoi(e); if (f >= 1) h->fill = f; }   // tuning override
   h->auto_order = 1;
@@ -410,7 +412,7 @@ int nmpc_solve(nmpc_handle* h, int32_t B, const double* p, const double* x0,
   A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && h->fuse_p) ? 1 : 0;
   A.run_steps = h->run_steps > 1 ? h->run_steps : 1; A.status_log = h->run_status_log; A.iters_log = h->run_iters_log; A.conv_count = h->run_conv;
   A.weights = h->weights;
-  A.align_group = h->align_group; A.align_mid = h->align_mid;
+  A.align_group = h->align_group; A.align_mid = h->align_mid; A.pair_trials = h->pair_trials;
   // fetch order: explicit (nmpc_set_order) > the order the previous call on this handle prepared for the same B > natural
   A.order = h->order_next; h->order_next = nullptr;
   if (!A.order && h->auto_order && h->have_order && h->prev_B == B) A.order = h->d_order[par];
@@ -646,7 +648,7 @@ int nmpc_get_stats(nmpc_handle* h, nmpc_stats* out) {
   CK(cudaMemcpy(st, h->stats_last ? h->stats_last : h->d_stats, sizeof st, cudaMemcpyDeviceToHost));
   out->kernel_launches = h->launches; out->factorizations = (int64_t)st[0]; out->ls_trials = (int64_t)st[1]; out->soc_accepted = (int64_t)st[2];
   out->resto_calls = (int64_t)st[3]; out->resto_iters = (int64_t)st[4]; out->watchdog_starts = (int64_t)st[5];
-  out->soft_resto_steps = (int64_t)st[6]; out->filter_resets = (int64_t)st[7];
+  out->soft_resto_steps = (int64_t)st[6]; out->filter_resets = (int64_t)st[7]; out->trial_passes = (int64_t)st[8];
   return 0;
 }
 

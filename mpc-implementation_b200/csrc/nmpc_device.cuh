@@ -68,7 +68,7 @@ constexpr int RIC_L = 54;     // 21: Cholesky factor of Lambda (packed lower) + 
 constexpr int RIC_K2 = 81;    // 6 : kappa of the SOC right-hand side
 constexpr int RIC_N = 88;
 constexpr int FILT_CAP = 24;
-constexpr int ALG_N = 48;     // per-warp algorithm state kept in shared memory
+constexpr int ALG_N = 50;     // per-warp algorithm state kept in shared memory
 constexpr int STG_N = 282;    // Riccati staging area (nmpc_riccati.cuh)
 
 // scalar results returned by the phases through shared memory
@@ -78,8 +78,10 @@ enum Res { R_F = 0, R_DU, R_PR, R_SUMY, R_SUMZ, R_VIOL, R_PMAX, R_PMIN, R_APR, R
            R_OTH, R_OINF,         // restoration mode: 1-norm / max-norm of the ORIGINAL problem's residual g - s
            R_DYMAX,               // max |dy| of the step (tiny-step logic)
            R_NFILT,               // filter length after an augmentation (written by lane 0)
+           R_FT2, R_THT2, R_LBT2, R_DTT2,     // R_FT .. R_DTT of the next backtracking trial point (paired ph_trial, lane SW)
            R_N };
-static_assert(R_N <= 24, "RES region is 24 doubles");
+constexpr int RES_N = 28;
+static_assert(R_N <= RES_N, "RES region is 28 doubles");
 
 __host__ __device__ inline int tri(int r, int c) { return r >= c ? r * (r + 1) / 2 + c : c * (c + 1) / 2 + r; }
 // state index of the five linear ("box") rows [z, theta, X5, X6, X7]   NMPC_TT.py:236-240
@@ -110,6 +112,16 @@ __device__ __forceinline__ double safe_value(double sl, double bnd) { return fma
 static __device__ __noinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
+  return v;
+}
+// warp_sum within each aligned group of W lanes.  When the lanes >= W hold +0.0, lane 0 gets bit for bit what warp_sum
+// gives it: the butterfly steps with offsets >= W then only add +0.0 to lane 0's partial sum, which changes nothing but
+// -0.0 -> +0.0, and the first add does exactly that.
+template <int W>
+static __device__ __noinline__ double seg_sum(double v) {
+  v = __dadd_rn(v, 0.0);
+#pragma unroll
+  for (int o = W / 2; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
   return v;
 }
 static __device__ __noinline__ double warp_max(double v) {
@@ -176,6 +188,7 @@ struct LayT {
   static constexpr int MODEL = MODEL_, NB = model_nb(MODEL_), NUA = model_nu(MODEL_), NPA = model_np(MODEL_);
   static constexpr int N = N_, S = N_ + 1, R = NB + NOBS_, NOBS = NOBS_;
   static constexpr int SW = S <= 8 ? 8 : (S <= 16 ? 16 : 32);      // width of the warp scans over the stages
+  static constexpr bool PAIR = 2 * SW <= 32;                        // a second trial point fits lanes SW .. 2 SW - 1 (ph_trial)
   static constexpr bool FOLD = FOLD_;
   static constexpr int LQ_NE = FOLD_ ? LQ_NFOLD : LQ_N;
   static constexpr int LV0 = 0;
@@ -195,7 +208,7 @@ struct LayT {
   static constexpr int OBS0 = STG0 + STG_N;
   static constexpr int ALG0 = even_up(OBS0 + 3 * NOBS_ + 1);     // algorithm state (nmpc_solve.cuh: AlgF), ALG_N doubles
   static constexpr int RES0 = ALG0 + ALG_N;
-  static constexpr int PAR0 = RES0 + 24;
+  static constexpr int PAR0 = RES0 + RES_N;
   static constexpr int TOTAL = even_up(PAR0 + 14);   // p (11), w1, w2 of this instance
   // warps (= concurrent instances) per block: as many slices as fit in the 227 KB a block may use, at most NMPC_WPB_MAX
   // ---- cold per-warp scratch in global memory (touched only by the watchdog, the soft restoration phase and the

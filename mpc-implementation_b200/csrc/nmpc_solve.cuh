@@ -77,16 +77,17 @@ struct SolveArgs {
   int *counter_next, *done, *done_next;
   unsigned long long* stats_next;
   int32_t* order_out;                // may be NULL (no automatic ordering)
-  unsigned long long* stats;         // [8]: factorizations, ls trials, soc accepted, restoration calls, restoration iterations,
-                                     //      watchdog starts, soft restoration steps, filter resets
+  unsigned long long* stats;         // [9]: factorizations, ls trials, soc accepted, restoration calls, restoration iterations,
+                                     //      watchdog starts, soft restoration steps, filter resets, trial passes
   double* ric; int ric_stride;       // L2-resident Riccati scratch, one slice per resident warp
   double* cold; int cold_stride;     // per-warp scratch of the rare paths (Lay::COLD_TOTAL)
   const unsigned* ricmap;            // per-lane ownership maps of the factorisation (nmpc_riccati.cuh: ric_map_build)
   double* dbg; int dbg_rows;         // optional per-iteration log [B][dbg_rows][10] (tests only)
   int align_group;                   // warps that start each IPM iteration together (0 = no alignment, else divides WPB)
   int align_mid;                     // bit mask of the mid-iteration alignment points in use (0 = iteration start only)
+  int pair_trials;                   // layouts with Lay::PAIR: each backtracking trial pass also evaluates the next trial point
 };
-constexpr int NSTAT = 8;
+constexpr int NSTAT = 9;
 constexpr int DBG_COLS = 10;
 
 constexpr double EPSM = 2.220446049250313e-16;
@@ -706,10 +707,18 @@ __device__ __noinline__ void ph_dir(const SolveArgs& A, int lane, double mu, dou
   __syncwarp();
 }
 
-// trial point u + alpha*du, s + alpha*ds (n, p for RS): objective, constraint violation, barrier pieces; residual into CT
+// trial point u + alpha*du, s + alpha*ds (n, p for RS): objective, constraint violation, barrier pieces; residual into CT.
+// pair (Lay::PAIR layouts only): lanes SW .. 2 SW - 1 evaluate the point at alpha * alpha_red -- the trial that follows a
+// plain rejection -- in the same instructions, stage k on lane SW + k, into R_FT2 .. R_DTT2.  The lower half computes
+// exactly what it computes without pairing; the upper half does not store CT (only ph_socrhs reads it, after the trial at
+// alpha_max, which is never a precomputed one).
 template <class L, bool RS>
-__device__ __noinline__ void ph_trial(const SolveArgs& A, int lane, double alpha, bool soc, double df, double mu, double* cold) {
+__device__ __noinline__ void ph_trial(const SolveArgs& A, int lane_, double alpha_, bool soc, double df, double mu, double* cold, bool pair) {
   const Prob& pr = A.pr;
+  pair = L::PAIR && pair;
+  const bool hi = pair && lane_ >= L::SW;
+  const int lane = pair ? lane_ & (L::SW - 1) : lane_;      // stage index: every lane-indexed access below uses it
+  const double alpha = hi ? alpha_ * A.o.alpha_red : alpha_;
   const bool act = lane <= L::N, hasu = lane < L::N;
   double ut[6], lb = 0.0, dt = 0.0, fr = 0.0;
   double prod = 1.0; int cnt = 0;
@@ -745,7 +754,8 @@ __device__ __noinline__ void ph_trial(const SolveArgs& A, int lane, double alpha
         const double ns = (nt), ps = (pt);
         prod *= ns * ps; cnt += 2; dt += ns + ps; l += A.o.resto_rho * (nt + pt);
       }
-      RG(G_CT, r) = ct; th += fabs(ct);      // (only the second-order correction reads it back)
+      if (!hi) RG(G_CT, r) = ct;      // (only the second-order correction reads it back)
+      th += fabs(ct);
       const Bnd b = row_bounds<L>(A, lane, r, dc);
       if (b.hl) { prod *= (sv - b.lo); ++cnt; }
       if (b.hu) { prod *= (b.hi - sv); ++cnt; }
@@ -756,9 +766,12 @@ __device__ __noinline__ void ph_trial(const SolveArgs& A, int lane, double alpha
     FOR_ROWS(st.X, body);
     if (cnt) lb += n_log(prod);
   }
-  const double fs = (RS ? 1.0 : df) * warp_sum(l);
-  th = warp_sum(th); lb = warp_sum(lb); dt = warp_sum(dt);
-  if (lane == 0) { RES(R_FT) = fs; RES(R_THT) = th; RES(R_LBT) = lb; RES(R_DTT) = dt; }
+  // per half-warp sums where pairing is possible (the lanes >= SW hold zeros when unpaired: lane 0's sums are warp_sum's)
+  auto sum = [](double v) { if constexpr (L::PAIR) return seg_sum<L::SW>(v); else return warp_sum(v); };
+  const double fs = (RS ? 1.0 : df) * sum(l);
+  th = sum(th); lb = sum(lb); dt = sum(dt);
+  if (lane_ == 0) { RES(R_FT) = fs; RES(R_THT) = th; RES(R_LBT) = lb; RES(R_DTT) = dt; }
+  if (pair && lane_ == L::SW) { RES(R_FT2) = fs; RES(R_THT2) = th; RES(R_LBT2) = lb; RES(R_DTT2) = dt; }
   __syncwarp();
 }
 
@@ -1127,7 +1140,7 @@ enum AlgF {
   F_NALG,
   F_MODE = F_NALG,                                  // 0 original problem, 1 restoration problem
   F_DW, F_APR, F_ADU, F_GBD, F_THETA, F_PHI,        // this iteration: delta_w, step limits, barrier slope, theta, barrier of the current point
-  F_C0,                                             // 8 work counters
+  F_C0,                                             // NSTAT work counters
   F_END = F_C0 + NSTAT
 };
 static_assert(F_END <= ALG_N, "algorithm state does not fit its shared-memory region");
@@ -1157,9 +1170,19 @@ template <class L>
 __device__ __forceinline__ void do_dir(const SolveArgs& A, int lane, int mode, bool soc, double dw, double* cold) {
   if (mode) ph_dir<L, true>(A, lane, AL(F_MU), AL(F_TAU), soc, dw, cold); else ph_dir<L, false>(A, lane, AL(F_MU), AL(F_TAU), soc, dw, cold);
 }
+// one trial pass (counted as a line-search trial and as a pass); pair: see ph_trial
 template <class L>
-__device__ __forceinline__ void do_trial(const SolveArgs& A, int lane, int mode, double alpha, bool soc, double df, double* cold) {
-  if (mode) ph_trial<L, true>(A, lane, alpha, soc, df, AL(F_MU), cold); else ph_trial<L, false>(A, lane, alpha, soc, df, AL(F_MU), cold);
+__device__ __forceinline__ void do_trial(const SolveArgs& A, int lane, int mode, double alpha, bool soc, double df, double* cold, bool pair = false) {
+  if (mode) ph_trial<L, true>(A, lane, alpha, soc, df, AL(F_MU), cold, pair); else ph_trial<L, false>(A, lane, alpha, soc, df, AL(F_MU), cold, pair);
+  al_count<L>(1, lane); al_count<L>(8, lane);
+}
+// the trial point the last paired pass evaluated ahead becomes the last trial point (a line-search trial without a pass)
+template <class L>
+__device__ __forceinline__ void take_ahead(int lane) {
+  const double ft = RES(R_FT2), tht = RES(R_THT2), lbt = RES(R_LBT2), dtt = RES(R_DTT2);
+  __syncwarp();
+  RES(R_FT) = ft; RES(R_THT) = tht; RES(R_LBT) = lbt; RES(R_DTT) = dtt;     // every lane stores the same values
+  __syncwarp();
   al_count<L>(1, lane);
 }
 template <class L>
@@ -1321,7 +1344,7 @@ __device__ __noinline__ void resto_enter(const SolveArgs& A, double* cold, int l
   alg_init<L>(mu_r, o.tau_min, o.tol);
   ph_resto_init<L>(A, lane, mu_r, cold);
   AL(F_MODE) = 1.0;
-  ph_trial<L, true>(A, lane, 0.0, false, df, mu_r, cold);
+  ph_trial<L, true>(A, lane, 0.0, false, df, mu_r, cold, false);
   take_trial_values<L>();
   __syncwarp();
 }
@@ -1338,7 +1361,7 @@ __device__ __noinline__ int resto_check(const SolveArgs& A, double* cold, int la
   if (o.kappa_resto == 0.0) infpr_max = 0.0;
   if (AL(F_FIRST) == 0.0 && !(oinf > infpr_max)) {
     const double omu = park[F_MU];
-    ph_trial<L, false>(A, lane, 0.0, false, df, omu, cold);       // original objective and barrier terms at the restoration iterate
+    ph_trial<L, false>(A, lane, 0.0, false, df, omu, cold, false);       // original objective and barrier terms at the restoration iterate
     const double tb = RES(R_FT) - omu * RES(R_LBT) + o.kappa_d * omu * RES(R_DTT);
     if (filter_ok(filter_of<L>(cold, 0), (int)park[F_NFILT], tb, oth) && ok_to_current(o, park[F_RBARR], park[F_RTH], tb, oth, true)) st = -2;
   }
@@ -1368,7 +1391,7 @@ __device__ __noinline__ void resto_leave(const SolveArgs& A, double* cold, int l
   const double zmax = ph_resto_finish<L>(A, lane, mu, tau, adu, 1, cold, 1);
   if (zmax > o.bound_mult_reset_threshold) ph_unit_mults<L>(A, lane);
   ph_accept<L, false>(A, lane, 0.0, 0.0, mu, 0.0, false, true, cold);      // kappa_Sigma reset (AcceptTrialPoint)
-  ph_trial<L, false>(A, lane, 0.0, false, df, mu, cold);
+  ph_trial<L, false>(A, lane, 0.0, false, df, mu, cold, false);
   take_trial_values<L>();
   AL(F_INSOFT) = 0.0; AL(F_SOFTC) = 0.0; AL(F_WSHORT) = 0.0;
   __syncwarp();
@@ -1417,7 +1440,7 @@ __device__ __noinline__ bool update_mu(const SolveArgs& A, double* cold, int lan
       const double sumy = RES(R_SUMY), sumz = RES(R_SUMZ);
       sd = fmax(o.s_max, (sumy + sumz) / (double)max(1, mtot + nz)) / o.s_max;
       sc = fmax(o.s_max, sumz / (double)max(1, nz)) / o.s_max;
-      ph_trial<L, true>(A, lane, 0.0, false, df, mu, cold);
+      ph_trial<L, true>(A, lane, 0.0, false, df, mu, cold, false);
       take_trial_values<L>();
     }
     if (tf) { done = true; tf = false; }
@@ -1434,6 +1457,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
   constexpr int DX0 = L::LV0 + LV_DX * S, DU0 = L::LV0 + LV_DU * S, DUS0 = L::soc(SOC_DUS), Q20 = L::soc(SOC_Q2);
   constexpr int mtot = R * S;
   const double T = pr.T;
+  const bool pair = L::PAIR && A.pair_trials;
 
   ph_load<L>(A, b, lane);
   double df = 1.0;
@@ -1454,7 +1478,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
   alg_init<L>(mu0, o.tau_min, o.tol);
   for (int f = F_NALG + lane; f < F_END; f += 32) AL(f) = 0.0;
   __syncwarp();
-  ph_trial<L, false>(A, lane, 0.0, false, df, mu0, cold);      // barrier pieces and constraint violation of the start
+  ph_trial<L, false>(A, lane, 0.0, false, df, mu0, cold, false);      // barrier pieces and constraint violation of the start
   take_trial_values<L>();
   const double mu_floor = fmin(o.tol, df * o.compl_inf_tol) / (o.kappa_eps + 1.0);
   int iter = 0, status = NMPC_MAXITER_EXCEEDED;
@@ -1584,8 +1608,13 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
           alpha = a_max; a_du = AL(F_ADU);
           double a_test = in_wd ? AL(F_WAT) : alpha;
           if (skip_first) alpha *= o.alpha_red;
+          // alpha of the trial point the last paired pass evaluated ahead (< 0: none).  Between two trials of this loop
+          // nothing moves the iterate, the direction, mu or the mode (a second-order correction has arrays of its own),
+          // so that result is the one a pass at this alpha would give.
+          double ahead = -1.0;
           while (alpha > amin || n_steps == 0) {
-            do_trial<L>(A, lane, mode, alpha, false, df, cold);
+            if (pair && alpha == ahead) { take_ahead<L>(lane); ahead = -1.0; }
+            else { do_trial<L>(A, lane, mode, alpha, false, df, cold, pair); if (pair) ahead = alpha * o.alpha_red; }
             th_t = RES(R_THT); phi_t = trial_barrier<L>(A);
             const bool okv = isfinite(th_t) && isfinite(phi_t);
             if (!in_wd) a_test = alpha;
