@@ -265,7 +265,7 @@ struct nmpc_handle {
   cudaStream_t own_stream, last_stream;
   int64_t launches;
   double* dbg; int dbg_rows;
-  int align_group, align_mid, fill, pair_trials;
+  int fill, pair_trials;
 };
 
 extern "C" {
@@ -315,18 +315,9 @@ int nmpc_create(const nmpc_spec* spec, int device, nmpc_handle** out) {
   }
   if (h->blocks_per_sm < 1) { delete h; return fail("nmpc_create: kernel does not fit on an SM"); }
   h->max_blocks = h->sm_count * h->blocks_per_sm;
-  h->align_group = h->warps_per_block;
-  if (const char* e = getenv("NMPC_B200_ALIGN_GROUP")) {     // tuning knob: 0 = off, else a divisor of the warps per block
-    const int g = atoi(e);
-    if (g == 0 || (g > 0 && h->warps_per_block % g == 0)) h->align_group = g;
-  }
-  h->align_mid = 1;           // point 1 (after the inertia-correction retries) on, point 2 (after the line search) off
-  if (const char* e = getenv("NMPC_B200_ALIGN_MID")) h->align_mid = atoi(e) & 3;      // tuning knob: mid-iteration alignment points
-  if (h->align_group == 0 || 3 * (h->warps_per_block / h->align_group) > 15) h->align_mid = 0;   // 16 named barriers per block
   h->pair_trials = 1;         // N <= 15: a trial pass of the line search also evaluates the next trial point (bit-identical)
   if (const char* e = getenv("NMPC_B200_PAIR_TRIALS")) h->pair_trials = atoi(e) != 0;      // tuning knob: 0 = one trial point per pass
   h->fill = spec->fill > 1 ? spec->fill : 1;
-  if (const char* e = getenv("NMPC_B200_FILL")) { const int f = atoi(e); if (f >= 1) h->fill = f; }   // tuning override
   h->auto_order = 1;
   if (const char* e = getenv("NMPC_B200_AUTO_ORDER")) h->auto_order = atoi(e) != 0;
   h->ric_stride = RIC_N * h->pr.N;
@@ -412,7 +403,7 @@ int nmpc_solve(nmpc_handle* h, int32_t B, const double* p, const double* x0,
   A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && h->fuse_p) ? 1 : 0;
   A.run_steps = h->run_steps > 1 ? h->run_steps : 1; A.status_log = h->run_status_log; A.iters_log = h->run_iters_log; A.conv_count = h->run_conv;
   A.weights = h->weights;
-  A.align_group = h->align_group; A.align_mid = h->align_mid; A.pair_trials = h->pair_trials;
+  A.pair_trials = h->pair_trials;
   // fetch order: explicit (nmpc_set_order) > the order the previous call on this handle prepared for the same B > natural
   A.order = h->order_next; h->order_next = nullptr;
   if (!A.order && h->auto_order && h->have_order && h->prev_B == B) A.order = h->d_order[par];

@@ -37,7 +37,6 @@ struct Opt {
   double obj_max_inc = 5.0; int max_filter_resets = 5, filter_reset_trigger = 5;
   int watchdog_trigger = 10, watchdog_trial_max = 3;
   int max_soft_resto = 10; double soft_resto_red = 1.0 - 1e-4;
-  int resto = 1;                       // 0: a failed line search ends the solve with NMPC_RESTORATION_FAILED (round-1 behaviour)
   double resto_rho = 1000.0, resto_eta_factor = 1.0, kappa_resto = 0.9;
   double bound_mult_reset_threshold = 1e3;
   double resto_theta_max_fact = 1e8;
@@ -83,8 +82,6 @@ struct SolveArgs {
   double* cold; int cold_stride;     // per-warp scratch of the rare paths (Lay::COLD_TOTAL)
   const unsigned* ricmap;            // per-lane ownership maps of the factorisation (nmpc_riccati.cuh: ric_map_build)
   double* dbg; int dbg_rows;         // optional per-iteration log [B][dbg_rows][10] (tests only)
-  int align_group;                   // warps that start each IPM iteration together (0 = no alignment, else divides WPB)
-  int align_mid;                     // bit mask of the mid-iteration alignment points in use (0 = iteration start only)
   int pair_trials;                   // layouts with Lay::PAIR: each backtracking trial pass also evaluates the next trial point
 };
 constexpr int NSTAT = 9;
@@ -129,39 +126,30 @@ __device__ __forceinline__ Bnd row_bounds(const SolveArgs& A, int k, int r, doub
   return b;
 }
 
-// Alignment barrier over the group of `g` consecutive warps this warp belongs to (named barrier 1 + group index),
-// OR-reducing `working` over the group.  Every warp of the group calls it the same number of times: working warps
-// once per IPM iteration, warps that ran out of work in a loop until the reduction says nobody is working -- the
-// exit decision comes out of the barrier itself, so no warp can leave while another still waits.  g == 0: no alignment.
-__device__ __forceinline__ int align_warps(int g, int working) {
-  if (g == 0) return 0;
+// Warp alignment (DESIGN.md section 2): all Lay::WPB warps of a block meet at named barrier 1 at the start of every
+// IPM iteration, and once more at named barrier 2 after the inertia-correction retries.  Both barriers count every
+// thread of the block; barrier 0 is __syncthreads'.
+//
+// Alignment barrier (named barrier 1), OR-reducing `working` over the block.  Every warp calls it the same number of
+// times: working warps once per IPM iteration, warps that ran out of work in a loop until the reduction says nobody is
+// working -- the exit decision comes out of the barrier itself, so no warp can leave while another still waits.
+template <class L>
+__device__ __forceinline__ int align_warps(int working) {
   unsigned out;
-  const unsigned id = 1 + (threadIdx.x >> 5) / g, nt = 32 * g;
-  asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.or.pred q, %2, %3, p;\n\tselp.u32 %0, 1, 0, q;\n\t}"
-               : "=r"(out) : "r"((unsigned)working), "r"(id), "r"(nt) : "memory");
+  asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.or.pred q, 1, %2, p;\n\tselp.u32 %0, 1, 0, q;\n\t}"
+               : "=r"(out) : "r"((unsigned)working), "n"(32 * L::WPB) : "memory");
   return (int)out;
 }
 
-// Mid-iteration alignment points (named barriers 1 + point * groups + group): between two calls of align_warps every
-// warp of the group passes each point in use exactly once, either waiting at it (mid_sync) or -- on a path that skips
-// it -- by announcing itself without waiting (mid_arrive), so nobody waits for a warp that will not come.
-__device__ __forceinline__ void mid_bar(int g, int groups, int point, bool wait) {
-  const unsigned id = 1 + point * groups + (threadIdx.x >> 5) / g, nt = 32 * g;
-  if (wait) asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(nt) : "memory");
-  else asm volatile("bar.arrive %0, %1;" :: "r"(id), "r"(nt) : "memory");
-}
+// Retry point (named barrier 2).  Between two calls of align_warps every warp passes it exactly once: it waits there
+// after the inertia-correction retries (retry_sync), and every path that skips that place -- an exit from the
+// iteration loop, a `continue`, the least-squares multiplier start, a warp out of work -- arrives without waiting
+// (retry_arrive).  A warp that did neither would leave the others waiting at bar.sync for ever; one that passed twice
+// would complete a round that another warp has not reached.
 template <class L>
-__device__ __forceinline__ void mid_sync(const SolveArgs& A, int point, int& done) {
-  if (A.align_mid >> (point - 1) & 1) { mid_bar(A.align_group, L::WPB / A.align_group, point, true); done |= 1 << (point - 1); }
-}
+__device__ __forceinline__ void retry_sync() { asm volatile("bar.sync 2, %0;" :: "n"(32 * L::WPB) : "memory"); }
 template <class L>
-__device__ __forceinline__ void mid_flush(const SolveArgs& A, int& done) {     // announce at the points this round did not pass; done < 0: no round open
-  if (done < 0) return;
-#pragma unroll
-  for (int pt = 1; pt <= 2; ++pt)
-    if ((A.align_mid >> (pt - 1) & 1) && !(done >> (pt - 1) & 1)) mid_bar(A.align_group, L::WPB / A.align_group, pt, false);
-  done = -1;
-}
+__device__ __forceinline__ void retry_arrive() { asm volatile("bar.arrive 2, %0;" :: "n"(32 * L::WPB) : "memory"); }
 
 #define LV(e) smem[L::LV0 + (e) * L::S + lane]
 #define RW(arr, r) smem[L::rw(arr, r) + lane]
@@ -1483,10 +1471,9 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
   const double mu_floor = fmin(o.tol, df * o.compl_inf_tol) / (o.kappa_eps + 1.0);
   int iter = 0, status = NMPC_MAXITER_EXCEEDED;
 
-  int mids = -1;
+  bool retry_owed = false;          // this round of the alignment barriers has not passed the retry point yet
   if (!warm) {   // least-squares multiplier start: (I + J^T J) t = -(grad_x L) - J^T (grad_s L),  y = J t + grad_s L
-    align_warps(A.align_group, 1); mids = 0;
-    mid_flush<L>(A, mids);
+    align_warps<L>(1); retry_arrive<L>();
     ph_derivs<L, false>(A, lane, true, df, o.mu_init, 0.0, false, cold);
     al_count<L>(0, lane);
     const bool ok = riccati_factor<L>(T, ric, A.ricmap, 1.0, 0.0, lane);
@@ -1497,8 +1484,8 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
     // Alignment point: the warps of a block start every IPM iteration together, so that they walk through the
     // same ~200 KB of phase code at the same time and share instruction-cache lines (unaligned warps thrash it:
     // `no_instruction` was 56 % of all stall cycles in v3).  Pure scheduling; results cannot depend on it.
-    mid_flush<L>(A, mids);
-    align_warps(A.align_group, 1); mids = 0;
+    if (retry_owed) retry_arrive<L>();
+    align_warps<L>(1); retry_owed = true;
     int mode = (int)AL(F_MODE);
     do_derivs<L>(A, lane, mode, df, 0.0, 0, cold);
     // ---- optimality error (scaled) and termination
@@ -1548,7 +1535,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
       }
     }
     bool goto_resto = !ok;                  // step computation failed: fall back to the restoration phase
-    mid_sync<L>(A, 1, mids);                // re-align after the inertia-correction retries (on by default: -5 % .. -21 % per iteration)
+    retry_sync<L>(); retry_owed = false;    // re-align after the inertia-correction retries (-5 % .. -21 % per iteration)
     if (ok) {
       if (dw > 0.0) AL(F_DWLAST) = dw;
       riccati_forward<L>(T, ric, false, lane, DX0, DU0);
@@ -1665,7 +1652,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
       }
       if (!accepted) {
         if (AL(F_INSOFT) == 0.0) augment_filter<L>(A, cold, mode, lane);
-        if (AL(F_THETA) <= 1e-2 * o.tol || !o.resto) { status = NMPC_RESTORATION_FAILED; break; }    // "... called, but point is almost feasible"
+        if (AL(F_THETA) <= 1e-2 * o.tol) { status = NMPC_RESTORATION_FAILED; break; }    // "... called, but point is almost feasible"
         tag = 'R';
         if (mode) { resto_inner<L>(A, cold, lane, df); alpha = 0.0; a_du = 0.0; moved = false; used_soc = false; accepted = true; }
         else entered_resto = true;
@@ -1679,7 +1666,6 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
       Lg[7] = AL(F_C0 + 1) - ls_before; Lg[8] = (double)tag; Lg[9] = (double)mode;
     }
     if (entered_resto) { resto_enter<L>(A, cold, lane, df); ++iter; continue; }
-    mid_sync<L>(A, 2, mids);                // re-align after the line search (off by default: measured neutral)
     // ---- accept (IpoptAlgorithm::AcceptTrialPoint)
     if (moved) do_accept<L>(A, lane, mode, 0.0, 0.0, dw, false, true, cold);     // the soft step already moved the iterate: kappa_Sigma reset only
     else do_accept<L>(A, lane, mode, alpha, a_du, dw, used_soc, true, cold);
@@ -1687,7 +1673,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
     if (mode) al_count<L>(4, lane);
     ++iter;
   }
-  mid_flush<L>(A, mids);
+  if (retry_owed) retry_arrive<L>();
   ph_output<L>(A, b, lane, df, status, iter, step);
   if (lane == 0 && A.stats) {
 #pragma unroll
@@ -1742,7 +1728,7 @@ __global__ void __launch_bounds__(32 * Lay<N_, NOBS_, MODEL_>::WPB, 1) nmpc_ipm_
     fin = __shfl_sync(FULL, fin, 0);
     if (fin == A.B - 1 && A.order_out) next_order<L>(A, lane);           // last instance of the call
   }
-  while (align_warps(A.align_group, 0)) { int m = 0; mid_flush<L>(A, m); }   // out of work: keep matching the alignment barriers until the group is done
+  while (align_warps<L>(0)) retry_arrive<L>();   // out of work: keep matching the alignment barriers until the block is done
 }
 
 #undef LV
