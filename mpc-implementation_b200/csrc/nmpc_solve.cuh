@@ -196,13 +196,28 @@ __device__ __forceinline__ double obs_value(const double* X, int jn, double& nx,
   iD = rcp(D); nx = dx_ * iD; ny = dy_ * iD;
   return smem[L::OBS0 + 3 * jn + 2] - D;
 }
-// Visit the rows of this lane's stage: the five box rows fully unrolled (static state index si), the obstacle
-// rows in a rolled loop.  body(r, box, si, gu, nx, ny, iD) with gu the unscaled row value.
-#define FOR_ROWS(X, body)                                                                           \
+// Per-lane scratch of a phase: 8 doubles per lane of the Riccati staging area, which is live only inside the riccati_*
+// calls.  The rolled row and control loops below keep there what they would otherwise index dynamically in registers
+// (which would put the array in local memory).
+template <class L>
+__device__ __forceinline__ double& stash(int i, int lane) { return smem[L::STG0 + i * 32 + lane]; }
+static_assert(8 * 32 <= STG_N, "stash must fit the Riccati staging area");
+// the states a box row reads, stashed for a FOR_ROWS over states held in registers
+template <class L>
+__device__ __forceinline__ void stash_box_states(const double* X, int lane) {
+#pragma unroll
+  for (int i = 2; i < 8; ++i) stash<L>(i, lane) = X[i];
+}
+
+// Visit the rows of this lane's stage: the box rows and the obstacle rows each in a rolled loop (one copy of the body
+// per kind of row: the phases that visit rows are what bounds the instruction cache, DESIGN.md section 2).
+// body(r, box, si, gu, nx, ny, iD) with gu the unscaled row value; si is the (run-time) state index of a box row, whose
+// value XB(si) reads from shared memory; X holds the states x, y of the obstacle rows.
+#define FOR_ROWS(XB, X, body)                                                                       \
   do {                                                                                              \
-    _Pragma("unroll") for (int r_ = 0; r_ < L::NB; ++r_) {                                          \
-      const int si_ = r_ == 0 ? 2 : (r_ == 1 ? 3 : r_ + 3);                                         \
-      body(r_, true, si_, (X)[si_], 0.0, 0.0, 0.0);                                                 \
+    _Pragma("unroll 1") for (int r_ = 0; r_ < L::NB; ++r_) {                                        \
+      const int si_ = box_state(r_);                                                                \
+      body(r_, true, si_, XB(si_), 0.0, 0.0, 0.0);                                                  \
     }                                                                                               \
     _Pragma("unroll 1") for (int jn_ = 0; jn_ < L::NOBS; ++jn_) {                                   \
       double nx_, ny_, iD_;                                                                         \
@@ -390,7 +405,9 @@ __device__ __noinline__ int ph_start(const SolveArgs& A, int lane, int b_, doubl
       else if (b.hl) bad_lb = true;                     // a lower bound on an obstacle row: not this NLP family
       nz += (b.hl ? 1 : 0) + (b.hu ? 1 : 0);
     };
-    FOR_ROWS(st.X, body);
+    stash_box_states<L>(st.X, lane);
+    auto xb = [&](int si) { return stash<L>(si, lane); };
+    FOR_ROWS(xb, st.X, body);
   }
   __syncwarp();
   const int total = __reduce_add_sync(FULL, nz);
@@ -441,9 +458,20 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
     for (int i = 0; i < 8; ++i) LV(LV_X + i) = st.X[i];
 #pragma unroll
     for (int v = 0; v < 6; ++v) { gl[v] *= df; LV(LV_GL + v) = gl[v]; a[cost_state(v)] = gl[v]; qa[cost_state(v)] = gl[v]; }
-    double q66[21], q22 = 0.0, nn[3] = {0.0, 0.0, 0.0};
+    double q66[21], nn[3] = {0.0, 0.0, 0.0};
 #pragma unroll
     for (int e = 0; e < 21; ++e) q66[e] = ls ? 0.0 : df * Hl[e];
+    // The box rows run in a rolled loop, and each touches the entries of its own state si only (the obstacle rows touch
+    // x, y only): their entries of a, qa, qb, qd and of the Hessian start in shared memory (a in the stash) and the rows
+    // accumulate there.  The explicit fma is what the compiler made of `acc += dc * v` in the unrolled form.
+#pragma unroll
+    for (int i = 2; i < 8; ++i) {
+      stash<L>(i, lane) = a[i]; LQ(LQ_QA + i) = qa[i];
+      if (!L::FOLD) { LQ(LQ_QB + i) = 0.0; LQ(LQ_QD + i) = 0.0; }
+    }
+#pragma unroll
+    for (int e = 3; e < 21; ++e) LQ(LQ_Q + e) = q66[e];
+    LQ(LQ_Q + 21) = 0.0;
     const double kd = A.o.kappa_d;
     auto body = [&](const int r, const bool box, const int si, const double gu, double nx, double ny, double iD) {
       const double dc = RW(A_DC, r);
@@ -455,29 +483,33 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
       double beta = iu - il;                              // barrier gradient per unit mu (with damping)
       if (hl && !hu) beta += kd;
       if (hu && !hl) beta -= kd;
-      double ya, w, yad;                                  // ya: delta_w- and mu-free part of y-hat; yad: seed of the adjoint
+      double ya, wk, yad;                                 // ya: delta_w- and mu-free part of y-hat; yad: seed of the adjoint; dc^2 wk: row weight
       if (RS) {
         oth += fabs(c); oinf = fmax(oinf, fabs(c));
         const RestoRow q = resto_row<L>(A, cold, lane, r, sig, beta, y, mu, dw);
         c += RG(G_N, r) - RG(G_P, r);
         const double chat = c + q.rs * rcp(q.D) + q.rp * rcp(q.Dp) - q.rn * rcp(q.Dn);
-        ya = y + q.Om * chat; w = dc * dc * q.Om; yad = y;
+        ya = y + q.Om * chat; wk = q.Om; yad = y;
         // n / p parts of the optimality error
         const double gn = A.o.resto_rho + y - q.zn, gp = A.o.resto_rho - y - q.zp;
         du_l = fmax(du_l, fmax(fabs(gn), fabs(gp))); if (want1) du1 += fabs(gn) + fabs(gp);
         sumz += q.zn + q.zp;
         compl_(q.n * q.zn); compl_(q.p * q.zp);
       } else if (L::FOLD && !ls) {      // mu and delta_w folded in: Q gets G^T (Sigma_s + dw) G, q gets G^T ((Sigma_s + dw) c + mu beta)
-        ya = (sig + dw) * c + mu * beta; w = dc * dc * (sig + dw); yad = y;
+        ya = (sig + dw) * c + mu * beta; wk = sig + dw; yad = y;
       } else {
-        ya = ls ? (vu - vl) : sig * c; w = dc * dc * sig; yad = y;
+        ya = ls ? (vu - vl) : sig * c; wk = sig; yad = y;
       }
       if (box) {
-        a[si] += dc * yad; qa[si] += dc * ya;
-        if (!RS && !L::FOLD) { qb[si] += dc * beta; qd[si] += dc * c; }
-        if (si == 3) q22 += w; else q66[tri(si < 3 ? si : si - 2, si < 3 ? si : si - 2)] += w;
+        stash<L>(si, lane) = __fma_rn(dc, yad, stash<L>(si, lane)); LQ(LQ_QA + si) = __fma_rn(dc, ya, LQ(LQ_QA + si));
+        if (!RS && !L::FOLD) {
+          LQ(LQ_QB + si) = ls ? 0.0 : __fma_rn(dc, beta, LQ(LQ_QB + si)); LQ(LQ_QD + si) = ls ? 0.0 : __fma_rn(dc, c, LQ(LQ_QD + si));
+        }
+        const int qi = si == 3 ? 21 : tri(si < 3 ? si : si - 2, si < 3 ? si : si - 2);
+        LQ(LQ_Q + qi) = __fma_rn(dc * dc, wk, LQ(LQ_Q + qi));
         if (!L::FOLD) LQ(LQ_DG + r) = RS ? 0.0 : dc * dc;
       } else {
+        const double w = dc * dc * wk;
         const double cur = ls ? 0.0 : -y * dc * iD;        // y * d2h,  d2h = -(I - n n^T)/D
         q66[0] += w * nx * nx + cur * (1.0 - nx * nx);
         q66[1] += w * nx * ny - cur * nx * ny;
@@ -501,16 +533,18 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
       if (lo_o > -1e19) viol = fmax(viol, lo_o - gu);
       if (hi_o < 1e19) viol = fmax(viol, gu - hi_o);
     };
-    FOR_ROWS(st.X, body);
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, st.X, body);
 #pragma unroll
-    for (int e = 0; e < 21; ++e) LQ(LQ_Q + e) = q66[e];
+    for (int i = 2; i < 8; ++i) a[i] = stash<L>(i, lane);
+#pragma unroll
+    for (int e = 0; e < 3; ++e) LQ(LQ_Q + e) = q66[e];
     LQ(LQ_ZERO) = 0.0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) LQ(LQ_QA + i) = qa[i];
+    LQ(LQ_QA + 0) = qa[0]; LQ(LQ_QA + 1) = qa[1];
     if (!L::FOLD) {
       LQ(LQ_NN + 0) = nn[0]; LQ(LQ_NN + 1) = nn[1]; LQ(LQ_NN + 2) = nn[2];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) { LQ(LQ_QB + i) = ls ? 0.0 : qb[i]; LQ(LQ_QD + i) = ls ? 0.0 : qd[i]; }
+      for (int i = 0; i < 2; ++i) { LQ(LQ_QB + i) = ls ? 0.0 : qb[i]; LQ(LQ_QD + i) = ls ? 0.0 : qd[i]; }
     }
     if (!L::FOLD && L::NB < 5) {      // rows that do not exist in this model
 #pragma unroll
@@ -518,7 +552,6 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
     }
     LQ(LQ_DD + 0) = st.cps * st.cth; LQ(LQ_DD + 1) = st.sps * st.cth; LQ(LQ_DD + 2) = st.sth;
     LQ(LQ_EE + 0) = dy.e03; LQ(LQ_EE + 1) = dy.e13; LQ(LQ_EE + 2) = dy.e23; LQ(LQ_EE + 3) = dy.e04; LQ(LQ_EE + 4) = dy.e14;
-    LQ(LQ_Q + 21) = q22;
   }
   double lamn[8];
   adjoint<L::SW>(a, dy, act, lane, lamn);
@@ -537,20 +570,20 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
     LQ(LQ_Q + 21) += q33; LQ(LQ_Q + 22) = q34; LQ(LQ_Q + 23) = q44;
     LQ(LQ_SV + 0) = svt; LQ(LQ_SV + 1) = svp;
     // controls: Sigma_x, gradient per unit mu, dual infeasibility, complementarity products
-    double glx[6];
-    glx[0] = T * (st.cps * st.cth * lamn[0] + st.sps * st.cth * lamn[1] + st.sth * lamn[2]);
+    // (the gradient glx goes through the stash to the rolled control loop)
+    stash<L>(0, lane) = T * (st.cps * st.cth * lamn[0] + st.sps * st.cth * lamn[1] + st.sth * lamn[2]);
 #pragma unroll
-    for (int r = 1; r < 6; ++r) glx[r] = T * lamn[r + 2];
+    for (int r = 1; r < 6; ++r) stash<L>(r, lane) = T * lamn[r + 2];
     const double eta = RS ? A.o.resto_eta_factor * sqrt(mu) : 0.0;
-#pragma unroll
+#pragma unroll 1
     for (int i = 0; i < 6; ++i) {
       double sig = 1.0, rb = 0.0;       // absent controls (model 1) keep the unit diagonal and a zero right-hand side
       if (hasu && i < L::NUA) {
         const Bnd b = ctl_bounds<L>(A, lane, i);
-        const double zl = LV(LV_ZL + i), zu = LV(LV_ZU + i);
-        const double sl = (u[i] - b.lo), su = (b.hi - u[i]);
-        double gR = 0.0;
-        if (RS) { const double ur = UREF(i), d = rcp(fmax(1.0, fabs(ur))); gR = eta * d * d * (u[i] - ur); glx[i] += gR; }
+        const double ui = LV(LV_U + i), zl = LV(LV_ZL + i), zu = LV(LV_ZU + i);
+        const double sl = (ui - b.lo), su = (b.hi - ui);
+        double gli = stash<L>(i, lane), gR = 0.0;
+        if (RS) { const double ur = UREF(i), d = rcp(fmax(1.0, fabs(ur))); gR = eta * d * d * (ui - ur); gli += gR; }
         if (ls) rb = zu - zl;
         else {
           const double il = b.hl ? rcp(sl) : 0.0, iu = b.hu ? rcp(su) : 0.0;
@@ -559,7 +592,7 @@ __device__ __noinline__ void ph_derivs(const SolveArgs& A, int lane, bool ls, do
           if (b.hu && !b.hl) rb -= A.o.kappa_d;
           if (RS) { const double ur = UREF(i), d = rcp(fmax(1.0, fabs(ur))); sig += eta * d * d; rb += gR / mu; }
         }
-        const double gx = fabs(glx[i] - zl + zu);
+        const double gx = fabs(gli - zl + zu);
         du_l = fmax(du_l, gx); if (want1) du1 += gx;
         sumz += zl + zu;
         if (b.hl) compl_(sl * zl);
@@ -592,11 +625,12 @@ __device__ __noinline__ void ph_lsy(const SolveArgs& A, int lane, bool ok) {
     for (int i = 0; i < 8; ++i) { X[i] = LV(LV_X + i); dx[i] = LV(LV_DX + i); }
     auto body = [&](const int r, const bool box, const int si, const double gu, double nx, double ny, double iD) {
       const double dc = RW(A_DC, r);
-      const double gd = box ? dc * dx[si] : -dc * (nx * dx[0] + ny * dx[1]);
+      const double gd = box ? dc * LV(LV_DX + si) : -dc * (nx * dx[0] + ny * dx[1]);
       const double yv = gd + (RW(A_VU, r) - (box ? RW(A_VL, r) : 0.0));
       RW(A_Y, r) = yv; ymax = fmax(ymax, fabs(yv));
     };
-    FOR_ROWS(X, body);
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, X, body);
   }
   ymax = warp_max(ymax);
   if (!ok || !(ymax <= A.o.constr_mult_init_max)) {
@@ -628,7 +662,7 @@ __device__ __noinline__ void ph_dir(const SolveArgs& A, int lane, double mu, dou
       double beta = iu - il;
       if (hl && !hu) beta += kd;
       if (hu && !hl) beta -= kd;
-      const double gd = box ? dc * dx[si] : -dc * (nx * dx[0] + ny * dx[1]);
+      const double gd = box ? dc * LV(LV_DX + si) : -dc * (nx * dx[0] + ny * dx[1]);
       double c, ds;
       if (RS) {
         const double y = RW(A_Y, r);
@@ -659,10 +693,11 @@ __device__ __noinline__ void ph_dir(const SolveArgs& A, int lane, double mu, dou
       gbd += mu * beta * ds; theta += fabs(c);
       nottiny = nottiny || (fabs(ds) > tt * (1.0 + fabs(s)));
     };
-    FOR_ROWS(X, body);
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, X, body);
     if (hasu) {
       const double eta = RS ? A.o.resto_eta_factor * sqrt(mu) : 0.0;
-#pragma unroll
+#pragma unroll 1
       for (int i = 0; i < 6; ++i) {
         const Bnd b = ctl_bounds<L>(A, lane, i);
         const double u = LV(LV_U + i), du = soc ? SOC(SOC_DUS + i) : LV(LV_DU + i), zl = LV(LV_ZL + i), zu = LV(LV_ZU + i);
@@ -710,20 +745,24 @@ __device__ __noinline__ void ph_trial(const SolveArgs& A, int lane_, double alph
   const bool act = lane <= L::N, hasu = lane < L::N;
   double ut[6], lb = 0.0, dt = 0.0, fr = 0.0;
   double prod = 1.0; int cnt = 0;
-#pragma unroll
+  // the trial controls go through the stash (physical lane: with pairing both halves use it) to the rollout
+#pragma unroll 1
   for (int i = 0; i < 6; ++i) {
-    ut[i] = 0.0;
+    double uti = 0.0;
     if (hasu) {
-      ut[i] = fma(alpha, soc ? SOC(SOC_DUS + i) : LV(LV_DU + i), LV(LV_U + i));   // same expression as ph_accept
+      uti = fma(alpha, soc ? SOC(SOC_DUS + i) : LV(LV_DU + i), LV(LV_U + i));   // same expression as ph_accept
       const Bnd b = ctl_bounds<L>(A, lane, i);
-      if (b.hl) prod *= (ut[i] - b.lo);
-      if (b.hu) prod *= (b.hi - ut[i]);
-      if (b.hl && !b.hu) dt += ut[i] - b.lo;
-      if (b.hu && !b.hl) dt += b.hi - ut[i];
+      if (b.hl) prod *= (uti - b.lo);
+      if (b.hu) prod *= (b.hi - uti);
+      if (b.hl && !b.hu) dt += uti - b.lo;
+      if (b.hu && !b.hl) dt += b.hi - uti;
       if (i == 2 || i == 5) { lb += n_log(prod); prod = 1.0; }
-      if (RS) { const double ur = UREF(i), d = rcp(fmax(1.0, fabs(ur))), e = d * (ut[i] - ur); fr += e * e; }
+      if (RS) { const double ur = UREF(i), d = rcp(fmax(1.0, fabs(ur))), e = d * (uti - ur); fr += e * e; }
     }
+    stash<L>(i, lane_) = uti;
   }
+#pragma unroll
+  for (int i = 0; i < 6; ++i) ut[i] = stash<L>(i, lane_);
   Stage st; rollout<L::SW>(pr, &PAR(0), ut, lane, st);
   double l = 0.0;
   if (!RS) l = hasu ? cost_val<L>(A, st.X, lane) : 0.0;
@@ -751,7 +790,9 @@ __device__ __noinline__ void ph_trial(const SolveArgs& A, int lane_, double alph
       if (b.hu && !b.hl) dt += b.hi - sv;
       if (cnt >= 4) { lb += n_log(prod); prod = 1.0; cnt = 0; }
     };
-    FOR_ROWS(st.X, body);
+    stash_box_states<L>(st.X, lane_);
+    auto xb = [&](int si) { return stash<L>(si, lane_); };
+    FOR_ROWS(xb, st.X, body);
     if (cnt) lb += n_log(prod);
   }
   // per half-warp sums where pairing is possible (the lanes >= SW hold zeros when unpaired: lane 0's sums are warp_sum's)
@@ -794,11 +835,13 @@ __device__ __noinline__ void ph_socrhs(const SolveArgs& A, int lane, double a_so
         const RestoRow w = resto_row<L>(A, cold, lane, r, sig, beta, y, mu, dw);
         yh = y + w.Om * (cs + w.rs * rcp(w.D) + w.rp * rcp(w.Dp) - w.rn * rcp(w.Dn));
       } else yh = (sig + dw) * cs + mu * beta;
-      if (box) q[si] += dc * yh; else { q[0] -= dc * yh * nx; q[1] -= dc * yh * ny; }
+      if (box) SOC(SOC_Q2 + si) = __fma_rn(dc, yh, SOC(SOC_Q2 + si)); else { q[0] -= dc * yh * nx; q[1] -= dc * yh * ny; }
     };
-    FOR_ROWS(X, body);
 #pragma unroll
-    for (int i = 0; i < 8; ++i) SOC(SOC_Q2 + i) = q[i];
+    for (int i = 2; i < 8; ++i) SOC(SOC_Q2 + i) = q[i];      // box entries: accumulated in place by the rolled box rows
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, X, body);
+    SOC(SOC_Q2 + 0) = q[0]; SOC(SOC_Q2 + 1) = q[1];
   }
   __syncwarp();
 }
@@ -849,7 +892,7 @@ __device__ __noinline__ void ph_accept(const SolveArgs& A, int lane, double alph
   const double smin = EPSM * fmin(1.0, mu);
   bool bad = false;
   if (hasu) {
-#pragma unroll
+#pragma unroll 1
     for (int i = 0; i < 6; ++i) {
       const Bnd b = ctl_bounds<L>(A, lane, i);
       const double u = LV(LV_U + i), du = soc ? SOC(SOC_DUS + i) : LV(LV_DU + i);
@@ -937,7 +980,8 @@ __device__ __noinline__ void ph_resto_init(const SolveArgs& A, int lane, double 
       if (box) RW(A_VL, r) = fmin(rho, RW(A_VL, r));
       RW(A_VU, r) = fmin(rho, RW(A_VU, r)); RW(A_Y, r) = 0.0;
     };
-    FOR_ROWS(X, body);
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, X, body);
 #pragma unroll
     for (int i = 0; i < 6; ++i) { UREF(i) = LV(LV_U + i); LV(LV_ZL + i) = fmin(rho, LV(LV_ZL + i)); LV(LV_ZU + i) = fmin(rho, LV(LV_ZU + i)); }
   }
@@ -956,7 +1000,8 @@ __device__ __noinline__ void ph_resto_np(const SolveArgs& A, int lane, double mu
       const double a = h - 0.5 * c, nv = a + sqrt(a * a + c * h);
       RG(G_N, r) = nv; RG(G_P, r) = c + nv; RG(G_DN, r) = 0.0; RG(G_DP, r) = 0.0; RG(G_DY, r) = 0.0;
     };
-    FOR_ROWS(X, body);
+    auto xb = [&](int si) { return LV(LV_X + si); };
+    FOR_ROWS(xb, X, body);
   }
   __syncwarp();
 }
@@ -1061,7 +1106,9 @@ __device__ __noinline__ void ph_output(const SolveArgs& A, int b, int lane, doub
     if (A.g) {
       double* go = A.g + (size_t)b * ng + lane * R;
       auto body = [&](const int r, const bool box, const int si, const double gu, double nx, double ny, double iD) { go[r] = gu; };
-      FOR_ROWS(st.X, body);
+      stash_box_states<L>(st.X, lane);
+      auto xb = [&](int si) { return stash<L>(si, lane); };
+      FOR_ROWS(xb, st.X, body);
     }
     if (A.lam_g) {
       double* lo = A.lam_g + (size_t)b * ng + lane * R;
