@@ -89,6 +89,13 @@ int nmpc_destroy(nmpc_handle* h);
 
 /* flags for nmpc_solve */
 #define NMPC_OBS_PER_INSTANCE 1u   /* obst is [B][n_obs][3] instead of [n_obs][3] */
+#define NMPC_PREDICT_TARGET 2u     /* nmpc_solve_and_step / nmpc_run_closed_loop only: every solve uses the target's own Euler
+                                      prediction over the horizon instead of the frozen target p[8:10] -- stage k of instance b
+                                      sees  th_k = th_t + (T om) k,  s_k = (T v)(cos th_k, sin th_k),  (x, y)_k = (x_t, y_t) +
+                                      (s_0 + ... + s_{k-1})  with (x_t, y_t, th_t) the target block of p and (v, om) this step's
+                                      target input (target_vw or the schedule), computed in the kernel, no host work per step.
+                                      Refused by the calls that have no (v, om) (nmpc_solve, nmpc_solve_host(_async), nmpc_eval,
+                                      nmpc_lam_p) and while a target trajectory is set (nmpc_set_target_trajectory). */
 
 /* solver(x0,lbx,ubx,lbg,ubg,p)  (NMPC_TT.py:358-365), B instances at once.
  *   p    [B][11]   x0  [B][6N]                       inputs
@@ -175,7 +182,9 @@ int nmpc_solve_and_step(nmpc_handle* h, int32_t B, double* p, double* u_warm,
  *   at mpc_iter, mpc_iter + 1, ...; the step counter advances by `steps`)
  *   x [B][n_w], f [B]: solution of the LAST step (may be NULL);  fov_centre [B][2], err_accum [B] (+=) as in nmpc_step
  *   status_log, iters_log [steps][B]: outcome of every solve (may be NULL);  converged [B]: += number of converged solves (may be NULL)
- * Not available with a per-step target prediction (nmpc_set_target_trajectory), which the host recomputes every step. */
+ * Every option of nmpc_solve_and_step applies to every step: the target prediction (flags |= NMPC_PREDICT_TARGET) is made from
+ * each step's own target, and moving obstacles (nmpc_set_obstacle_motion) move after each step.  Not available with a
+ * caller-given target trajectory (nmpc_set_target_trajectory), which would hold for one step only. */
 int nmpc_run_closed_loop(nmpc_handle* h, int32_t B, int32_t steps, double* p, double* u_warm,
                          const double* lbx, const double* ubx, const double* lbg, const double* ubg,
                          const double* obst, uint32_t flags, const double* target_vw,
@@ -224,8 +233,19 @@ int nmpc_set_weights(nmpc_handle* h, const double* dev_weights);
 /* Predicted target trajectory (north star: "p = [UAV state; predicted target trajectory]"; SURVEY 8f-2).  The reference
  * holds the target at p[8:10] over the whole horizon (NMPC_TT.py:219-220); with dev_targets [B][N][2] = (x_t, y_t) of
  * stage k = 0..N-1 every stage cost uses its own prediction instead.  Read by every subsequent nmpc_solve /
- * nmpc_solve_host / nmpc_eval on this handle (must stay allocated, at least B rows); NULL restores p[8:10]. */
+ * nmpc_solve_host / nmpc_eval / nmpc_solve_and_step on this handle (must stay allocated, at least B rows); NULL restores
+ * p[8:10].  A closed loop that wants the target's own Euler prediction every step passes NMPC_PREDICT_TARGET instead,
+ * which computes it in the kernel (and works in nmpc_run_closed_loop); the two exclude each other. */
 int nmpc_set_target_trajectory(nmpc_handle* h, const double* dev_targets);
+
+/* Moving obstacles (MATLAB/Dynamic Obstacles: obstacle positions are parameters that move every step; SURVEY 8f-2).
+ * dev_obst [B][n_obs][3] = (cx, cy, r_uav + r_obs) is the writable per-instance obstacle field that the following
+ * nmpc_solve_and_step / nmpc_run_closed_loop calls pass as `obst` (with NMPC_OBS_PER_INSTANCE when B > 1); dev_vel
+ * [B][n_obs][2] holds the obstacle velocities.  After each solve those calls advance the centres in place,
+ * cx += T vx, cy += T vy (rounded as o + (T v)); the constraint rows of that solve use the positions before the move.
+ * They fail if `obst` is not dev_obst, or is a shared table while B > 1.  The other calls neither check nor move.
+ * NULL, NULL removes the motion.  Both arrays stay owned by the caller and must outlive their use. */
+int nmpc_set_obstacle_motion(nmpc_handle* h, double* dev_obst, const double* dev_vel);
 
 /* NON-REFERENCE fast mode (SURVEY.md 8f-4): warm start of the multipliers -- CasADi's lam_x0 / lam_g0 inputs with
  * ipopt.warm_start_init_point = "yes".  No reference script uses it (they pass neither, NMPC_TT.py:358-365), and it changes

@@ -13,6 +13,7 @@ _CSRC = Path(__file__).resolve().parent / "csrc"
 LIB_PATH = Path(__import__("os").environ.get("NMPC_B200_LIB", _CSRC / "libnmpc_b200.so"))     # override: A/B timing of library builds
 
 NMPC_OBS_PER_INSTANCE = 1
+NMPC_PREDICT_TARGET = 2      # nmpc_solve_and_step / nmpc_run_closed_loop: the target's own Euler prediction, made in the kernel
 
 # CasADi's stats()['return_status'] strings of the IPOPT plugin
 STATUS_NAMES = {0: "Solve_Succeeded", 1: "Maximum_Iterations_Exceeded", 2: "Restoration_Failed",
@@ -42,7 +43,7 @@ class NmpcStats(C.Structure):
 
 
 EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_step",
-           "nmpc_get_stats", "nmpc_set_debug_log", "nmpc_set_order", "nmpc_set_weights", "nmpc_set_target_trajectory", "nmpc_set_schedule", "nmpc_set_warm_start", "nmpc_measure_fp64_peak", "nmpc_n_w", "nmpc_n_g", "nmpc_n_p",
+           "nmpc_get_stats", "nmpc_set_debug_log", "nmpc_set_order", "nmpc_set_weights", "nmpc_set_target_trajectory", "nmpc_set_obstacle_motion", "nmpc_set_schedule", "nmpc_set_warm_start", "nmpc_measure_fp64_peak", "nmpc_n_w", "nmpc_n_g", "nmpc_n_p",
            "nmpc_last_error", "nmpc_version"]
 
 _lib = None
@@ -87,6 +88,8 @@ def lib():
         L.nmpc_set_warm_start.argtypes = [vp, vp, vp, C.POINTER(NmpcWarmOpts)]
     if hasattr(L, "nmpc_set_schedule"):      # (absent only in old builds loaded through NMPC_B200_LIB for A/B timing)
         L.nmpc_set_schedule.argtypes = [vp, vp, C.c_int32, C.c_int32, vp, vp, C.c_int32]
+    if hasattr(L, "nmpc_set_obstacle_motion"):
+        L.nmpc_set_obstacle_motion.argtypes = [vp, vp, vp]
     L.nmpc_measure_fp64_peak.argtypes = [C.c_int, C.POINTER(C.c_double)]
     L.nmpc_n_w.argtypes = [C.POINTER(NmpcSpec)]
     L.nmpc_n_g.argtypes = [C.POINTER(NmpcSpec)]

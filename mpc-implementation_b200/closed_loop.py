@@ -35,7 +35,10 @@ class ClosedLoop:
         prediction over the horizon (same model as the target step of shift_timestep, NMPC_TT.py:24-27) instead of
         the frozen target the reference uses.  obstacles [B, n_obs, 3] = (cx, cy, r_uav + r_obs) per instance and
         obstacle_vel [B, n_obs, 2]: obstacle fields as data, moved by T * velocity after every step (the moving
-        obstacles of MATLAB/Dynamic Obstacles/Dynamic Obstacle avoidance.m:128-133, whose positions are parameters)."""
+        obstacles of MATLAB/Dynamic Obstacles/Dynamic Obstacle avoidance.m:128-133, whose positions are parameters; a shared
+        [n_obs, 3] field with [n_obs, 2] velocities is given every instance as its own copy).  The fused step and run_free
+        make the prediction and move the obstacles inside the kernel (NMPC_PREDICT_TARGET, nmpc_set_obstacle_motion), bit-identical
+        to target_prediction() and _move_obstacles(), which the unfused step (want_g / want_lam) still uses."""
         self.predict_target = predict_target
         dev0 = device or f"cuda:{solver.device}"
         t64 = lambda a: None if a is None else torch.as_tensor(np.asarray(a, dtype=np.float64) if not torch.is_tensor(a) else a,
@@ -45,6 +48,10 @@ class ClosedLoop:
         dev = device or f"cuda:{solver.device}"
         self.p = torch.as_tensor(np.asarray(p0, dtype=np.float64), device=dev).reshape(-1, scenario.n_p).contiguous().clone()
         self.B = self.p.shape[0]
+        if self.obstacles is not None and self.obstacle_vel is not None:      # per-instance fields: the kernel moves them in place
+            n_obs = self.obstacles.shape[-2]
+            self.obstacles = self.obstacles.reshape(-1, n_obs, 3).expand(self.B, n_obs, 3).contiguous()
+            self.obstacle_vel = self.obstacle_vel.reshape(-1, n_obs, 2).expand(self.B, n_obs, 2).contiguous()
         self.u_warm = torch.zeros((self.B, scenario.n_w), dtype=torch.float64, device=dev)     # u0 = 0  (:329)
         lbx, ubx, lbg, ubg = scenario.bounds()
         to = lambda a: torch.as_tensor(a, dtype=torch.float64, device=dev)
@@ -90,6 +97,9 @@ class ClosedLoop:
         rows = self._sched_dev if self._sched_dev is not None else torch.zeros_like(at)
         self.vw.copy_(self.sched_table[rows, at])
 
+    def _moving_vel(self):
+        return self.obstacle_vel if self.obstacles is not None else None
+
     def _move_obstacles(self):
         if self.obstacles is not None and self.obstacle_vel is not None:
             self.obstacles[:, :, :2] += self.sc.T * self.obstacle_vel
@@ -117,20 +127,19 @@ class ClosedLoop:
 
     def step(self, want_g: bool = False, want_lam: bool = False, want_x: bool = True):
         """One closed-loop batch step; returns the solver output dict (device tensors).  Without g / multipliers
-        the solve and the shift are one launch (nmpc_solve_and_step)."""
-        if self._const_vw or self.predict_target or want_g or want_lam:
-            self._schedule_vw()
+        the solve and the shift -- with the target prediction and the obstacle motion -- are one launch (nmpc_solve_and_step)
+        and the step costs no host work."""
         if self.warm_duals and (want_g or want_lam):
             raise ValueError("ClosedLoop: warm_duals needs the fused step (want_g = want_lam = False)")
         if not (want_g or want_lam):
             sol = self.solver.solve_and_step(self.p, self.u_warm, self.lbx, self.ubx, self.lbg, self.ubg,
                                              self.vw if self._const_vw else None, self.fov,
                                              self.err_sum, obstacles=self.obstacles, want_x=want_x,
-                                             target_traj=self.target_prediction() if self.predict_target else None)
-            self._move_obstacles()
+                                             predict_target=self.predict_target, obstacle_vel=self._moving_vel())
             self.mpc_iter += 1
             self.last = sol
             return sol
+        self._schedule_vw()
         sol = self.solver(x0=self.u_warm, p=self.p, lbx=self.lbx, ubx=self.ubx, lbg=self.lbg, ubg=self.ubg, obstacles=self.obstacles,
                           want_g=want_g, want_lam=want_lam,
                           target_traj=self.target_prediction() if self.predict_target else None)
@@ -145,12 +154,11 @@ class ClosedLoop:
 
     def run_free(self, steps: int, log: bool = True, want_x: bool = False):
         """`steps` closed-loop steps of every instance in one launch with no batch-wide barrier between the steps
-        (Solver.run_closed_loop): the fast way through a Monte-Carlo study; per instance bit-identical to step() x steps."""
-        if self.predict_target or self.obstacle_vel is not None:
-            raise ValueError("ClosedLoop.run_free: target predictions / moving obstacles are recomputed on the host every step; use step()")
+        (Solver.run_closed_loop): the fast way through a Monte-Carlo study; per instance bit-identical to step() x steps, also with
+        the target prediction and moving obstacles."""
         out = self.solver.run_closed_loop(steps, self.p, self.u_warm, self.lbx, self.ubx, self.lbg, self.ubg,
                                           self.vw if self._const_vw else None, self.fov, self.err_sum, obstacles=self.obstacles,
-                                          want_x=want_x, log=log)
+                                          want_x=want_x, log=log, predict_target=self.predict_target, obstacle_vel=self._moving_vel())
         self.mpc_iter += steps
         self.last = out
         return out

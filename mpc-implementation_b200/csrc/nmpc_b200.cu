@@ -256,6 +256,8 @@ struct nmpc_handle {
   int run_steps; int32_t *run_status_log, *run_iters_log, *run_conv;   // set for the duration of nmpc_run_closed_loop
   double *fuse_p, *fuse_u, *fuse_fov, *fuse_err; const double* fuse_vw;   // set for the duration of nmpc_solve_and_step
   const double* sched_table; const int32_t *sched_id, *sched_phase; int sched_rows, sched_len, sched_iter;   // nmpc_set_schedule
+  double* d_tgt_pred; int tgt_pred_cap;        // NMPC_PREDICT_TARGET: the trajectory the kernel predicts, [tgt_pred_cap][N][2]
+  double* move_obs; const double* move_vel;    // nmpc_set_obstacle_motion
   int* d_counter;                  // [4]: queue counter x2, done counter x2
   unsigned long long* d_stats;     // [2][NSTAT]
   unsigned long long* stats_last;  // the half written by the last call
@@ -355,7 +357,7 @@ int nmpc_destroy(nmpc_handle* h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
   void* ptrs[] = {h->d_ric, h->d_cold, h->d_counter, h->d_stats, h->d_p, h->d_x0, h->d_lbx, h->d_ubx, h->d_lbg, h->d_ubg, h->d_obs,
-                  h->d_x, h->d_f, h->d_g, h->d_lamx, h->d_lamg, h->d_status, h->d_iters, h->d_order[0], h->d_order[1], h->d_keep_iters, h->d_ricmap};
+                  h->d_x, h->d_f, h->d_g, h->d_lamx, h->d_lamg, h->d_status, h->d_iters, h->d_order[0], h->d_order[1], h->d_keep_iters, h->d_ricmap, h->d_tgt_pred};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   delete h;
@@ -371,6 +373,10 @@ int nmpc_solve(nmpc_handle* h, int32_t B, const double* p, const double* x0,
   if (B <= 0) return 0;
   if (!p || !x0 || !lbx || !ubx || !lbg || !ubg || (!x && !h->fuse_p)) return fail("nmpc_solve: null required pointer");
   if (h->pr.n_obs > 0 && !obst) return fail("nmpc_solve: obstacle table required");
+  const bool predict = (flags & NMPC_PREDICT_TARGET) != 0;
+  if (predict && !h->fuse_p)
+    return fail("nmpc_solve: NMPC_PREDICT_TARGET needs the target's (v, omega) of the step: use nmpc_solve_and_step or nmpc_run_closed_loop");
+  if (predict && h->tgt) return fail("nmpc_solve: NMPC_PREDICT_TARGET and a target trajectory (nmpc_set_target_trajectory) exclude each other");
   CK(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)cuda_stream;
   SolveArgs A;
@@ -396,10 +402,19 @@ int nmpc_solve(nmpc_handle* h, int32_t B, const double* p, const double* x0,
     CK(cudaMalloc(&h->d_keep_iters, sizeof(int32_t) * B));
     h->order_cap = B;
   }
+  if (predict && B > h->tgt_pred_cap) {     // the predicted trajectories, grown like the scheduling buffers
+    CK(cudaStreamSynchronize(s));
+    if (h->d_tgt_pred) cudaFree(h->d_tgt_pred);
+    h->d_tgt_pred = nullptr; h->tgt_pred_cap = 0;
+    CK(cudaMalloc(&h->d_tgt_pred, sizeof(double) * 2 * (size_t)h->pr.N * B));
+    h->tgt_pred_cap = B;
+  }
   A.iters_keep = h->d_keep_iters;
   A.step_p = h->fuse_p; A.step_u = h->fuse_u; A.step_vw = h->fuse_vw; A.step_fov = h->fuse_fov; A.step_err = h->fuse_err;
   A.sched_table = h->sched_table; A.sched_id = h->sched_id; A.sched_phase = h->sched_phase; A.sched_len = h->sched_len; A.sched_iter = h->sched_iter;
-  A.tgt = h->tgt;
+  A.tgt_pred = predict ? h->d_tgt_pred : nullptr;
+  A.tgt = predict ? h->d_tgt_pred : h->tgt;
+  A.obs_move = h->fuse_p ? h->move_obs : nullptr; A.obs_vel = h->move_vel;
   A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && h->fuse_p) ? 1 : 0;
   A.run_steps = h->run_steps > 1 ? h->run_steps : 1; A.status_log = h->run_status_log; A.iters_log = h->run_iters_log; A.conv_count = h->run_conv;
   A.weights = h->weights;
@@ -448,6 +463,10 @@ int nmpc_solve_and_step(nmpc_handle* h, int32_t B, double* p, double* u_warm,
   if (!target_vw && !h->sched_table) return fail("nmpc_solve_and_step: target_vw is NULL and no schedule is set (nmpc_set_schedule)");
   if (err_accum && !fov_centre) return fail("nmpc_solve_and_step: err_accum needs fov_centre");
   if (x == u_warm) return fail("nmpc_solve_and_step: x must not alias u_warm (pass NULL if the solution itself is not needed)");
+  if (h->move_obs && obst != h->move_obs)
+    return fail("nmpc_solve_and_step: obstacle motion is set (nmpc_set_obstacle_motion): obst must be the registered field");
+  if (h->move_obs && B > 1 && !(flags & NMPC_OBS_PER_INSTANCE))
+    return fail("nmpc_solve_and_step: obstacle motion needs a per-instance obstacle field (NMPC_OBS_PER_INSTANCE)");
   h->fuse_p = p; h->fuse_u = u_warm; h->fuse_vw = target_vw; h->fuse_fov = fov_centre; h->fuse_err = err_accum;
   const int rc = nmpc_solve(h, B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, x, f, nullptr, nullptr, nullptr, status, iters, cuda_stream);
   h->fuse_p = nullptr; h->fuse_u = nullptr; h->fuse_vw = nullptr; h->fuse_fov = nullptr; h->fuse_err = nullptr;
@@ -462,7 +481,8 @@ int nmpc_run_closed_loop(nmpc_handle* h, int32_t B, int32_t steps, double* p, do
                          int32_t* status_log, int32_t* iters_log, int32_t* converged, void* cuda_stream) {
   if (!h) return fail("nmpc_run_closed_loop: null handle");
   if (steps < 1) return fail("nmpc_run_closed_loop: steps must be >= 1");
-  if (h->tgt) return fail("nmpc_run_closed_loop: a per-step target prediction (nmpc_set_target_trajectory) needs the step-by-step calls");
+  if (h->tgt) return fail("nmpc_run_closed_loop: a caller-given target trajectory (nmpc_set_target_trajectory) needs the step-by-step calls; "
+                          "NMPC_PREDICT_TARGET predicts it on the device");
   h->run_steps = steps; h->run_status_log = status_log; h->run_iters_log = iters_log; h->run_conv = converged;
   const int sched0 = h->sched_iter;
   const int rc = nmpc_solve_and_step(h, B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, target_vw, x, f, fov_centre, err_accum,
@@ -504,6 +524,7 @@ int nmpc_solve_host_async(nmpc_handle* h, int32_t B, const double* p, const doub
                           int32_t* status, int32_t* iters) {
   if (!h) return fail("nmpc_solve_host: null handle");
   if (B <= 0) return 0;
+  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_solve_host: NMPC_PREDICT_TARGET needs the target's (v, omega): use nmpc_solve_and_step or nmpc_run_closed_loop");
   if (B > h->spec.max_batch) return fail("nmpc_solve_host: B exceeds spec.max_batch");
   CK(cudaSetDevice(h->device));
   cudaStream_t s = h->own_stream;
@@ -535,6 +556,7 @@ int nmpc_eval(nmpc_handle* h, int32_t B, const double* w, const double* p, const
               double* f, double* g, double* grad_f, double* jtv, double* hv, void* cuda_stream) {
   if (!h) return fail("nmpc_eval: null handle");
   if (B <= 0) return 0;
+  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_eval: NMPC_PREDICT_TARGET is available in nmpc_solve_and_step and nmpc_run_closed_loop only");
   if (!w || !p) return fail("nmpc_eval: null required pointer");
   if (h->pr.n_obs > 0 && !obst) return fail("nmpc_eval: obstacle table required");
   if (jtv && !lam) return fail("nmpc_eval: jtv needs lam");
@@ -555,6 +577,7 @@ int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, 
                const double* lam_g, double* lam_p, void* cuda_stream) {
   if (!h) return fail("nmpc_lam_p: null handle");
   if (B <= 0) return 0;
+  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_lam_p: NMPC_PREDICT_TARGET is available in nmpc_solve_and_step and nmpc_run_closed_loop only");
   if (!x_sol || !p || !lam_g || !lam_p) return fail("nmpc_lam_p: null required pointer");
   if (h->pr.n_obs > 0 && !obst) return fail("nmpc_lam_p: obstacle table required");
   CK(cudaSetDevice(h->device));
@@ -598,6 +621,14 @@ int nmpc_set_weights(nmpc_handle* h, const double* dev_weights) {
 int nmpc_set_target_trajectory(nmpc_handle* h, const double* dev_targets) {
   if (!h) return fail("nmpc_set_target_trajectory: null handle");
   h->tgt = dev_targets;
+  return 0;
+}
+
+int nmpc_set_obstacle_motion(nmpc_handle* h, double* dev_obst, const double* dev_vel) {
+  if (!h) return fail("nmpc_set_obstacle_motion: null handle");
+  if ((dev_obst == nullptr) != (dev_vel == nullptr)) return fail("nmpc_set_obstacle_motion: give both the obstacle field and the velocities, or neither");
+  if (dev_obst && h->pr.n_obs == 0) return fail("nmpc_set_obstacle_motion: this handle has no obstacle rows (spec.n_obs = 0)");
+  h->move_obs = dev_obst; h->move_vel = dev_vel;
   return 0;
 }
 

@@ -67,7 +67,13 @@ struct SolveArgs {
   // target schedule on the device (nmpc_set_schedule): when step_vw == NULL the target's (v, omega) of this step is
   // sched_table[sched_id[b]][min(sched_iter + sched_phase[b], sched_len - 1)]  -- the scripts' `con_t` keyed on mpc_iter
   const double* sched_table; const int32_t *sched_id, *sched_phase; int sched_len, sched_iter;
-  int32_t* iters_keep;               // handle-owned copy of iters[] (drives the next call's fetch order)
+  // target prediction on the device (NMPC_PREDICT_TARGET, fused calls only): ph_predict writes the target's own Euler prediction
+  // over the horizon from p's target block and this step's (v, omega) to tgt_pred [B][N][2], which is then also `tgt`
+  double* tgt_pred;
+  // obstacle motion (nmpc_set_obstacle_motion, fused calls only): after the shift the epilogue advances the per-instance table
+  // obs_move [B][n_obs][3] (the same array as `obs`) by T * obs_vel [B][n_obs][2]
+  double* obs_move; const double* obs_vel;
+  int32_t* iters_keep;              // handle-owned copy of iters[] (drives the next call's fetch order)
   const int32_t* order;              // optional processing order (longest-first scheduling); NULL = 0..B-1
   int* counter;                      // work queue of THIS call
   // Bookkeeping for the NEXT call on the same handle is done by this launch, so that a solve is ONE launch: the first
@@ -227,12 +233,23 @@ __device__ __forceinline__ void stash_box_states(const double* X, int lane) {
   } while (0)
 
 // target position seen by this lane's stage: the reference keeps (x_t, y_t) = p[8:10] over the horizon
-// (NMPC_TT.py:219-220); with a predicted trajectory (nmpc_set_target_trajectory) stage k has its own
+// (NMPC_TT.py:219-220); with a predicted trajectory (nmpc_set_target_trajectory, NMPC_PREDICT_TARGET) stage k has its own.
+// Coherent loads: with NMPC_PREDICT_TARGET the kernel itself has written the trajectory (ph_predict).
 template <class L>
 __device__ __forceinline__ double2 stage_target(const SolveArgs& A, int lane) {
   if (!A.tgt || lane >= L::N) return make_double2(PAR(8), PAR(9));
   const double* t = A.tgt + ((size_t)PAR(NPAR + 2) * L::N + lane) * 2;
-  return make_double2(__ldg(t), __ldg(t + 1));
+  return make_double2(__ldcg(t), __ldcg(t + 1));
+}
+
+// the target's (v, omega) of closed-loop step `step` of this call (fused calls): the caller's target_vw, or the device
+// schedule sched_table[row][min(sched_iter + step + phase, len - 1)] -- the scripts' `con_t` keyed on mpc_iter
+__device__ __forceinline__ double2 target_input(const SolveArgs& A, int b, int step) {
+  if (A.step_vw) return make_double2(__ldg(A.step_vw + 2 * (size_t)b), __ldg(A.step_vw + 2 * (size_t)b + 1));
+  const int row = A.sched_id ? __ldg(A.sched_id + b) : 0, ph = A.sched_phase ? __ldg(A.sched_phase + b) : 0;
+  const int at = min(A.sched_iter + step + ph, A.sched_len - 1);
+  const double* e = A.sched_table + ((size_t)row * A.sched_len + at) * 2;
+  return make_double2(__ldg(e), __ldg(e + 1));
 }
 
 // stage cost of this lane's stage (value / value + gradient + Hessian over (x, y, z, X5, X6, X7)) for the model of the layout
@@ -269,10 +286,37 @@ __device__ __forceinline__ RestoRow resto_row(const SolveArgs& A, const double* 
   return q;
 }
 
-// ---------------------------------------------------------------------------------------------------
-// load one instance: p -> PAR, warm start -> LV_U, obstacle table, unit scaling
+// NMPC_PREDICT_TARGET (end of ph_load): the target's own Euler prediction over the horizon from the target
+// block (x_t, y_t, th_t) of p and this step's (v, omega) into A.tgt_pred, in exactly the arithmetic of
+// ClosedLoop.target_prediction() (bit-identical; no FMA contraction, sin and cos called separately):
+//   th_k = th_t + (T w) k,   s_k = (T v) (cos th_k, sin th_k),   pos_k = (x_t, y_t) + (((0 + s_0) + s_1) + ... + s_{k-1})
+// The prefix sum runs left to right, as torch's cumsum over a non-innermost dimension does.  A function of its own: inlined,
+// the trigonometric reduction would add to ph_load's registers.
 template <class L>
-__device__ __noinline__ void ph_load(const SolveArgs& A, int b, int lane) {
+__device__ __noinline__ void ph_predict(const SolveArgs& A, int b, int lane, int step) {
+  const double* pt = A.p + (size_t)b * L::NPA + L::NPA - 3;     // (L2 path: a free-running call re-reads what its own epilogue wrote)
+  const double xt = __ldcg(pt), yt = __ldcg(pt + 1), tht = __ldcg(pt + 2);
+  const double2 vw = target_input(A, b, step);
+  const double Tv = __dmul_rn(A.pr.T, vw.x), Tw = __dmul_rn(A.pr.T, vw.y);
+  const double th = __dadd_rn(tht, __dmul_rn(Tw, (double)lane));
+  const double sx = __dmul_rn(Tv, cos(th)), sy = __dmul_rn(Tv, sin(th));
+  double ax = 0.0, ay = 0.0;
+#pragma unroll 1
+  for (int j = 0; j < L::N - 1; ++j) {
+    const double qx = __shfl_sync(FULL, sx, j), qy = __shfl_sync(FULL, sy, j);
+    if (j < lane) { ax = __dadd_rn(ax, qx); ay = __dadd_rn(ay, qy); }
+  }
+  if (lane < L::N) {
+    double* t = A.tgt_pred + ((size_t)b * L::N + lane) * 2;
+    t[0] = __dadd_rn(xt, ax); t[1] = __dadd_rn(yt, ay);
+  }
+  __syncwarp();
+}
+
+// ---------------------------------------------------------------------------------------------------
+// load one instance: p -> PAR, warm start -> LV_U, obstacle table, unit scaling; the target prediction of step `step`
+template <class L>
+__device__ __noinline__ void ph_load(const SolveArgs& A, int b, int lane, int step) {
   if (L::MODEL) {      // p = [state(5); target(3)]: the camera states are zero
     if (lane < NPAR) PAR(lane) = lane < 5 ? __ldcg(A.p + (size_t)b * L::NPA + lane) : (lane < 8 ? 0.0 : __ldcg(A.p + (size_t)b * L::NPA + lane - 3));
   } else if (lane < NPAR) PAR(lane) = __ldcg(A.p + (size_t)b * NPAR + lane);      // (L2 path: a free-running call re-reads what its own epilogue wrote)
@@ -289,6 +333,7 @@ __device__ __noinline__ void ph_load(const SolveArgs& A, int b, int lane) {
     for (int r = 0; r < L::R; ++r) { RW(A_DC, r) = 1.0; RW(A_DS, r) = 0.0; }
   }
   __syncwarp();
+  if (A.tgt_pred) ph_predict<L>(A, b, lane, step);
 }
 
 // gradient-based scaling at the user's starting point (IPOPT nlp_scaling_method = gradient-based): returns df, sets DC
@@ -1142,16 +1187,19 @@ __device__ __noinline__ void ph_output(const SolveArgs& A, int b, int lane, doub
       if (lane == 0 && status != NMPC_SOLVE_SUCCEEDED) lx[0] = CUDART_NAN;
     }
     if (lane == 0) {
-      double tv, tw;
-      if (A.step_vw) { tv = __ldg(A.step_vw + 2 * (size_t)b); tw = __ldg(A.step_vw + 2 * (size_t)b + 1); }
-      else {
-        const int row = A.sched_id ? __ldg(A.sched_id + b) : 0, ph = A.sched_phase ? __ldg(A.sched_phase + b) : 0;
-        const int at = min(A.sched_iter + step + ph, A.sched_len - 1);
-        const double* e = A.sched_table + ((size_t)row * A.sched_len + at) * 2;
-        tv = __ldg(e); tw = __ldg(e + 1);
-      }
-      closed_loop_shift_model(L::MODEL, pr.T, pr.hv, pr.hh, A.step_p + (size_t)b * L::NPA, u, tv, tw,
+      const double2 vw = target_input(A, b, step);
+      closed_loop_shift_model(L::MODEL, pr.T, pr.hv, pr.hh, A.step_p + (size_t)b * L::NPA, u, vw.x, vw.y,
                         A.step_fov ? A.step_fov + 2 * (size_t)b : nullptr, A.step_err ? A.step_err + b : nullptr);
+    }
+    if (A.obs_move) {     // moving obstacles: o += T v from the copy this solve used (the rows g above saw the positions before the move),
+                          // rounded as the torch update o + (T v); the lane mapping is ph_load's, so the next step of a free-running
+                          // call reads its own write
+      const double* vel = A.obs_vel + (size_t)b * 2 * L::NOBS;
+      double* om = A.obs_move + (size_t)b * 3 * L::NOBS;
+      for (int i = lane; i < 3 * L::NOBS; i += 32) {
+        const int j = i / 3, c = i - 3 * j;
+        if (c < 2) om[i] = __dadd_rn(smem[L::OBS0 + i], __dmul_rn(pr.T, __ldg(vel + 2 * j + c)));
+      }
     }
   }
   __syncwarp();
@@ -1494,7 +1542,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
   const double T = pr.T;
   const bool pair = L::PAIR && A.pair_trials;
 
-  ph_load<L>(A, b, lane);
+  ph_load<L>(A, b, lane, step);
   double df = 1.0;
   if (o.scaling) {
     df = ph_scaling<L>(A, lane);

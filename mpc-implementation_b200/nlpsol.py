@@ -278,6 +278,34 @@ class Solver:
                 L.nmpc_set_weights(self._h, None)
         return cm()
 
+    def _motion(self, obstacles, obstacle_vel, B):
+        """Context manager: nmpc_set_obstacle_motion for the duration of one fused call (the kernel moves `obstacles` in place)."""
+        import contextlib
+        if obstacle_vel is None:
+            return contextlib.nullcontext()
+        if self.n_obs == 0:
+            raise ValueError("solver: obstacle_vel given, but this solver has no obstacle rows")
+        if not (_is_cuda_tensor(obstacles) and obstacles.dtype == torch.float64 and obstacles.is_contiguous()
+                and tuple(obstacles.shape) == (B, self.n_obs, 3)):
+            raise ValueError(f"solver: moving obstacles (obstacle_vel) need obstacles as a contiguous CUDA float64 [B, n_obs, 3] = "
+                             f"[{B}, {self.n_obs}, 3] tensor, which is moved in place")
+        if not (_is_cuda_tensor(obstacle_vel) and obstacle_vel.dtype == torch.float64 and tuple(obstacle_vel.shape) == (B, self.n_obs, 2)):
+            raise ValueError(f"solver: obstacle_vel must be a CUDA float64 [B, n_obs, 2] = [{B}, {self.n_obs}, 2] tensor")
+        if obstacle_vel.device != obstacles.device:
+            raise ValueError("solver: obstacles and obstacle_vel must be on the same device")
+        vel = obstacle_vel.contiguous()
+        L = _ffi.lib()
+
+        @contextlib.contextmanager
+        def cm():
+            _ffi.check(L.nmpc_set_obstacle_motion(self._h, obstacles.data_ptr(), vel.data_ptr()), "nmpc_set_obstacle_motion")
+            try:
+                yield
+            finally:
+                self._keep_motion = (obstacles, vel)     # the kernel reads the velocities and writes the field later
+                L.nmpc_set_obstacle_motion(self._h, None, None)
+        return cm()
+
     def _obst(self, obstacles, B):
         if obstacles is None:
             return self.obstacles, 0
@@ -427,13 +455,21 @@ class Solver:
 
     # -- shift_timestep (NMPC_TT.py:13-30) on device --------------------------------------------
     def solve_and_step(self, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre=None, err_accum=None, obstacles=None,
-                       want_x: bool = False, weights=None, target_traj=None):
+                       want_x: bool = False, weights=None, target_traj=None, predict_target: bool = False, obstacle_vel=None):
+        """predict_target: every solve uses the target's own Euler prediction over the horizon, made in the kernel from p's
+        target block and this step's target input (NMPC_PREDICT_TARGET; the arithmetic of ClosedLoop.target_prediction()).
+        obstacle_vel [B, n_obs, 2] (CUDA float64): obstacles, then a CUDA float64 [B, n_obs, 3] tensor, is moved in place by
+        T * obstacle_vel after the solve (nmpc_set_obstacle_motion); this step's constraint rows use the positions before."""
+        if predict_target and target_traj is not None:
+            raise ValueError("solver: predict_target and target_traj exclude each other (the prediction replaces the trajectory)")
         if weights is not None or target_traj is not None:
             with self._weights(weights, p), self._traj(target_traj, p):
-                return self.solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x)
-        return self._solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x)
+                return self.solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x,
+                                           predict_target=predict_target, obstacle_vel=obstacle_vel)
+        with self._motion(obstacles, obstacle_vel, p.shape[0]):
+            return self._solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, predict_target)
 
-    def _solve_and_step(self, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x):
+    def _solve_and_step(self, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, predict_target=False):
         """One closed-loop step of B instances in ONE kernel launch (nmpc_solve_and_step): solves from the warm start
         u_warm with parameters p, then shifts p / u_warm in place (torch CUDA float64 tensors).  Returns dict(x, f)
         with x None unless want_x; status / iterations through stats()."""
@@ -448,6 +484,8 @@ class Solver:
         else:
             obs = obstacles.to(torch.float64).contiguous()
             flags = _ffi.NMPC_OBS_PER_INSTANCE if obs.numel() == 3 * self.n_obs * B and B > 1 else 0
+        if predict_target:
+            flags |= _ffi.NMPC_PREDICT_TARGET
         x = torch.empty((B, self.n_w), dtype=torch.float64, device=dev) if want_x else None
         f = torch.empty(B, dtype=torch.float64, device=dev)
         status = torch.empty(B, dtype=torch.int32, device=dev)
@@ -464,11 +502,18 @@ class Solver:
         return dict(x=x, f=f, g=None, lam_x=None, lam_g=None)
 
     def run_closed_loop(self, steps: int, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre=None, err_accum=None,
-                        obstacles=None, want_x: bool = False, log: bool = True):
+                        obstacles=None, want_x: bool = False, log: bool = True, predict_target: bool = False, obstacle_vel=None):
         """`steps` closed-loop steps of every instance in ONE launch, without a batch-wide barrier between the steps
         (nmpc_run_closed_loop; the scripts' `while mpc_iter < sim_time / T` loop, NMPC_TT.py:346-402).  p / u_warm are advanced in
         place.  Returns dict(x, f of the last step, status_log / iters_log [steps, B] when log, converged [B] = number of
-        converged solves per instance); stats() reports the last step.  Bit-identical to `steps` solve_and_step calls."""
+        converged solves per instance); stats() reports the last step.  Bit-identical to `steps` solve_and_step calls, also
+        with predict_target / obstacle_vel (as in solve_and_step: the prediction is made every step, the obstacles move every step)."""
+        with self._motion(obstacles, obstacle_vel, p.shape[0]):
+            return self._run_closed_loop(steps, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, log,
+                                         predict_target)
+
+    def _run_closed_loop(self, steps, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, log,
+                         predict_target):
         L = _ffi.lib()
         dev = p.device
         B = p.shape[0]
@@ -480,6 +525,8 @@ class Solver:
         else:
             obs = obstacles.to(torch.float64).contiguous()
             flags = _ffi.NMPC_OBS_PER_INSTANCE if obs.numel() == 3 * self.n_obs * B and B > 1 else 0
+        if predict_target:
+            flags |= _ffi.NMPC_PREDICT_TARGET
         if target_vw is None and getattr(self, "_sched", None) is None:
             raise ValueError("solver: target_vw is None and no schedule is set (set_schedule)")
         x = torch.empty((B, self.n_w), dtype=torch.float64, device=dev) if want_x else None
