@@ -253,8 +253,6 @@ struct nmpc_handle {
   int32_t *d_order[2], *d_keep_iters; int order_cap, prev_B, auto_order, parity, have_order; const int32_t* order_next;
   const double *weights, *tgt;
   double *ws_lamx, *ws_lamg;       // nmpc_set_warm_start
-  int run_steps; int32_t *run_status_log, *run_iters_log, *run_conv;   // set for the duration of nmpc_run_closed_loop
-  double *fuse_p, *fuse_u, *fuse_fov, *fuse_err; const double* fuse_vw;   // set for the duration of nmpc_solve_and_step
   const double* sched_table; const int32_t *sched_id, *sched_phase; int sched_rows, sched_len, sched_iter;   // nmpc_set_schedule
   double* d_tgt_pred; int tgt_pred_cap;        // NMPC_PREDICT_TARGET: the trajectory the kernel predicts, [tgt_pred_cap][N][2]
   double* move_obs; const double* move_vel;    // nmpc_set_obstacle_motion
@@ -269,6 +267,131 @@ struct nmpc_handle {
   double* dbg; int dbg_rows;
   int fill, pair_trials;
 };
+
+// The refusals several entry points share, each naming `fn`, the public function the caller called.  Those in `which` are
+// checked in this order; an entry point that makes them at different places of its own order calls this once per place.
+enum : unsigned { NULL_HANDLE = 1u, NO_OBSTACLES = 2u, PREDICT_WITHOUT_VW = 4u, PREDICT_WITH_TRAJECTORY = 8u };
+static int refused(const nmpc_handle* h, const char* fn, unsigned which, const double* obst = nullptr, uint32_t flags = 0) {
+  if ((which & NULL_HANDLE) && !h) return fail(std::string(fn) + ": null handle");
+  if ((which & NO_OBSTACLES) && h->pr.n_obs > 0 && !obst) return fail(std::string(fn) + ": obstacle table required");
+  if ((which & PREDICT_WITHOUT_VW) && (flags & NMPC_PREDICT_TARGET))
+    return fail(std::string(fn) + ": NMPC_PREDICT_TARGET needs the target's (v, omega) of the step: use nmpc_solve_and_step or nmpc_run_closed_loop");
+  if ((which & PREDICT_WITH_TRAJECTORY) && (flags & NMPC_PREDICT_TARGET) && h->tgt)
+    return fail(std::string(fn) + ": NMPC_PREDICT_TARGET and a target trajectory (nmpc_set_target_trajectory) exclude each other");
+  return 0;
+}
+
+// What every solve entry point passes on from its caller, in the order of SolveArgs; the rest starts null / zero.
+static SolveArgs solve_args(int32_t B, const double* p, const double* x0, const double* lbx, const double* ubx, const double* lbg, const double* ubg,
+                            const double* obst, uint32_t flags, double* x, double* f, double* g, double* lam_x, double* lam_g, int32_t* status, int32_t* iters) {
+  return SolveArgs{{}, {}, B, p, x0, lbx, ubx, lbg, ubg, obst, (flags & NMPC_OBS_PER_INSTANCE) ? 1 : 0, x, f, g, lam_x, lam_g, status, iters};
+}
+
+// One launch of the IPM kernel for the entry point `fn`, after nmpc_solve's checks and, when `fused`, those of the fused calls
+// before them.  A holds what the caller passed (step_* for the fused calls, run_* for the free-running one); the rest is handle state.
+static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream_t s, const char* fn, bool fused = false) {
+  const std::string f(fn);
+  if (refused(h, fn, NULL_HANDLE)) return 1;
+  if (fused) {
+    if (!A.step_p || !A.step_u) return fail(f + ": null required pointer");
+    if (!A.step_vw && !h->sched_table) return fail(f + ": target_vw is NULL and no schedule is set (nmpc_set_schedule)");
+    if (A.step_err && !A.step_fov) return fail(f + ": err_accum needs fov_centre");
+    if (A.x == A.step_u) return fail(f + ": x must not alias u_warm (pass NULL if the solution itself is not needed)");
+    if (h->move_obs && A.obs != h->move_obs) return fail(f + ": obstacle motion is set (nmpc_set_obstacle_motion): obst must be the registered field");
+    if (h->move_obs && A.B > 1 && !(flags & NMPC_OBS_PER_INSTANCE)) return fail(f + ": obstacle motion needs a per-instance obstacle field (NMPC_OBS_PER_INSTANCE)");
+  }
+  A.run_steps = A.run_steps > 1 ? A.run_steps : 1;
+  const int sched_steps = fused && !A.step_vw ? A.run_steps : 0;      // the schedule's step counter (mpc_iter) advances, B <= 0 included
+  const int B = A.B;
+  if (B <= 0) { h->sched_iter += sched_steps; return 0; }
+  if (!A.p || !A.x0 || !A.lbx || !A.ubx || !A.lbg || !A.ubg || (!A.x && !fused)) return fail(f + ": null required pointer");
+  if (refused(h, fn, NO_OBSTACLES | (fused ? PREDICT_WITH_TRAJECTORY : PREDICT_WITHOUT_VW), A.obs, flags)) return 1;
+  CK(cudaSetDevice(h->device));
+  const bool predict = (flags & NMPC_PREDICT_TARGET) != 0;
+  A.pr = h->pr; A.o = h->opt;
+  const int par = h->parity;            // flipped only after a successful launch (see below)
+  A.counter = h->d_counter + par; A.counter_next = h->d_counter + (par ^ 1);
+  A.done = h->d_counter + 2 + par; A.done_next = h->d_counter + 2 + (par ^ 1);
+  A.stats = h->d_stats + NSTAT * par; A.stats_next = h->d_stats + NSTAT * (par ^ 1);
+  A.ric = h->d_ric; A.ric_stride = h->ric_stride; A.ricmap = h->d_ricmap;
+  A.cold = h->d_cold; A.cold_stride = h->cold_stride;
+  A.dbg = h->dbg; A.dbg_rows = h->dbg_rows;
+  if (B > h->order_cap) {     // (re)allocate the scheduling buffers; the previous counts are dropped
+    CK(cudaStreamSynchronize(s));
+    for (int i = 0; i < 2; ++i) { if (h->d_order[i]) cudaFree(h->d_order[i]); h->d_order[i] = nullptr; }
+    if (h->d_keep_iters) cudaFree(h->d_keep_iters);
+    h->d_keep_iters = nullptr; h->order_cap = 0; h->prev_B = 0; h->have_order = 0;
+    // (a failure here returns before anything of this call was enqueued: parity and counters are untouched, the
+    //  partially allocated buffers are freed by the next attempt or by nmpc_destroy)
+    CK(cudaMalloc(&h->d_order[0], sizeof(int32_t) * B)); CK(cudaMalloc(&h->d_order[1], sizeof(int32_t) * B));
+    CK(cudaMalloc(&h->d_keep_iters, sizeof(int32_t) * B));
+    h->order_cap = B;
+  }
+  if (predict && B > h->tgt_pred_cap) {     // the predicted trajectories, grown like the scheduling buffers
+    CK(cudaStreamSynchronize(s));
+    if (h->d_tgt_pred) cudaFree(h->d_tgt_pred);
+    h->d_tgt_pred = nullptr; h->tgt_pred_cap = 0;
+    CK(cudaMalloc(&h->d_tgt_pred, sizeof(double) * 2 * (size_t)h->pr.N * B));
+    h->tgt_pred_cap = B;
+  }
+  A.iters_keep = h->d_keep_iters;
+  A.sched_table = h->sched_table; A.sched_id = h->sched_id; A.sched_phase = h->sched_phase; A.sched_len = h->sched_len; A.sched_iter = h->sched_iter;
+  A.tgt_pred = predict ? h->d_tgt_pred : nullptr;
+  A.tgt = predict ? h->d_tgt_pred : h->tgt;
+  A.obs_move = A.step_p ? h->move_obs : nullptr; A.obs_vel = h->move_vel;
+  A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && A.step_p) ? 1 : 0;
+  A.weights = h->weights;
+  A.pair_trials = h->pair_trials;
+  // fetch order: explicit (nmpc_set_order) > the order the previous call on this handle prepared for the same B > natural
+  A.order = h->order_next; h->order_next = nullptr;
+  if (!A.order && h->auto_order && h->have_order && h->prev_B == B) A.order = h->d_order[par];
+  A.order_out = h->auto_order ? h->d_order[par ^ 1] : nullptr;       // ... and this call prepares the next one's
+  // Grid: one block per SM at most; with `fill` > 1 a small batch is packed onto fewer SMs (fill instances per warp,
+  // refilled from the queue) so that concurrent solves of other handles find free SMs instead of SMs held by blocks
+  // whose eight warps wait for one straggler.
+  int blocks = B < h->max_blocks ? B : h->max_blocks;
+  if (h->fill > 1) {
+    const int packed = (B + h->warps_per_block * h->fill - 1) / (h->warps_per_block * h->fill);
+    if (packed < blocks) blocks = packed < 1 ? 1 : packed;
+  }
+  if (const int rc = h->inst->launch(A, blocks, h->smem_bytes, s)) {
+    // The kernel that would have reset the NEXT call's queue / done / work counters did not run: keep the parity (the
+    // next call reuses THIS call's buffers) and put them back to their clean state, so that a later call can never
+    // start from a stale queue counter and return without having written its outputs.
+    cudaMemsetAsync(h->d_counter, 0, 4 * sizeof(int), s);
+    cudaMemsetAsync(h->d_stats, 0, 2 * NSTAT * sizeof(unsigned long long), s);
+    h->have_order = 0; h->prev_B = 0;
+    return fail(f + ": launch failed: " + cudaGetErrorString((cudaError_t)rc));
+  }
+  // the launch is enqueued: it owns buffer set `par` and prepares set `par ^ 1` for the next call
+  h->parity = par ^ 1;
+  h->stats_last = h->d_stats + NSTAT * par;
+  h->have_order = h->auto_order;
+  h->launches = 1;
+  h->prev_B = B;
+  h->last_stream = s;
+  h->sched_iter += sched_steps;
+  return 0;
+}
+
+// nmpc_eval and nmpc_lam_p: A holds the call's arrays; `missing` says that one the entry point requires is NULL.
+static int launch_eval(nmpc_handle* h, const char* fn, EvalArgs A, uint32_t flags, bool missing, void* cuda_stream) {
+  if (refused(h, fn, NULL_HANDLE)) return 1;
+  if (A.B <= 0) return 0;
+  if (refused(h, fn, PREDICT_WITHOUT_VW, nullptr, flags)) return 1;
+  if (missing) return fail(std::string(fn) + ": null required pointer");
+  if (refused(h, fn, NO_OBSTACLES, A.obs)) return 1;
+  if (A.jtv && !A.lam) return fail(std::string(fn) + ": jtv needs lam");
+  if (A.hv && !A.v) return fail(std::string(fn) + ": hv needs v");
+  CK(cudaSetDevice(h->device));
+  A.pr = h->pr; A.obs_per_instance = (flags & NMPC_OBS_PER_INSTANCE) ? 1 : 0;
+  A.weights = h->weights; A.tgt = h->tgt;
+  const int warps = 4;
+  nmpc_eval_kernel<<<(A.B + warps - 1) / warps, warps * 32, 0, (cudaStream_t)cuda_stream>>>(A);
+  CK(cudaGetLastError());
+  h->last_stream = (cudaStream_t)cuda_stream; h->launches = 1;
+  return 0;
+}
 
 extern "C" {
 
@@ -369,88 +492,8 @@ int nmpc_solve(nmpc_handle* h, int32_t B, const double* p, const double* x0,
                const double* obst, uint32_t flags,
                double* x, double* f, double* g, double* lam_x, double* lam_g,
                int32_t* status, int32_t* iters, void* cuda_stream) {
-  if (!h) return fail("nmpc_solve: null handle");
-  if (B <= 0) return 0;
-  if (!p || !x0 || !lbx || !ubx || !lbg || !ubg || (!x && !h->fuse_p)) return fail("nmpc_solve: null required pointer");
-  if (h->pr.n_obs > 0 && !obst) return fail("nmpc_solve: obstacle table required");
-  const bool predict = (flags & NMPC_PREDICT_TARGET) != 0;
-  if (predict && !h->fuse_p)
-    return fail("nmpc_solve: NMPC_PREDICT_TARGET needs the target's (v, omega) of the step: use nmpc_solve_and_step or nmpc_run_closed_loop");
-  if (predict && h->tgt) return fail("nmpc_solve: NMPC_PREDICT_TARGET and a target trajectory (nmpc_set_target_trajectory) exclude each other");
-  CK(cudaSetDevice(h->device));
-  cudaStream_t s = (cudaStream_t)cuda_stream;
-  SolveArgs A;
-  A.pr = h->pr; A.o = h->opt; A.B = B;
-  A.p = p; A.x0 = x0; A.lbx = lbx; A.ubx = ubx; A.lbg = lbg; A.ubg = ubg; A.obs = obst;
-  A.obs_per_instance = (flags & NMPC_OBS_PER_INSTANCE) ? 1 : 0;
-  A.x = x; A.f = f; A.g = g; A.lam_x = lam_x; A.lam_g = lam_g; A.status = status; A.iters = iters;
-  const int par = h->parity;            // flipped only after a successful launch (see below)
-  A.counter = h->d_counter + par; A.counter_next = h->d_counter + (par ^ 1);
-  A.done = h->d_counter + 2 + par; A.done_next = h->d_counter + 2 + (par ^ 1);
-  A.stats = h->d_stats + NSTAT * par; A.stats_next = h->d_stats + NSTAT * (par ^ 1);
-  A.ric = h->d_ric; A.ric_stride = h->ric_stride; A.ricmap = h->d_ricmap;
-  A.cold = h->d_cold; A.cold_stride = h->cold_stride;
-  A.dbg = h->dbg; A.dbg_rows = h->dbg_rows;
-  if (B > h->order_cap) {     // (re)allocate the scheduling buffers; the previous counts are dropped
-    CK(cudaStreamSynchronize(s));
-    for (int i = 0; i < 2; ++i) { if (h->d_order[i]) cudaFree(h->d_order[i]); h->d_order[i] = nullptr; }
-    if (h->d_keep_iters) cudaFree(h->d_keep_iters);
-    h->d_keep_iters = nullptr; h->order_cap = 0; h->prev_B = 0; h->have_order = 0;
-    // (a failure here returns before anything of this call was enqueued: parity and counters are untouched, the
-    //  partially allocated buffers are freed by the next attempt or by nmpc_destroy)
-    CK(cudaMalloc(&h->d_order[0], sizeof(int32_t) * B)); CK(cudaMalloc(&h->d_order[1], sizeof(int32_t) * B));
-    CK(cudaMalloc(&h->d_keep_iters, sizeof(int32_t) * B));
-    h->order_cap = B;
-  }
-  if (predict && B > h->tgt_pred_cap) {     // the predicted trajectories, grown like the scheduling buffers
-    CK(cudaStreamSynchronize(s));
-    if (h->d_tgt_pred) cudaFree(h->d_tgt_pred);
-    h->d_tgt_pred = nullptr; h->tgt_pred_cap = 0;
-    CK(cudaMalloc(&h->d_tgt_pred, sizeof(double) * 2 * (size_t)h->pr.N * B));
-    h->tgt_pred_cap = B;
-  }
-  A.iters_keep = h->d_keep_iters;
-  A.step_p = h->fuse_p; A.step_u = h->fuse_u; A.step_vw = h->fuse_vw; A.step_fov = h->fuse_fov; A.step_err = h->fuse_err;
-  A.sched_table = h->sched_table; A.sched_id = h->sched_id; A.sched_phase = h->sched_phase; A.sched_len = h->sched_len; A.sched_iter = h->sched_iter;
-  A.tgt_pred = predict ? h->d_tgt_pred : nullptr;
-  A.tgt = predict ? h->d_tgt_pred : h->tgt;
-  A.obs_move = h->fuse_p ? h->move_obs : nullptr; A.obs_vel = h->move_vel;
-  A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && h->fuse_p) ? 1 : 0;
-  A.run_steps = h->run_steps > 1 ? h->run_steps : 1; A.status_log = h->run_status_log; A.iters_log = h->run_iters_log; A.conv_count = h->run_conv;
-  A.weights = h->weights;
-  A.pair_trials = h->pair_trials;
-  // fetch order: explicit (nmpc_set_order) > the order the previous call on this handle prepared for the same B > natural
-  A.order = h->order_next; h->order_next = nullptr;
-  if (!A.order && h->auto_order && h->have_order && h->prev_B == B) A.order = h->d_order[par];
-  A.order_out = h->auto_order ? h->d_order[par ^ 1] : nullptr;       // ... and this call prepares the next one's
-  // Grid: one block per SM at most; with `fill` > 1 a small batch is packed onto fewer SMs (fill instances per warp,
-  // refilled from the queue) so that concurrent solves of other handles find free SMs instead of SMs held by blocks
-  // whose eight warps wait for one straggler.
-  int blocks = B < h->max_blocks ? B : h->max_blocks;
-  if (h->fill > 1) {
-    const int packed = (B + h->warps_per_block * h->fill - 1) / (h->warps_per_block * h->fill);
-    if (packed < blocks) blocks = packed < 1 ? 1 : packed;
-  }
-  {
-    const int rc = h->inst->launch(A, blocks, h->smem_bytes, s);
-    if (rc != 0) {
-      // The kernel that would have reset the NEXT call's queue / done / work counters did not run: keep the parity (the
-      // next call reuses THIS call's buffers) and put them back to their clean state, so that a later call can never
-      // start from a stale queue counter and return without having written its outputs.
-      cudaMemsetAsync(h->d_counter, 0, 4 * sizeof(int), s);
-      cudaMemsetAsync(h->d_stats, 0, 2 * NSTAT * sizeof(unsigned long long), s);
-      h->have_order = 0; h->prev_B = 0;
-      return fail(std::string("nmpc_solve: launch failed: ") + cudaGetErrorString((cudaError_t)rc));
-    }
-  }
-  // the launch is enqueued: it owns buffer set `par` and prepares set `par ^ 1` for the next call
-  h->parity = par ^ 1;
-  h->stats_last = h->d_stats + NSTAT * par;
-  h->have_order = h->auto_order;
-  h->launches = 1;
-  h->prev_B = B;
-  h->last_stream = s;
-  return 0;
+  SolveArgs A = solve_args(B, p, x0, lbx, ubx, lbg, ubg, obst, flags, x, f, g, lam_x, lam_g, status, iters);
+  return launch_solve(h, A, flags, (cudaStream_t)cuda_stream, "nmpc_solve");
 }
 
 int nmpc_solve_and_step(nmpc_handle* h, int32_t B, double* p, double* u_warm,
@@ -458,20 +501,9 @@ int nmpc_solve_and_step(nmpc_handle* h, int32_t B, double* p, double* u_warm,
                         const double* obst, uint32_t flags, const double* target_vw,
                         double* x, double* f, double* fov_centre, double* err_accum,
                         int32_t* status, int32_t* iters, void* cuda_stream) {
-  if (!h) return fail("nmpc_solve_and_step: null handle");
-  if (!p || !u_warm) return fail("nmpc_solve_and_step: null required pointer");
-  if (!target_vw && !h->sched_table) return fail("nmpc_solve_and_step: target_vw is NULL and no schedule is set (nmpc_set_schedule)");
-  if (err_accum && !fov_centre) return fail("nmpc_solve_and_step: err_accum needs fov_centre");
-  if (x == u_warm) return fail("nmpc_solve_and_step: x must not alias u_warm (pass NULL if the solution itself is not needed)");
-  if (h->move_obs && obst != h->move_obs)
-    return fail("nmpc_solve_and_step: obstacle motion is set (nmpc_set_obstacle_motion): obst must be the registered field");
-  if (h->move_obs && B > 1 && !(flags & NMPC_OBS_PER_INSTANCE))
-    return fail("nmpc_solve_and_step: obstacle motion needs a per-instance obstacle field (NMPC_OBS_PER_INSTANCE)");
-  h->fuse_p = p; h->fuse_u = u_warm; h->fuse_vw = target_vw; h->fuse_fov = fov_centre; h->fuse_err = err_accum;
-  const int rc = nmpc_solve(h, B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, x, f, nullptr, nullptr, nullptr, status, iters, cuda_stream);
-  h->fuse_p = nullptr; h->fuse_u = nullptr; h->fuse_vw = nullptr; h->fuse_fov = nullptr; h->fuse_err = nullptr;
-  if (rc == 0 && !target_vw) ++h->sched_iter;        // the schedule is keyed on the number of closed-loop steps taken (mpc_iter)
-  return rc;
+  SolveArgs A = solve_args(B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, x, f, nullptr, nullptr, nullptr, status, iters);
+  A.step_p = p; A.step_u = u_warm; A.step_vw = target_vw; A.step_fov = fov_centre; A.step_err = err_accum;
+  return launch_solve(h, A, flags, (cudaStream_t)cuda_stream, "nmpc_solve_and_step", true);
 }
 
 int nmpc_run_closed_loop(nmpc_handle* h, int32_t B, int32_t steps, double* p, double* u_warm,
@@ -479,17 +511,14 @@ int nmpc_run_closed_loop(nmpc_handle* h, int32_t B, int32_t steps, double* p, do
                          const double* obst, uint32_t flags, const double* target_vw,
                          double* x, double* f, double* fov_centre, double* err_accum,
                          int32_t* status_log, int32_t* iters_log, int32_t* converged, void* cuda_stream) {
-  if (!h) return fail("nmpc_run_closed_loop: null handle");
+  if (refused(h, "nmpc_run_closed_loop", NULL_HANDLE)) return 1;
   if (steps < 1) return fail("nmpc_run_closed_loop: steps must be >= 1");
   if (h->tgt) return fail("nmpc_run_closed_loop: a caller-given target trajectory (nmpc_set_target_trajectory) needs the step-by-step calls; "
                           "NMPC_PREDICT_TARGET predicts it on the device");
-  h->run_steps = steps; h->run_status_log = status_log; h->run_iters_log = iters_log; h->run_conv = converged;
-  const int sched0 = h->sched_iter;
-  const int rc = nmpc_solve_and_step(h, B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, target_vw, x, f, fov_centre, err_accum,
-                                     nullptr, nullptr, cuda_stream);
-  h->run_steps = 0; h->run_status_log = nullptr; h->run_iters_log = nullptr; h->run_conv = nullptr;
-  if (rc == 0 && !target_vw) h->sched_iter = sched0 + steps;
-  return rc;
+  SolveArgs A = solve_args(B, p, u_warm, lbx, ubx, lbg, ubg, obst, flags, x, f, nullptr, nullptr, nullptr, nullptr, nullptr);
+  A.step_p = p; A.step_u = u_warm; A.step_vw = target_vw; A.step_fov = fov_centre; A.step_err = err_accum;
+  A.run_steps = steps; A.status_log = status_log; A.iters_log = iters_log; A.conv_count = converged;
+  return launch_solve(h, A, flags, (cudaStream_t)cuda_stream, "nmpc_run_closed_loop", true);
 }
 
 int nmpc_solve_host(nmpc_handle* h, int32_t B, const double* p, const double* x0,
@@ -522,9 +551,9 @@ int nmpc_solve_host_async(nmpc_handle* h, int32_t B, const double* p, const doub
                           const double* obst, uint32_t flags,
                           double* x, double* f, double* g, double* lam_x, double* lam_g,
                           int32_t* status, int32_t* iters) {
-  if (!h) return fail("nmpc_solve_host: null handle");
+  if (refused(h, "nmpc_solve_host", NULL_HANDLE)) return 1;
   if (B <= 0) return 0;
-  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_solve_host: NMPC_PREDICT_TARGET needs the target's (v, omega): use nmpc_solve_and_step or nmpc_run_closed_loop");
+  if (refused(h, "nmpc_solve_host", PREDICT_WITHOUT_VW, nullptr, flags)) return 1;
   if (B > h->spec.max_batch) return fail("nmpc_solve_host: B exceeds spec.max_batch");
   CK(cudaSetDevice(h->device));
   cudaStream_t s = h->own_stream;
@@ -537,10 +566,9 @@ int nmpc_solve_host_async(nmpc_handle* h, int32_t B, const double* p, const doub
   CK(cudaMemcpyAsync(h->d_lbg, lbg, sizeof(double) * ng, cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(h->d_ubg, ubg, sizeof(double) * ng, cudaMemcpyHostToDevice, s));
   if (nobs) CK(cudaMemcpyAsync(h->d_obs, obst, sizeof(double) * nobs, cudaMemcpyHostToDevice, s));
-  int rc = nmpc_solve(h, B, h->d_p, h->d_x0, h->d_lbx, h->d_ubx, h->d_lbg, h->d_ubg, h->d_obs, flags,
-                      h->d_x, h->d_f, g ? h->d_g : nullptr, lam_x ? h->d_lamx : nullptr, lam_g ? h->d_lamg : nullptr,
-                      h->d_status, h->d_iters, (void*)s);
-  if (rc) return rc;
+  SolveArgs A = solve_args(B, h->d_p, h->d_x0, h->d_lbx, h->d_ubx, h->d_lbg, h->d_ubg, h->d_obs, flags, h->d_x, h->d_f,
+                           g ? h->d_g : nullptr, lam_x ? h->d_lamx : nullptr, lam_g ? h->d_lamg : nullptr, h->d_status, h->d_iters);
+  if (const int rc = launch_solve(h, A, flags, s, "nmpc_solve_host")) return rc;
   CK(cudaMemcpyAsync(x, h->d_x, sizeof(double) * B * nw, cudaMemcpyDeviceToHost, s));
   if (f) CK(cudaMemcpyAsync(f, h->d_f, sizeof(double) * B, cudaMemcpyDeviceToHost, s));
   if (g) CK(cudaMemcpyAsync(g, h->d_g, sizeof(double) * B * ng, cudaMemcpyDeviceToHost, s));
@@ -554,42 +582,13 @@ int nmpc_solve_host_async(nmpc_handle* h, int32_t B, const double* p, const doub
 int nmpc_eval(nmpc_handle* h, int32_t B, const double* w, const double* p, const double* obst, uint32_t flags,
               double sigma, const double* lam, const double* v,
               double* f, double* g, double* grad_f, double* jtv, double* hv, void* cuda_stream) {
-  if (!h) return fail("nmpc_eval: null handle");
-  if (B <= 0) return 0;
-  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_eval: NMPC_PREDICT_TARGET is available in nmpc_solve_and_step and nmpc_run_closed_loop only");
-  if (!w || !p) return fail("nmpc_eval: null required pointer");
-  if (h->pr.n_obs > 0 && !obst) return fail("nmpc_eval: obstacle table required");
-  if (jtv && !lam) return fail("nmpc_eval: jtv needs lam");
-  if (hv && !v) return fail("nmpc_eval: hv needs v");
-  CK(cudaSetDevice(h->device));
-  EvalArgs A;
-  A.pr = h->pr; A.B = B; A.w = w; A.p = p; A.obs = obst; A.obs_per_instance = (flags & NMPC_OBS_PER_INSTANCE) ? 1 : 0;
-  A.weights = h->weights; A.tgt = h->tgt;
-  A.sigma = sigma; A.lam = lam; A.v = v; A.f = f; A.g = g; A.grad = grad_f; A.jtv = jtv; A.hv = hv; A.lamp = nullptr;
-  const int warps = 4;
-  nmpc_eval_kernel<<<(B + warps - 1) / warps, warps * 32, 0, (cudaStream_t)cuda_stream>>>(A);
-  CK(cudaGetLastError());
-  h->last_stream = (cudaStream_t)cuda_stream; h->launches = 1;
-  return 0;
+  return launch_eval(h, "nmpc_eval", EvalArgs{{}, B, w, p, obst, 0, nullptr, nullptr, sigma, lam, v, f, g, grad_f, jtv, hv}, flags, !w || !p, cuda_stream);
 }
 
 int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* obst, uint32_t flags,
                const double* lam_g, double* lam_p, void* cuda_stream) {
-  if (!h) return fail("nmpc_lam_p: null handle");
-  if (B <= 0) return 0;
-  if (flags & NMPC_PREDICT_TARGET) return fail("nmpc_lam_p: NMPC_PREDICT_TARGET is available in nmpc_solve_and_step and nmpc_run_closed_loop only");
-  if (!x_sol || !p || !lam_g || !lam_p) return fail("nmpc_lam_p: null required pointer");
-  if (h->pr.n_obs > 0 && !obst) return fail("nmpc_lam_p: obstacle table required");
-  CK(cudaSetDevice(h->device));
-  EvalArgs A;
-  A.pr = h->pr; A.B = B; A.w = x_sol; A.p = p; A.obs = obst; A.obs_per_instance = (flags & NMPC_OBS_PER_INSTANCE) ? 1 : 0;
-  A.weights = h->weights; A.tgt = h->tgt;
-  A.sigma = 1.0; A.lam = lam_g; A.v = nullptr; A.f = nullptr; A.g = nullptr; A.grad = nullptr; A.jtv = nullptr; A.hv = nullptr; A.lamp = lam_p;
-  const int warps = 4;
-  nmpc_eval_kernel<<<(B + warps - 1) / warps, warps * 32, 0, (cudaStream_t)cuda_stream>>>(A);
-  CK(cudaGetLastError());
-  h->last_stream = (cudaStream_t)cuda_stream; h->launches = 1;
-  return 0;
+  const EvalArgs A{{}, B, x_sol, p, obst, 0, nullptr, nullptr, 1.0, lam_g, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, lam_p};
+  return launch_eval(h, "nmpc_lam_p", A, flags, !x_sol || !p || !lam_g || !lam_p, cuda_stream);
 }
 
 int nmpc_step(nmpc_handle* h, int32_t B, const double* x_sol, double* p,

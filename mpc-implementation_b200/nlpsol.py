@@ -16,6 +16,7 @@ solver.stats() ('return_status', 'success', 'iter_count'), which the reference n
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 from typing import Any, Dict, Optional
 
@@ -104,6 +105,8 @@ class Solver:
         self._dev_cache: Dict[str, Any] = {}
         self._stats: Dict[str, Any] = {}
         self._warm = None
+        self._sched = None
+        self._held: Dict[str, Any] = {}      # tensors of the last call's per-call settings (_setting)
         self._create(max_batch)
 
     # -- handle management ---------------------------------------------------------------------
@@ -181,25 +184,23 @@ class Solver:
             raise ValueError("solver: p is required")
         if any(v is None for v in (lbx, ubx, lbg, ubg)):
             raise ValueError("solver: lbx, ubx, lbg, ubg are required (the reference passes all four)")
-        if self._d["warm"] and lam_x0 is not None and lam_g0 is not None:
-            if not _is_cuda_tensor(p):       # the multiplier guesses live on the device: take the device path, hand numpy back
-                dev = f"cuda:{self.device}"
-                t = lambda a, n: None if a is None else torch.as_tensor(np.asarray(a, dtype=np.float64), device=dev).reshape(-1, n)
-                B = self._batch_of(p)
-                out = self(x0=t(x0, self.n_w), p=t(p, self.n_p), lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg, obstacles=obstacles, want_g=want_g,
-                           want_lam=want_lam, order=order, weights=weights, target_traj=target_traj, lam_x0=lam_x0, lam_g0=lam_g0)
-                torch.cuda.synchronize()
-                self._stats = {k: v.cpu().numpy() for k, v in self._stats.items()}
-                return {k: (None if v is None else v.cpu().numpy()) for k, v in out.items()}
-            B = self._batch_of(p)
-            self.set_warm_start(torch.as_tensor(lam_x0, dtype=torch.float64, device=p.device).reshape(B, self.n_w),
-                                torch.as_tensor(lam_g0, dtype=torch.float64, device=p.device).reshape(B, self.n_g))
-            try:
-                return self(x0=x0, p=p, lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg, obstacles=obstacles, want_g=want_g, want_lam=want_lam,
-                            order=order, weights=weights, target_traj=target_traj)
-            finally:
-                self.set_warm_start(None, None)
-        with self._weights(weights, p), self._traj(target_traj, p):
+        warm = self._d["warm"] and lam_x0 is not None and lam_g0 is not None
+        if warm and not _is_cuda_tensor(p):       # the multiplier guesses live on the device: take the device path, hand numpy back
+            dev = f"cuda:{self.device}"
+            t = lambda a, n: None if a is None else torch.as_tensor(np.asarray(a, dtype=np.float64), device=dev).reshape(-1, n)
+            out = self(x0=t(x0, self.n_w), p=t(p, self.n_p), lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg, obstacles=obstacles, want_g=want_g,
+                       want_lam=want_lam, order=order, weights=weights, target_traj=target_traj, lam_x0=lam_x0, lam_g0=lam_g0)
+            torch.cuda.synchronize()
+            self._stats = {k: v.cpu().numpy() for k, v in self._stats.items()}
+            return {k: (None if v is None else v.cpu().numpy()) for k, v in out.items()}
+        B = self._batch_of(p)
+        if B > self._max_batch and not _is_cuda_tensor(p):     # spec.max_batch sizes the staging buffers of the host path only
+            self._create(max(B, 2 * self._max_batch))
+        with self._settings(B, weights, target_traj) as stack:
+            if warm:
+                self.set_warm_start(torch.as_tensor(lam_x0, dtype=torch.float64, device=p.device).reshape(B, self.n_w),
+                                    torch.as_tensor(lam_g0, dtype=torch.float64, device=p.device).reshape(B, self.n_g))
+                stack.callback(self.set_warm_start, None, None)
             if _is_cuda_tensor(p):
                 return self._call_device(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, order)
             return self._call_host(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking)
@@ -230,92 +231,82 @@ class Solver:
             return int(p.numel() // self.n_p)
         return int(np.asarray(p, dtype=np.float64).size // self.n_p)
 
-    def _traj(self, traj, p):
-        """Context manager: nmpc_set_target_trajectory for the duration of one call."""
-        import contextlib
-        if traj is None:
-            return contextlib.nullcontext()
-        B = self._batch_of(p)
-        t = torch.as_tensor(traj if _is_cuda_tensor(traj) else np.asarray(traj, dtype=np.float64),
-                            dtype=torch.float64, device=f"cuda:{self.device}").reshape(-1, self.N, 2).contiguous()
-        if t.shape[0] != B:
-            raise ValueError("solver: target_traj must be [B, N, 2]")
-        L = _ffi.lib()
+    @contextlib.contextmanager
+    def _setting(self, setter: str, *tensors):
+        """One per-call handle setting (nmpc_set_weights, nmpc_set_target_trajectory, nmpc_set_obstacle_motion) for the duration
+        of a call.  The tensors stay referenced afterwards: the kernel may read them later (device call, or blocking=False)."""
+        fn = getattr(_ffi.lib(), setter)
+        _ffi.check(fn(self._h, *(t.data_ptr() for t in tensors)), setter)
+        try:
+            yield
+        finally:
+            self._held[setter] = tensors
+            fn(self._h, *(None for _ in tensors))
 
-        @contextlib.contextmanager
-        def cm():
-            if B > self._max_batch:
-                self._create(max(B, 2 * self._max_batch))
-            _ffi.check(L.nmpc_set_target_trajectory(self._h, t.data_ptr()), "nmpc_set_target_trajectory")
-            try:
-                yield
-            finally:
-                self._keep_t = t            # the solve may still be in flight (device call, or blocking=False): hold the tensor
-                L.nmpc_set_target_trajectory(self._h, None)
-        return cm()
+    def _settings(self, B, weights=None, target_traj=None, obstacles=None, obstacle_vel=None) -> contextlib.ExitStack:
+        """The per-call settings of a call of B instances as one context, all validated before the first is applied.
+        obstacle_vel: the kernel moves `obstacles` in place after the solve (fused calls only)."""
+        rows = lambda a, *shape: torch.as_tensor(a if _is_cuda_tensor(a) else np.asarray(a, dtype=np.float64), dtype=torch.float64,
+                                                 device=f"cuda:{self.device}").reshape(-1, *shape).contiguous()
+        todo = []
+        if weights is not None:
+            w = rows(weights, 2)
+            if w.shape[0] != B:
+                raise ValueError("solver: weights must be [B, 2]")
+            todo.append(("nmpc_set_weights", w))
+        if target_traj is not None:
+            t = rows(target_traj, self.N, 2)
+            if t.shape[0] != B:
+                raise ValueError("solver: target_traj must be [B, N, 2]")
+            todo.append(("nmpc_set_target_trajectory", t))
+        if obstacle_vel is not None:
+            if self.n_obs == 0:
+                raise ValueError("solver: obstacle_vel given, but this solver has no obstacle rows")
+            if not (_is_cuda_tensor(obstacles) and obstacles.dtype == torch.float64 and obstacles.is_contiguous()
+                    and tuple(obstacles.shape) == (B, self.n_obs, 3)):
+                raise ValueError(f"solver: moving obstacles (obstacle_vel) need obstacles as a contiguous CUDA float64 [B, n_obs, 3] = "
+                                 f"[{B}, {self.n_obs}, 3] tensor, which is moved in place")
+            if not (_is_cuda_tensor(obstacle_vel) and obstacle_vel.dtype == torch.float64 and tuple(obstacle_vel.shape) == (B, self.n_obs, 2)):
+                raise ValueError(f"solver: obstacle_vel must be a CUDA float64 [B, n_obs, 2] = [{B}, {self.n_obs}, 2] tensor")
+            if obstacle_vel.device != obstacles.device:
+                raise ValueError("solver: obstacles and obstacle_vel must be on the same device")
+            todo.append(("nmpc_set_obstacle_motion", obstacles, obstacle_vel.contiguous()))
+        with contextlib.ExitStack() as stack:
+            for setter, *tensors in todo:
+                stack.enter_context(self._setting(setter, *tensors))
+            return stack.pop_all()
 
-    def _weights(self, weights, p):
-        """Context manager: nmpc_set_weights for the duration of one call."""
-        import contextlib
-        if weights is None:
-            return contextlib.nullcontext()
-        B = self._batch_of(p)
-        w = torch.as_tensor(weights if _is_cuda_tensor(weights) else np.asarray(weights, dtype=np.float64),
-                            dtype=torch.float64, device=f"cuda:{self.device}").reshape(-1, 2).contiguous()
-        if w.shape[0] != B:
-            raise ValueError("solver: weights must be [B, 2]")
-        L = _ffi.lib()
-
-        @contextlib.contextmanager
-        def cm():
-            if B > self._max_batch:          # grow first: the weights belong to the handle that runs the call
-                self._create(max(B, 2 * self._max_batch))
-            _ffi.check(L.nmpc_set_weights(self._h, w.data_ptr()), "nmpc_set_weights")
-            try:
-                yield
-            finally:
-                self._keep_w = w            # asynchronous call (device tensors, or blocking=False): the kernel reads w later
-                L.nmpc_set_weights(self._h, None)
-        return cm()
-
-    def _motion(self, obstacles, obstacle_vel, B):
-        """Context manager: nmpc_set_obstacle_motion for the duration of one fused call (the kernel moves `obstacles` in place)."""
-        import contextlib
-        if obstacle_vel is None:
-            return contextlib.nullcontext()
-        if self.n_obs == 0:
-            raise ValueError("solver: obstacle_vel given, but this solver has no obstacle rows")
-        if not (_is_cuda_tensor(obstacles) and obstacles.dtype == torch.float64 and obstacles.is_contiguous()
-                and tuple(obstacles.shape) == (B, self.n_obs, 3)):
-            raise ValueError(f"solver: moving obstacles (obstacle_vel) need obstacles as a contiguous CUDA float64 [B, n_obs, 3] = "
-                             f"[{B}, {self.n_obs}, 3] tensor, which is moved in place")
-        if not (_is_cuda_tensor(obstacle_vel) and obstacle_vel.dtype == torch.float64 and tuple(obstacle_vel.shape) == (B, self.n_obs, 2)):
-            raise ValueError(f"solver: obstacle_vel must be a CUDA float64 [B, n_obs, 2] = [{B}, {self.n_obs}, 2] tensor")
-        if obstacle_vel.device != obstacles.device:
-            raise ValueError("solver: obstacles and obstacle_vel must be on the same device")
-        vel = obstacle_vel.contiguous()
-        L = _ffi.lib()
-
-        @contextlib.contextmanager
-        def cm():
-            _ffi.check(L.nmpc_set_obstacle_motion(self._h, obstacles.data_ptr(), vel.data_ptr()), "nmpc_set_obstacle_motion")
-            try:
-                yield
-            finally:
-                self._keep_motion = (obstacles, vel)     # the kernel reads the velocities and writes the field later
-                L.nmpc_set_obstacle_motion(self._h, None, None)
-        return cm()
+    def _obs_flag(self, size: int, B: int) -> int:
+        """The obstacle shape rule: 3 n_obs entries are one table shared by the batch, 3 n_obs B entries one table per instance."""
+        if size == 3 * self.n_obs:
+            return 0
+        if size == 3 * self.n_obs * B:
+            return _ffi.NMPC_OBS_PER_INSTANCE
+        raise ValueError("solver: obstacles must be [n_obs,3] or [B,n_obs,3] of (cx, cy, r_uav + r_obs)")
 
     def _obst(self, obstacles, B):
         if obstacles is None:
             return self.obstacles, 0
         o = obstacles.detach().cpu().numpy() if (torch is not None and isinstance(obstacles, torch.Tensor)) else obstacles
         o = np.ascontiguousarray(np.asarray(o, dtype=np.float64))
-        if o.size == 3 * self.n_obs:
-            return o.reshape(self.n_obs, 3), 0
-        if o.size == 3 * self.n_obs * B:
-            return o.reshape(B, self.n_obs, 3), _ffi.NMPC_OBS_PER_INSTANCE
-        raise ValueError("solver: obstacles must be [n_obs,3] or [B,n_obs,3] of (cx, cy, r_uav + r_obs)")
+        return o, self._obs_flag(o.size, B)
+
+    def _dev_inputs(self, B: int, obstacles, bounds=()):
+        """The batch-shared inputs of a device call of B instances: the bounds (lbx, ubx, lbg, ubg) as cached device copies,
+        length-checked, and the obstacle table with its flag.  A contiguous CUDA float64 obstacle tensor is used as it is
+        (nmpc_set_obstacle_motion registers it and the kernel moves it in place)."""
+        dev_bounds = []
+        for key, a, n in zip(("lbx", "ubx", "lbg", "ubg"), bounds, (self.n_w, self.n_w, self.n_g, self.n_g)):
+            dev_bounds.append(self._dev_const(key, a))
+            if dev_bounds[-1].numel() != n:
+                raise ValueError("solver: bound vector has the wrong length")
+        if obstacles is None:
+            return dev_bounds, self._dev_const("obs", self.obstacles), 0
+        if _is_cuda_tensor(obstacles):
+            obs = obstacles.to(torch.float64).contiguous()
+            return dev_bounds, obs, self._obs_flag(obs.numel(), B)
+        o, flags = self._obst(obstacles, B)
+        return dev_bounds, torch.from_numpy(o).to(f"cuda:{self.device}"), flags
 
     def _call_host(self, x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking=True):
         L = _ffi.lib()
@@ -328,8 +319,6 @@ class Solver:
         lbx, ubx = self._host(lbx, self.n_w, "lbx", True), self._host(ubx, self.n_w, "ubx", True)
         lbg, ubg = self._host(lbg, self.n_g, "lbg", True), self._host(ubg, self.n_g, "ubg", True)
         obs, flags = self._obst(obstacles, B)
-        if B > self._max_batch:
-            self._create(max(B, 2 * self._max_batch))
         new = (lambda k, shape, dt=np.float64: np.empty(shape, dtype=dt)) if blocking else self._pinned
         x = new("x", (B, self.n_w)); f = new("f", (B,))
         g = new("g", (B, self.n_g)) if want_g else None
@@ -365,20 +354,7 @@ class Solver:
         p = p.to(torch.float64).reshape(-1, self.n_p).contiguous()
         B = p.shape[0]
         x0 = torch.zeros((B, self.n_w), dtype=torch.float64, device=dev) if x0 is None else x0.to(torch.float64).reshape(B, self.n_w).contiguous()
-        lbx, ubx = self._dev_const("lbx", lbx), self._dev_const("ubx", ubx)
-        lbg, ubg = self._dev_const("lbg", lbg), self._dev_const("ubg", ubg)
-        flags = 0
-        if obstacles is None:
-            obs = self._dev_const("obs", self.obstacles)
-        elif _is_cuda_tensor(obstacles):
-            obs = obstacles.to(torch.float64).contiguous()
-            flags = _ffi.NMPC_OBS_PER_INSTANCE if obs.numel() == 3 * self.n_obs * B and B > 1 else 0
-        else:
-            o, flags = self._obst(obstacles, B)
-            obs = torch.from_numpy(o).to(dev)
-        for t, n in ((lbx, self.n_w), (ubx, self.n_w), (lbg, self.n_g), (ubg, self.n_g)):
-            if t.numel() != n:
-                raise ValueError("solver: bound vector has the wrong length")
+        (lbx, ubx, lbg, ubg), obs, flags = self._dev_inputs(B, obstacles, (lbx, ubx, lbg, ubg))
         x = torch.empty((B, self.n_w), dtype=torch.float64, device=dev)
         f = torch.empty(B, dtype=torch.float64, device=dev)
         g = torch.empty((B, self.n_g), dtype=torch.float64, device=dev) if want_g else None
@@ -424,10 +400,6 @@ class Solver:
 
     # -- function-level evaluation (nlp_f / nlp_g / nlp_grad_f / nlp_hess_l of the reference's nlpsol) ----
     def evaluate(self, w, p, lam=None, v=None, sigma: float = 1.0, obstacles=None, weights=None, target_traj=None):
-        if weights is not None or target_traj is not None:
-            pp = np.asarray(p) if not _is_cuda_tensor(p) else p
-            with self._weights(weights, pp), self._traj(target_traj, pp):
-                return self.evaluate(w, p, lam=lam, v=v, sigma=sigma, obstacles=obstacles)
         L = _ffi.lib()
         dev = f"cuda:{self.device}"
         to = lambda a, n: torch.as_tensor(np.asarray(a, dtype=np.float64) if not _is_cuda_tensor(a) else a,
@@ -436,68 +408,35 @@ class Solver:
         B = w.shape[0]
         lam_t = to(lam, self.n_g) if lam is not None else None
         v_t = to(v, self.n_w) if v is not None else None
-        flags = 0
-        if obstacles is None:
-            obs = self._dev_const("obs", self.obstacles)
-        else:
-            o, flags = self._obst(obstacles, B)
-            obs = torch.from_numpy(o).to(dev)
+        _, obs, flags = self._dev_inputs(B, obstacles)
         z = lambda *s: torch.empty(s, dtype=torch.float64, device=dev)
         f, g, grad = z(B), z(B, self.n_g), z(B, self.n_w)
         jtv = z(B, self.n_w) if lam_t is not None else None
         hv = z(B, self.n_w) if v_t is not None else None
         ptr = lambda t: None if t is None else t.data_ptr()
         stream = torch.cuda.current_stream(torch.device(dev)).cuda_stream
-        _ffi.check(L.nmpc_eval(self._h, B, ptr(w), ptr(p), ptr(obs), flags, float(sigma), ptr(lam_t), ptr(v_t),
-                               ptr(f), ptr(g), ptr(grad), ptr(jtv), ptr(hv), stream), "nmpc_eval")
+        with self._settings(B, weights, target_traj):
+            _ffi.check(L.nmpc_eval(self._h, B, ptr(w), ptr(p), ptr(obs), flags, float(sigma), ptr(lam_t), ptr(v_t),
+                                   ptr(f), ptr(g), ptr(grad), ptr(jtv), ptr(hv), stream), "nmpc_eval")
         torch.cuda.synchronize()
         return dict(f=f, g=g, grad=grad, jtv=jtv, hv=hv)
 
     # -- shift_timestep (NMPC_TT.py:13-30) on device --------------------------------------------
     def solve_and_step(self, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre=None, err_accum=None, obstacles=None,
                        want_x: bool = False, weights=None, target_traj=None, predict_target: bool = False, obstacle_vel=None):
-        """predict_target: every solve uses the target's own Euler prediction over the horizon, made in the kernel from p's
+        """One closed-loop step of B instances in ONE kernel launch (nmpc_solve_and_step): solves from the warm start
+        u_warm with parameters p, then shifts p / u_warm in place (torch CUDA float64 tensors).  Returns dict(x, f)
+        with x None unless want_x; status / iterations through stats().
+        predict_target: every solve uses the target's own Euler prediction over the horizon, made in the kernel from p's
         target block and this step's target input (NMPC_PREDICT_TARGET; the arithmetic of ClosedLoop.target_prediction()).
         obstacle_vel [B, n_obs, 2] (CUDA float64): obstacles, then a CUDA float64 [B, n_obs, 3] tensor, is moved in place by
         T * obstacle_vel after the solve (nmpc_set_obstacle_motion); this step's constraint rows use the positions before."""
         if predict_target and target_traj is not None:
             raise ValueError("solver: predict_target and target_traj exclude each other (the prediction replaces the trajectory)")
-        if weights is not None or target_traj is not None:
-            with self._weights(weights, p), self._traj(target_traj, p):
-                return self.solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x,
-                                           predict_target=predict_target, obstacle_vel=obstacle_vel)
-        with self._motion(obstacles, obstacle_vel, p.shape[0]):
-            return self._solve_and_step(p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, predict_target)
-
-    def _solve_and_step(self, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, predict_target=False):
-        """One closed-loop step of B instances in ONE kernel launch (nmpc_solve_and_step): solves from the warm start
-        u_warm with parameters p, then shifts p / u_warm in place (torch CUDA float64 tensors).  Returns dict(x, f)
-        with x None unless want_x; status / iterations through stats()."""
-        L = _ffi.lib()
-        dev = p.device
-        B = p.shape[0]
-        lbx, ubx = self._dev_const("lbx", lbx), self._dev_const("ubx", ubx)
-        lbg, ubg = self._dev_const("lbg", lbg), self._dev_const("ubg", ubg)
-        flags = 0
-        if obstacles is None:
-            obs = self._dev_const("obs", self.obstacles)
-        else:
-            obs = obstacles.to(torch.float64).contiguous()
-            flags = _ffi.NMPC_OBS_PER_INSTANCE if obs.numel() == 3 * self.n_obs * B and B > 1 else 0
-        if predict_target:
-            flags |= _ffi.NMPC_PREDICT_TARGET
-        x = torch.empty((B, self.n_w), dtype=torch.float64, device=dev) if want_x else None
-        f = torch.empty(B, dtype=torch.float64, device=dev)
-        status = torch.empty(B, dtype=torch.int32, device=dev)
-        iters = torch.empty(B, dtype=torch.int32, device=dev)
-        ptr = lambda t: None if t is None else t.data_ptr()
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        if target_vw is None and getattr(self, "_sched", None) is None:
-            raise ValueError("solver: target_vw is None and no schedule is set (set_schedule)")
-        _ffi.check(L.nmpc_solve_and_step(self._h, B, ptr(p), ptr(u_warm), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags,
-                                         ptr(target_vw), ptr(x), ptr(f), ptr(fov_centre), ptr(err_accum), ptr(status), ptr(iters),
-                                         stream), "nmpc_solve_and_step")
-        self._keep = (obs,)
+        status = torch.empty(p.shape[0], dtype=torch.int32, device=p.device)
+        iters = torch.empty(p.shape[0], dtype=torch.int32, device=p.device)
+        x, f = self._fused("nmpc_solve_and_step", (), (status, iters), p, u_warm, (lbx, ubx, lbg, ubg), target_vw, fov_centre,
+                           err_accum, obstacles, want_x, predict_target, obstacle_vel, weights, target_traj)
         self._stats = dict(return_status=status, iter_count=iters)
         return dict(x=x, f=f, g=None, lam_x=None, lam_g=None)
 
@@ -508,40 +447,34 @@ class Solver:
         place.  Returns dict(x, f of the last step, status_log / iters_log [steps, B] when log, converged [B] = number of
         converged solves per instance); stats() reports the last step.  Bit-identical to `steps` solve_and_step calls, also
         with predict_target / obstacle_vel (as in solve_and_step: the prediction is made every step, the obstacles move every step)."""
-        with self._motion(obstacles, obstacle_vel, p.shape[0]):
-            return self._run_closed_loop(steps, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, log,
-                                         predict_target)
-
-    def _run_closed_loop(self, steps, p, u_warm, lbx, ubx, lbg, ubg, target_vw, fov_centre, err_accum, obstacles, want_x, log,
-                         predict_target):
-        L = _ffi.lib()
-        dev = p.device
         B = p.shape[0]
-        lbx, ubx = self._dev_const("lbx", lbx), self._dev_const("ubx", ubx)
-        lbg, ubg = self._dev_const("lbg", lbg), self._dev_const("ubg", ubg)
-        flags = 0
-        if obstacles is None:
-            obs = self._dev_const("obs", self.obstacles)
-        else:
-            obs = obstacles.to(torch.float64).contiguous()
-            flags = _ffi.NMPC_OBS_PER_INSTANCE if obs.numel() == 3 * self.n_obs * B and B > 1 else 0
-        if predict_target:
-            flags |= _ffi.NMPC_PREDICT_TARGET
-        if target_vw is None and getattr(self, "_sched", None) is None:
-            raise ValueError("solver: target_vw is None and no schedule is set (set_schedule)")
-        x = torch.empty((B, self.n_w), dtype=torch.float64, device=dev) if want_x else None
-        f = torch.empty(B, dtype=torch.float64, device=dev)
-        slog = torch.empty((steps, B), dtype=torch.int32, device=dev) if log else None
-        ilog = torch.empty((steps, B), dtype=torch.int32, device=dev) if log else None
-        conv = torch.zeros(B, dtype=torch.int32, device=dev)
-        ptr = lambda t: None if t is None else t.data_ptr()
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        _ffi.check(L.nmpc_run_closed_loop(self._h, B, int(steps), ptr(p), ptr(u_warm), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags,
-                                          ptr(target_vw), ptr(x), ptr(f), ptr(fov_centre), ptr(err_accum), ptr(slog), ptr(ilog), ptr(conv),
-                                          stream), "nmpc_run_closed_loop")
-        self._keep = (obs,)
+        slog = torch.empty((steps, B), dtype=torch.int32, device=p.device) if log else None
+        ilog = torch.empty((steps, B), dtype=torch.int32, device=p.device) if log else None
+        conv = torch.zeros(B, dtype=torch.int32, device=p.device)
+        x, f = self._fused("nmpc_run_closed_loop", (int(steps),), (slog, ilog, conv), p, u_warm, (lbx, ubx, lbg, ubg), target_vw,
+                           fov_centre, err_accum, obstacles, want_x, predict_target, obstacle_vel)
         self._stats = dict(return_status=slog[-1], iter_count=ilog[-1]) if log else {}
         return dict(x=x, f=f, status_log=slog, iters_log=ilog, converged=conv)
+
+    def _fused(self, entry, lead, logs, p, u_warm, bounds, target_vw, fov_centre, err_accum, obstacles, want_x, predict_target,
+               obstacle_vel, weights=None, target_traj=None):
+        """One call of the fused closed-loop entry point `entry`: `lead` are its arguments between B and p, `logs` its outputs
+        after err_accum.  Returns (x, f)."""
+        B = p.shape[0]
+        bounds, obs, flags = self._dev_inputs(B, obstacles, bounds)
+        if predict_target:
+            flags |= _ffi.NMPC_PREDICT_TARGET
+        if target_vw is None and self._sched is None:
+            raise ValueError("solver: target_vw is None and no schedule is set (set_schedule)")
+        x = torch.empty((B, self.n_w), dtype=torch.float64, device=p.device) if want_x else None
+        f = torch.empty(B, dtype=torch.float64, device=p.device)
+        ptr = lambda t: None if t is None else t.data_ptr()
+        with self._settings(B, weights, target_traj, obstacles, obstacle_vel):
+            _ffi.check(getattr(_ffi.lib(), entry)(self._h, B, *lead, ptr(p), ptr(u_warm), *map(ptr, bounds), ptr(obs), flags,
+                                                  ptr(target_vw), ptr(x), ptr(f), ptr(fov_centre), ptr(err_accum), *map(ptr, logs),
+                                                  torch.cuda.current_stream(p.device).cuda_stream), entry)
+        self._keep = (obs,)
+        return x, f
 
     def set_warm_start(self, lam_x0, lam_g0):
         """nmpc_set_warm_start: CUDA float64 tensors lam_x0 [B, n_w], lam_g0 [B, n_g] read by the following solves (and

@@ -180,5 +180,32 @@ def test_refusals(pkg):
     with pytest.raises(ValueError, match="no obstacle rows"):
         pkg.nlpsol("g", "ipm", gl, max_batch=B).solve_and_step(t(pkg.random_instances(gl, B, 1)[0]), torch.zeros((B, gl.n_w), dtype=torch.float64, device=dev),
                                                                 *gl.bounds(), vwt, obstacle_vel=vel)
+    # a bound vector with extra entries, an obstacle tensor with three entries more than [B, n_obs, 3]: every device path
+    bounds = list(sc.bounds())
+    too_long = [np.concatenate([bounds[0], bounds[0][:2]])] + bounds[1:]
+    big = torch.cat([obs.reshape(-1), obs.reshape(-1)[:3]])
+    for bnd, ob in ((too_long, None), (bounds, big)):
+        with pytest.raises(ValueError, match="bound vector|obstacles must be"):
+            s.solve_and_step(p, u, *bnd, vwt, obstacles=ob)
+        with pytest.raises(ValueError, match="bound vector|obstacles must be"):
+            s.run_closed_loop(2, p, u, *bnd, vwt, obstacles=ob)
+        with pytest.raises(ValueError, match="bound vector|obstacles must be"):
+            s(x0=u, p=p, lbx=bnd[0], ubx=bnd[1], lbg=bnd[2], ubg=bnd[3], obstacles=ob)
     torch.cuda.synchronize()
     assert torch.equal(p, t(p0))          # none of them launched
+
+
+@pytest.mark.gpu
+def test_device_call_keeps_the_handle(pkg):
+    """max_batch sizes the staging buffers of the host path only: a device-tensor call with more instances and weights= keeps the
+    handle, and with it the schedule set before."""
+    sc = pkg.SCENARIOS["t_trajectory"]
+    B = 4
+    s = pkg.nlpsol("s", "ipm", sc, max_batch=1)
+    s.set_schedule(np.array([[sc.schedule(k) for k in range(sc.steps)]]))
+    p = torch.as_tensor(pkg.random_instances(sc, B, seed=6)[0], dtype=torch.float64, device="cuda:0").contiguous()
+    u = torch.zeros((B, sc.n_w), dtype=torch.float64, device="cuda:0")
+    s(x0=u, p=p, lbx=sc.bounds()[0], ubx=sc.bounds()[1], lbg=sc.bounds()[2], ubg=sc.bounds()[3], weights=np.tile([sc.w1, sc.w2], (B, 1)))
+    s.solve_and_step(p, u, *sc.bounds(), None)
+    torch.cuda.synchronize()
+    assert bool((s.stats()["return_status"] >= 0).all())
