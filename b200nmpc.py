@@ -17,6 +17,7 @@ _pkg = sys.modules[_NAME]
 
 nlpsol = _pkg.nlpsol
 Solver = _pkg.Solver
+SolveFunction = _pkg.SolveFunction
 Scenario = _pkg.Scenario
 SCENARIOS = _pkg.SCENARIOS
 scenarios = _pkg.scenarios

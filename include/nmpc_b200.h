@@ -96,6 +96,10 @@ int nmpc_destroy(nmpc_handle* h);
                                       target input (target_vw or the schedule), computed in the kernel, no host work per step.
                                       Refused by the calls that have no (v, om) (nmpc_solve, nmpc_solve_host(_async), nmpc_eval,
                                       nmpc_lam_p) and while a target trajectory is set (nmpc_set_target_trajectory). */
+#define NMPC_KEEP_BARRIER 4u       /* nmpc_solve, nmpc_solve_host, nmpc_solve_host_async only: the solve also keeps the barrier data
+                                      of its final iterate (the Sigma_x and Sigma_g of the sensitivity system below) in buffers the
+                                      handle owns, for nmpc_sensitivity.  The results of the solve are bit-identical with and
+                                      without it.  Refused by nmpc_solve_and_step and nmpc_run_closed_loop. */
 
 /* solver(x0,lbx,ubx,lbg,ubg,p)  (NMPC_TT.py:358-365), B instances at once.
  *   p    [B][11]   x0  [B][6N]                       inputs
@@ -149,6 +153,33 @@ int nmpc_eval(nmpc_handle* h, int32_t B, const double* w, const double* p, const
  * enter the NLP and their multipliers are 0. */
 int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* obst, uint32_t flags,
                const double* lam_g, double* lam_p, void* cuda_stream);
+
+/* Solution sensitivities of the last solve on this handle, which must have passed NMPC_KEEP_BARRIER with the same B: CasADi's
+ * jac:x:p (and sIPOPT's), and the derivative with respect to the cost weights.  For each instance it is the implicit-function
+ * derivative of the barrier KKT system at the solve's final iterate, with no inertia correction (delta_w = 0):
+ *     K dx/dth = -(grad2_{x th} L + J^T Sigma_g J_th),     K = grad2_{xx} L + Sigma_x + J^T Sigma_g J,     L = f + lam_g^T g,
+ * with J = dg/dx, J_th = dg/dth, Sigma_x = z_L / (x - l) + z_U / (u - x) from the solve's own bound multipliers and distances to
+ * its relaxed bounds, and Sigma_g the same for the row slacks, all in the unscaled units of lam_x / lam_g (DESIGN.md section 1).
+ * It is computed from those kept Sigmas, not from lam_x / lam_g and g(x): x is clipped to the original bounds and g(x) differs
+ * from the solve's slacks by up to the tolerance, which for an active row is more than the slack's distance to its bound.
+ *   x_sol [B][n_w], p [B][n_p], lam_g [B][n_g]: as that solve returned them (and given to it);  obst / flags as for nmpc_solve
+ *   dx_dp [B][n_w][n_p] = dx/dp.  The theta_t column is exactly 0 (theta_t does not enter the NLP), and so are the target columns
+ *     while a target trajectory is set (nmpc_set_target_trajectory), as in nmpc_lam_p
+ *   dx_dw [B][n_w][2] = dx/d(w1, w2) (may be NULL; model 0 only): with per-instance weights (nmpc_set_weights), each instance's own
+ *   sens_status [B] (may be NULL): 0, or 1 when the reduced Hessian is not positive definite at delta_w = 0 -- the sensitivity is
+ *     then undefined and the instance's columns are NaN
+ * The weights and the target trajectory set on the handle are read as by the solve: they must be the solve's.  The columns are
+ * computed for every instance; only those of converged instances (status NMPC_SOLVE_SUCCEEDED) are a sensitivity of a solution.
+ * Refused when the last solve did not keep its barrier data, when B differs from its B, and when dx_dw is given for model 1.
+ * cuda_stream may differ from the solve's (e.g. after nmpc_solve_host, which runs on the handle's own stream): the launch waits
+ * for the keeping solve, and the next solve on the handle waits for the launch (they share the handle's Riccati scratch). */
+int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g, const double* obst,
+                     uint32_t flags, double* dx_dp, double* dx_dw, int32_t* sens_status, void* cuda_stream);
+/* The barrier data nmpc_sensitivity uses: sig_x [B][n_w], sig_g [B][n_g] (device pointers, either may be NULL) <- the Sigma_x and
+ * Sigma_g kept by the last solve, B its batch size.  Lets a caller check the sensitivity system or form other right-hand sides.
+ * Refused when the last solve did not keep them.  (An addition to the sensitivity call: the tests build the sensitivity system
+ * from these Sigmas.)  The copies wait for the keeping solve. */
+int nmpc_barrier_data(nmpc_handle* h, double* sig_x, double* sig_g, void* cuda_stream);
 
 /* shift_timestep (NMPC_TT.py:13-30) + FOV centre (:399-402) for B instances, in place on the
  * parameter block the next solve reads:

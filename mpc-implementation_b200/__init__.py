@@ -5,7 +5,7 @@ Scope: the hot path of devsonni/MPC-Implementation only -- `sol = solver(x0,lbx,
 Import as `import b200nmpc` (root shim; this directory's name is not a valid module name).
 """
 from . import _ffi, scenarios
-from .nlpsol import Solver, nlpsol
+from .nlpsol import SolveFunction, Solver, nlpsol
 from .scenarios import SCENARIOS, Scenario, random_instances
 
-__all__ = ["nlpsol", "Solver", "Scenario", "SCENARIOS", "scenarios", "random_instances", "_ffi"]
+__all__ = ["nlpsol", "Solver", "SolveFunction", "Scenario", "SCENARIOS", "scenarios", "random_instances", "_ffi"]

@@ -14,6 +14,7 @@ LIB_PATH = Path(__import__("os").environ.get("NMPC_B200_LIB", _CSRC / "libnmpc_b
 
 NMPC_OBS_PER_INSTANCE = 1
 NMPC_PREDICT_TARGET = 2      # nmpc_solve_and_step / nmpc_run_closed_loop: the target's own Euler prediction, made in the kernel
+NMPC_KEEP_BARRIER = 4        # nmpc_solve(_host): keep the final iterate's barrier data for nmpc_sensitivity
 
 # CasADi's stats()['return_status'] strings of the IPOPT plugin
 STATUS_NAMES = {0: "Solve_Succeeded", 1: "Maximum_Iterations_Exceeded", 2: "Restoration_Failed",
@@ -42,7 +43,7 @@ class NmpcStats(C.Structure):
                 ("trial_passes", C.c_int64)]
 
 
-EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_step",
+EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_sensitivity", "nmpc_barrier_data", "nmpc_step",
            "nmpc_get_stats", "nmpc_set_debug_log", "nmpc_set_order", "nmpc_set_weights", "nmpc_set_target_trajectory", "nmpc_set_obstacle_motion", "nmpc_set_schedule", "nmpc_set_warm_start", "nmpc_measure_fp64_peak", "nmpc_n_w", "nmpc_n_g", "nmpc_n_p",
            "nmpc_last_error", "nmpc_version"]
 
@@ -79,6 +80,9 @@ def lib():
     L.nmpc_step.argtypes = [vp, C.c_int32] + [vp] * 6 + [vp]
     if hasattr(L, "nmpc_lam_p"):
         L.nmpc_lam_p.argtypes = [vp, C.c_int32, vp, vp, vp, C.c_uint32, vp, vp, vp]
+    if hasattr(L, "nmpc_sensitivity"):
+        L.nmpc_sensitivity.argtypes = [vp, C.c_int32, vp, vp, vp, vp, C.c_uint32, vp, vp, vp, vp]
+        L.nmpc_barrier_data.argtypes = [vp, vp, vp, vp]
     L.nmpc_get_stats.argtypes = [vp, C.POINTER(NmpcStats)]
     L.nmpc_set_debug_log.argtypes = [vp, vp, C.c_int32]
     L.nmpc_set_order.argtypes = [vp, vp]

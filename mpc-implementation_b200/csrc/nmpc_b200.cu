@@ -28,12 +28,17 @@ namespace nmpc {
 #define NMPC_DECL_INST(N, O, M)                      \
   int ipm_prepare_##N##_##O##_##M(int*, size_t*, int*, int*);  \
   int ipm_ricmap_##N##_##O##_##M(unsigned*, cudaStream_t);     \
-  int ipm_launch_##N##_##O##_##M(const SolveArgs&, int, size_t, cudaStream_t);
+  int ipm_launch_##N##_##O##_##M(const SolveArgs&, int, size_t, cudaStream_t);  \
+  int ipm_sens_##N##_##O##_##M(const SolveArgs&, int, cudaStream_t);
 NMPC_DECL_INST(15, 3, 0) NMPC_DECL_INST(15, 10, 0) NMPC_DECL_INST(30, 10, 0) NMPC_DECL_INST(30, 3, 0) NMPC_DECL_INST(5, 3, 0) NMPC_DECL_INST(15, 7, 0)
 NMPC_DECL_INST(15, 0, 1)
 }  // namespace nmpc
-struct IpmInst { int N, n_obs, model; int (*prepare)(int*, size_t*, int*, int*); int (*ricmap)(unsigned*, cudaStream_t); int (*launch)(const SolveArgs&, int, size_t, cudaStream_t); };
-#define NMPC_INST(N, O, M) {N, O, M, nmpc::ipm_prepare_##N##_##O##_##M, nmpc::ipm_ricmap_##N##_##O##_##M, nmpc::ipm_launch_##N##_##O##_##M}
+struct IpmInst {
+  int N, n_obs, model;
+  int (*prepare)(int*, size_t*, int*, int*); int (*ricmap)(unsigned*, cudaStream_t); int (*launch)(const SolveArgs&, int, size_t, cudaStream_t);
+  int (*sens)(const SolveArgs&, int, cudaStream_t);      // nmpc_sensitivity (nmpc_sens.cuh)
+};
+#define NMPC_INST(N, O, M) {N, O, M, nmpc::ipm_prepare_##N##_##O##_##M, nmpc::ipm_ricmap_##N##_##O##_##M, nmpc::ipm_launch_##N##_##O##_##M, nmpc::ipm_sens_##N##_##O##_##M}
 static const IpmInst IPM_INSTS[] = {NMPC_INST(15, 3, 0), NMPC_INST(15, 10, 0), NMPC_INST(30, 10, 0), NMPC_INST(30, 3, 0), NMPC_INST(5, 3, 0),
                                     NMPC_INST(15, 7, 0),      // the 7 obstacle rows of MATLAB/Dynamic Obstacles/Dynamic Obstacle avoidance.m:126-134
                                     NMPC_INST(15, 0, 1)};     // the gimbal-less tracker of MATLAB/Dynamic Obstacles/NMPC_TT.m
@@ -256,6 +261,11 @@ struct nmpc_handle {
   const double* sched_table; const int32_t *sched_id, *sched_phase; int sched_rows, sched_len, sched_iter;   // nmpc_set_schedule
   double* d_tgt_pred; int tgt_pred_cap;        // NMPC_PREDICT_TARGET: the trajectory the kernel predicts, [tgt_pred_cap][N][2]
   double* move_obs; const double* move_vel;    // nmpc_set_obstacle_motion
+  double *d_sigx, *d_sigg; int sig_cap;        // NMPC_KEEP_BARRIER: Sigma_x [sig_cap][n_w], Sigma_g [sig_cap][n_g] of the last solve
+  int kept_B;                                  // B of the last solve when it kept them, else 0 (what nmpc_sensitivity needs)
+  // nmpc_sensitivity reads the kept Sigmas and uses the Riccati scratch, possibly on another stream than the solves (the host
+  // calls run on own_stream): ev_keep marks the end of the keeping solve, ev_sens the end of the last sensitivity launch
+  cudaEvent_t ev_keep, ev_sens; cudaStream_t keep_stream, sens_stream; int sens_pending;
   int* d_counter;                  // [4]: queue counter x2, done counter x2
   unsigned long long* d_stats;     // [2][NSTAT]
   unsigned long long* stats_last;  // the half written by the last call
@@ -270,14 +280,25 @@ struct nmpc_handle {
 
 // The refusals several entry points share, each naming `fn`, the public function the caller called.  Those in `which` are
 // checked in this order; an entry point that makes them at different places of its own order calls this once per place.
-enum : unsigned { NULL_HANDLE = 1u, NO_OBSTACLES = 2u, PREDICT_WITHOUT_VW = 4u, PREDICT_WITH_TRAJECTORY = 8u };
-static int refused(const nmpc_handle* h, const char* fn, unsigned which, const double* obst = nullptr, uint32_t flags = 0) {
+enum : unsigned { NULL_HANDLE = 1u, NO_OBSTACLES = 2u, PREDICT_WITHOUT_VW = 4u, PREDICT_WITH_TRAJECTORY = 8u, KEEP_WITHOUT_OUTPUTS = 16u,
+                  NOT_KEPT = 32u, KEPT_OTHER_B = 64u, WEIGHTS_OF_MODEL_1 = 128u };
+static int refused(const nmpc_handle* h, const char* fn, unsigned which, const double* obst = nullptr, uint32_t flags = 0, int32_t B = 0,
+                   const double* dx_dw = nullptr) {
   if ((which & NULL_HANDLE) && !h) return fail(std::string(fn) + ": null handle");
   if ((which & NO_OBSTACLES) && h->pr.n_obs > 0 && !obst) return fail(std::string(fn) + ": obstacle table required");
   if ((which & PREDICT_WITHOUT_VW) && (flags & NMPC_PREDICT_TARGET))
     return fail(std::string(fn) + ": NMPC_PREDICT_TARGET needs the target's (v, omega) of the step: use nmpc_solve_and_step or nmpc_run_closed_loop");
   if ((which & PREDICT_WITH_TRAJECTORY) && (flags & NMPC_PREDICT_TARGET) && h->tgt)
     return fail(std::string(fn) + ": NMPC_PREDICT_TARGET and a target trajectory (nmpc_set_target_trajectory) exclude each other");
+  if ((which & KEEP_WITHOUT_OUTPUTS) && (flags & NMPC_KEEP_BARRIER))
+    return fail(std::string(fn) + ": NMPC_KEEP_BARRIER is for nmpc_solve, nmpc_solve_host and nmpc_solve_host_async (the fused and "
+                                  "free-running calls return no multipliers to differentiate with)");
+  if ((which & NOT_KEPT) && !h->kept_B)
+    return fail(std::string(fn) + ": the last solve on this handle did not keep its barrier data (pass NMPC_KEEP_BARRIER to it)");
+  if ((which & KEPT_OTHER_B) && B != h->kept_B)
+    return fail(std::string(fn) + ": B = " + std::to_string(B) + " differs from the B = " + std::to_string(h->kept_B) + " of the last solve");
+  if ((which & WEIGHTS_OF_MODEL_1) && dx_dw && h->pr.model)
+    return fail(std::string(fn) + ": dx_dw is for model 0 only (the gimbal-less model has no cost weights)");
   return 0;
 }
 
@@ -292,7 +313,9 @@ static SolveArgs solve_args(int32_t B, const double* p, const double* x0, const 
 static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream_t s, const char* fn, bool fused = false) {
   const std::string f(fn);
   if (refused(h, fn, NULL_HANDLE)) return 1;
+  h->kept_B = 0;                        // whatever this call does, the barrier data of an earlier solve no longer belongs to the last solve
   if (fused) {
+    if (refused(h, fn, KEEP_WITHOUT_OUTPUTS, nullptr, flags)) return 1;
     if (!A.step_p || !A.step_u) return fail(f + ": null required pointer");
     if (!A.step_vw && !h->sched_table) return fail(f + ": target_vw is NULL and no schedule is set (nmpc_set_schedule)");
     if (A.step_err && !A.step_fov) return fail(f + ": err_accum needs fov_centre");
@@ -316,6 +339,8 @@ static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream
   A.ric = h->d_ric; A.ric_stride = h->ric_stride; A.ricmap = h->d_ricmap;
   A.cold = h->d_cold; A.cold_stride = h->cold_stride;
   A.dbg = h->dbg; A.dbg_rows = h->dbg_rows;
+  if (h->sens_pending && h->sens_stream != s) CK(cudaStreamWaitEvent(s, h->ev_sens, 0));     // the Riccati scratch is shared
+  h->sens_pending = 0;
   if (B > h->order_cap) {     // (re)allocate the scheduling buffers; the previous counts are dropped
     CK(cudaStreamSynchronize(s));
     for (int i = 0; i < 2; ++i) { if (h->d_order[i]) cudaFree(h->d_order[i]); h->d_order[i] = nullptr; }
@@ -326,6 +351,16 @@ static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream
     CK(cudaMalloc(&h->d_order[0], sizeof(int32_t) * B)); CK(cudaMalloc(&h->d_order[1], sizeof(int32_t) * B));
     CK(cudaMalloc(&h->d_keep_iters, sizeof(int32_t) * B));
     h->order_cap = B;
+  }
+  const bool keep = (flags & NMPC_KEEP_BARRIER) != 0;
+  if (keep && B > h->sig_cap) {     // the kept barrier data, grown like the scheduling buffers
+    CK(cudaStreamSynchronize(s));
+    if (h->d_sigx) cudaFree(h->d_sigx);
+    if (h->d_sigg) cudaFree(h->d_sigg);
+    h->d_sigx = h->d_sigg = nullptr; h->sig_cap = 0;
+    CK(cudaMalloc(&h->d_sigx, sizeof(double) * (size_t)model_nu(h->pr.model) * h->pr.N * B));
+    CK(cudaMalloc(&h->d_sigg, sizeof(double) * (size_t)h->pr.R * h->pr.S * B));
+    h->sig_cap = B;
   }
   if (predict && B > h->tgt_pred_cap) {     // the predicted trajectories, grown like the scheduling buffers
     CK(cudaStreamSynchronize(s));
@@ -342,6 +377,7 @@ static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream
   A.lam_x0 = h->ws_lamx; A.lam_g0 = h->ws_lamg; A.ws_shift = (h->ws_lamx && A.step_p) ? 1 : 0;
   A.weights = h->weights;
   A.pair_trials = h->pair_trials;
+  A.sig_x = keep ? h->d_sigx : nullptr; A.sig_g = keep ? h->d_sigg : nullptr;
   // fetch order: explicit (nmpc_set_order) > the order the previous call on this handle prepared for the same B > natural
   A.order = h->order_next; h->order_next = nullptr;
   if (!A.order && h->auto_order && h->have_order && h->prev_B == B) A.order = h->d_order[par];
@@ -371,6 +407,8 @@ static int launch_solve(nmpc_handle* h, SolveArgs& A, uint32_t flags, cudaStream
   h->prev_B = B;
   h->last_stream = s;
   h->sched_iter += sched_steps;
+  h->kept_B = keep ? B : 0;
+  if (keep) { CK(cudaEventRecord(h->ev_keep, s)); h->keep_stream = s; }
   return 0;
 }
 
@@ -459,6 +497,8 @@ int nmpc_create(const nmpc_spec* spec, int device, nmpc_handle** out) {
   CKH(cudaMalloc(&h->d_stats, 2 * NSTAT * sizeof(unsigned long long)));
   CKH(cudaMemset(h->d_stats, 0, 2 * NSTAT * sizeof(unsigned long long)));
   CKH(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
+  CKH(cudaEventCreateWithFlags(&h->ev_keep, cudaEventDisableTiming));
+  CKH(cudaEventCreateWithFlags(&h->ev_sens, cudaEventDisableTiming));
   const int mb = spec->max_batch > 0 ? spec->max_batch : 0;
   if (mb > 0) {
     const size_t nw = (size_t)model_nu(spec->model) * spec->N, ng = (size_t)h->pr.R * h->pr.S;
@@ -480,9 +520,12 @@ int nmpc_destroy(nmpc_handle* h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
   void* ptrs[] = {h->d_ric, h->d_cold, h->d_counter, h->d_stats, h->d_p, h->d_x0, h->d_lbx, h->d_ubx, h->d_lbg, h->d_ubg, h->d_obs,
-                  h->d_x, h->d_f, h->d_g, h->d_lamx, h->d_lamg, h->d_status, h->d_iters, h->d_order[0], h->d_order[1], h->d_keep_iters, h->d_ricmap, h->d_tgt_pred};
+                  h->d_x, h->d_f, h->d_g, h->d_lamx, h->d_lamg, h->d_status, h->d_iters, h->d_order[0], h->d_order[1], h->d_keep_iters, h->d_ricmap, h->d_tgt_pred,
+                  h->d_sigx, h->d_sigg};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
+  if (h->ev_keep) cudaEventDestroy(h->ev_keep);
+  if (h->ev_sens) cudaEventDestroy(h->ev_sens);
   delete h;
   return 0;
 }
@@ -589,6 +632,45 @@ int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, 
                const double* lam_g, double* lam_p, void* cuda_stream) {
   const EvalArgs A{{}, B, x_sol, p, obst, 0, nullptr, nullptr, 1.0, lam_g, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, lam_p};
   return launch_eval(h, "nmpc_lam_p", A, flags, !x_sol || !p || !lam_g || !lam_p, cuda_stream);
+}
+
+int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g, const double* obst,
+                     uint32_t flags, double* dx_dp, double* dx_dw, int32_t* sens_status, void* cuda_stream) {
+  const char* fn = "nmpc_sensitivity";
+  const std::string f(fn);
+  if (refused(h, fn, NULL_HANDLE)) return 1;
+  if (B <= 0) return 0;
+  if (refused(h, fn, NOT_KEPT | KEPT_OTHER_B | WEIGHTS_OF_MODEL_1 | PREDICT_WITHOUT_VW, nullptr, flags, B, dx_dw)) return 1;
+  if (!x_sol || !p || !lam_g || !dx_dp) return fail(f + ": null required pointer");
+  if (refused(h, fn, NO_OBSTACLES, obst)) return 1;
+  CK(cudaSetDevice(h->device));
+  // x_sol enters as the start point x0 (ph_load puts it where the solve keeps its iterate) and as x
+  SolveArgs A = solve_args(B, p, x_sol, nullptr, nullptr, nullptr, nullptr, obst, flags, const_cast<double*>(x_sol), nullptr, nullptr,
+                           nullptr, const_cast<double*>(lam_g), nullptr, nullptr);
+  A.pr = h->pr; A.o = h->opt;
+  A.weights = h->weights; A.tgt = h->tgt;
+  A.sig_x = h->d_sigx; A.sig_g = h->d_sigg;
+  A.ric = h->d_ric; A.ric_stride = h->ric_stride; A.ricmap = h->d_ricmap;
+  A.dx_dp = dx_dp; A.dx_dw = dx_dw; A.sens_status = sens_status;
+  const cudaStream_t s = (cudaStream_t)cuda_stream;
+  if (h->keep_stream != s) CK(cudaStreamWaitEvent(s, h->ev_keep, 0));      // the kept Sigmas are complete
+  const int slots = h->max_blocks * h->warps_per_block;      // the Riccati scratch holds one slot per resident warp of the solve
+  if (const int rc = h->inst->sens(A, B < slots ? B : slots, s)) return fail(f + ": launch failed: " + cudaGetErrorString((cudaError_t)rc));
+  CK(cudaEventRecord(h->ev_sens, s));
+  h->sens_pending = 1; h->sens_stream = s;
+  h->last_stream = s; h->launches = 1;
+  return 0;
+}
+
+int nmpc_barrier_data(nmpc_handle* h, double* sig_x, double* sig_g, void* cuda_stream) {
+  if (refused(h, "nmpc_barrier_data", NULL_HANDLE)) return 1;
+  if (refused(h, "nmpc_barrier_data", NOT_KEPT)) return 1;
+  CK(cudaSetDevice(h->device));
+  if (h->keep_stream != (cudaStream_t)cuda_stream) CK(cudaStreamWaitEvent((cudaStream_t)cuda_stream, h->ev_keep, 0));
+  const size_t B = h->kept_B, nw = (size_t)model_nu(h->pr.model) * h->pr.N, ng = (size_t)h->pr.R * h->pr.S;
+  if (sig_x) CK(cudaMemcpyAsync(sig_x, h->d_sigx, sizeof(double) * B * nw, cudaMemcpyDeviceToDevice, (cudaStream_t)cuda_stream));
+  if (sig_g) CK(cudaMemcpyAsync(sig_g, h->d_sigg, sizeof(double) * B * ng, cudaMemcpyDeviceToDevice, (cudaStream_t)cuda_stream));
+  return 0;
 }
 
 int nmpc_step(nmpc_handle* h, int32_t B, const double* x_sol, double* p,

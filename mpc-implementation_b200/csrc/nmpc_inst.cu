@@ -2,7 +2,7 @@
 //   nvcc -DINST_N=15 -DINST_NOBS=3 [-DINST_MODEL=0] -c nmpc_inst.cu -o inst_15_3.o
 #include <cuda_runtime.h>
 #include "../../include/nmpc_b200.h"
-#include "nmpc_solve.cuh"
+#include "nmpc_sens.cuh"
 
 #if !defined(INST_N) || !defined(INST_NOBS)
 #error "compile with -DINST_N=<horizon> -DINST_NOBS=<obstacle rows>"
@@ -23,6 +23,8 @@ int NMPC_CAT(ipm_prepare, INST_N, INST_NOBS)(int* blocks_per_sm, size_t* smem_by
   *cold_doubles = L::COLD_TOTAL;
   cudaError_t e = cudaFuncSetAttribute(nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   if (e != cudaSuccess) return (int)e;
+  e = cudaFuncSetAttribute(nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) return (int)e;
   e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL>, 32 * L::WPB, bytes);
   *smem_bytes = bytes;
   return (int)e;
@@ -36,7 +38,18 @@ int NMPC_CAT(ipm_ricmap, INST_N, INST_NOBS)(unsigned* dev_table, cudaStream_t s)
 
 int NMPC_CAT(ipm_launch, INST_N, INST_NOBS)(const SolveArgs& A, int blocks, size_t bytes, cudaStream_t s) {
   using L = Lay<INST_N, INST_NOBS, INST_MODEL>;
-  nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL><<<blocks, 32 * L::WPB, bytes, s>>>(A);
+  if (A.sig_x) nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL, true><<<blocks, 32 * L::WPB, bytes, s>>>(A);      // NMPC_KEEP_BARRIER
+  else nmpc_ipm_kernel<INST_N, INST_NOBS, INST_MODEL><<<blocks, 32 * L::WPB, bytes, s>>>(A);
+  return (int)cudaGetLastError();
+}
+
+// nmpc_sensitivity: `blocks` warps (one per block) over the B instances, each on Riccati scratch slot blockIdx.x
+int NMPC_CAT(ipm_sens, INST_N, INST_NOBS)(const SolveArgs& A, int blocks, cudaStream_t s) {
+  using L = Lay<INST_N, INST_NOBS, INST_MODEL>;
+  const size_t bytes = sizeof(double) * L::TOTAL;
+  cudaError_t e = cudaFuncSetAttribute(nmpc_sens_kernel<INST_N, INST_NOBS, INST_MODEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) return (int)e;
+  nmpc_sens_kernel<INST_N, INST_NOBS, INST_MODEL><<<blocks, 32, bytes, s>>>(A);
   return (int)cudaGetLastError();
 }
 

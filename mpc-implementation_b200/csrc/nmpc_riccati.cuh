@@ -261,13 +261,15 @@ __device__ __noinline__ bool riccati_factor(double T, double* __restrict__ ric, 
 // Forward sweep: du_k = -K_k dx_k - kappa_k, dx_{k+1} = A_k dx_k + B_k du_k.  Lane r < 6 computes row r of du
 // from its row of [K | kappa] (prefetched one stage ahead from the L2-resident scratch); dx is replicated.
 // Lane k keeps its own stage's dx, du and writes them to the shared-memory entries dx0 / du0 (offsets, [.][S]).
-template <class L>
+// X0 (the sensitivity kernel, nmpc_sens.cuh): the sweep starts from the dx_0 the caller has put in the stage-0 entries of dx0
+// instead of from 0.
+template <class L, bool X0 = false>
 __device__ __noinline__ void riccati_forward(double T, const double* ric, bool soc, int lane, int dx0, int du0) {
   constexpr int S = L::S, N = L::N, LQ0 = L::LQ0;
   const int r = lane < 6 ? lane : 5;
   double dx[8], mydx[8], mydu[6];
 #pragma unroll
-  for (int i = 0; i < 8; ++i) { dx[i] = 0.0; mydx[i] = 0.0; }
+  for (int i = 0; i < 8; ++i) { dx[i] = X0 ? smem[dx0 + i * S] : 0.0; mydx[i] = 0.0; }
 #pragma unroll
   for (int i = 0; i < 6; ++i) mydu[i] = 0.0;
   double row[9];

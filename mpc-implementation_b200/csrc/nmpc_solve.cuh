@@ -89,6 +89,11 @@ struct SolveArgs {
   const unsigned* ricmap;            // per-lane ownership maps of the factorisation (nmpc_riccati.cuh: ric_map_build)
   double* dbg; int dbg_rows;         // optional per-iteration log [B][dbg_rows][10] (tests only)
   int pair_trials;                   // layouts with Lay::PAIR: each backtracking trial pass also evaluates the next trial point
+  // barrier data of the final iterate (NMPC_KEEP_BARRIER: non-NULL launches the KEEP instantiation of the kernel, whose
+  // ph_output writes them), in the unscaled units of lam_x / lam_g: sig_x [B][n_w] = z_L / (w - l~) + z_U / (u~ - w),
+  // sig_g [B][n_g] the same for the row slacks.  The sensitivity kernel (nmpc_sens.cuh) reads them, with x / lam_g as inputs.
+  double *sig_x, *sig_g;
+  double *dx_dp, *dx_dw; int32_t* sens_status;     // nmpc_sensitivity: [B][n_w][n_p], [B][n_w][2] (may be NULL), [B]
 };
 constexpr int NSTAT = 9;
 constexpr int DBG_COLS = 10;
@@ -1108,8 +1113,9 @@ __device__ __noinline__ void ph_unit_mults(const SolveArgs& A, int lane) {
   __syncwarp();
 }
 
-// outputs: honour the original bounds, unscale multipliers, f and g at the returned point
-template <class L>
+// outputs: honour the original bounds, unscale multipliers, f and g at the returned point; KEEP (the kernel instantiation
+// that NMPC_KEEP_BARRIER selects): also the barrier data sig_x / sig_g
+template <class L, bool KEEP = false>
 __device__ __noinline__ void ph_output(const SolveArgs& A, int b, int lane, double df, int status, int iter, int step) {
   const Prob& pr = A.pr; constexpr int N = L::N, R = L::R, S = L::S;
   const bool act = lane <= N, hasu = lane < N;
@@ -1130,6 +1136,16 @@ __device__ __noinline__ void ph_output(const SolveArgs& A, int b, int lane, doub
       const double idf = 1.0 / df;
 #pragma unroll
       for (int i = 0; i < L::NUA; ++i) lo[i] = (LV(LV_ZU + i) - LV(LV_ZL + i)) * idf;
+    }
+    if (KEEP) {      // Sigma_x of the final iterate as ph_derivs forms it, unscaled (the objective scaling df divides out)
+      double* so = A.sig_x + (size_t)b * nw + L::NUA * lane;
+      const double idf = 1.0 / df;
+#pragma unroll 1
+      for (int i = 0; i < L::NUA; ++i) {
+        const Bnd c = ctl_bounds<L>(A, lane, i);
+        const double ui = LV(LV_U + i), il = c.hl ? rcp(ui - c.lo) : 0.0, iu = c.hu ? rcp(c.hi - ui) : 0.0;
+        so[i] = (LV(LV_ZL + i) * il + LV(LV_ZU + i) * iu) * idf;
+      }
     }
   }
   Stage st; rollout<L::SW>(pr, &PAR(0), u, lane, st);
@@ -1160,6 +1176,12 @@ __device__ __noinline__ void ph_output(const SolveArgs& A, int b, int lane, doub
       const double idf = 1.0 / df;
 #pragma unroll 1
       for (int r = 0; r < R; ++r) lo[r] = RW(A_Y, r) * RW(A_DC, r) * idf;
+    }
+    if (KEEP) {      // Sigma_s of the final iterate, unscaled: the scaled row weight enters the Newton matrix as dc^2 Sigma_s / df
+      double* so = A.sig_g + (size_t)b * ng + lane * R;
+      const double idf = 1.0 / df;
+#pragma unroll 1
+      for (int r = 0; r < R; ++r) { const double dc = RW(A_DC, r); so[r] = (VL_(r) * IL_(r) + RW(A_VU, r) * RW(A_IU, r)) * (dc * dc) * idf; }
     }
   }
   if (A.step_p) {     // fused closed-loop shift of this instance (NMPC_TT.py:13-30): warm start, plant, target, FOV error
@@ -1533,7 +1555,7 @@ __device__ __noinline__ bool update_mu(const SolveArgs& A, double* cold, int lan
   return true;
 }
 
-template <class L>
+template <class L, bool KEEP = false>
 __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, double* cold, int b, int lane, int step) {
   const Prob& pr = A.pr; const Opt& o = A.o;
   constexpr int S = L::S, R = L::R;
@@ -1555,7 +1577,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
   const double mu0 = warm ? o.ws_mu_init : o.mu_init;
   const int nzt = ph_start<L>(A, lane, b, df, warm);
   if (nzt < 0) {       // a finite lower bound on an obstacle row (never the case in the reference's NLPs): refused, reported as data
-    ph_output<L>(A, b, lane, df, NMPC_INVALID_NUMBER, 0, step);
+    ph_output<L, KEEP>(A, b, lane, df, NMPC_INVALID_NUMBER, 0, step);
     return;
   }
   alg_init<L>(mu0, o.tau_min, o.tol);
@@ -1769,7 +1791,7 @@ __device__ __noinline__ void solve_instance(const SolveArgs& A, double* ric, dou
     ++iter;
   }
   if (retry_owed) retry_arrive<L>();
-  ph_output<L>(A, b, lane, df, status, iter, step);
+  ph_output<L, KEEP>(A, b, lane, df, status, iter, step);
   if (lane == 0 && A.stats) {
 #pragma unroll
     for (int c = 0; c < NSTAT; ++c) atomicAdd(&A.stats[c], (unsigned long long)AL(F_C0 + c));
@@ -1796,8 +1818,10 @@ __device__ __noinline__ void next_order(const SolveArgs& A, int lane) {
 }
 
 // persistent kernel: Lay::WPB warps per block (one block per SM), one instance per warp at a time, instances from
-// an atomic work queue (optionally in a caller-given order)
-template <int N_, int NOBS_, int MODEL_>
+// an atomic work queue (optionally in a caller-given order).  KEEP: the instantiation that also writes the barrier data
+// (NMPC_KEEP_BARRIER).  It is a kernel of its own because ptxas compiles a kernel with all its device functions as one unit:
+// any code added to ph_output of the production kernel changes the machine code of the per-iteration phases too.
+template <int N_, int NOBS_, int MODEL_, bool KEEP = false>
 __global__ void __launch_bounds__(32 * Lay<N_, NOBS_, MODEL_>::WPB, 1) nmpc_ipm_kernel(const __grid_constant__ SolveArgs A) {
   using L = Lay<N_, NOBS_, MODEL_>;
   const int lane = threadIdx.x & 31;
@@ -1816,7 +1840,7 @@ __global__ void __launch_bounds__(32 * Lay<N_, NOBS_, MODEL_>::WPB, 1) nmpc_ipm_
     const int b = A.order ? A.order[q] : q;
     // free-running closed loop: the steps of one instance follow each other here (the epilogue of step k has written p and the
     // warm start of step k + 1 in place), with no batch-wide barrier between the steps
-    for (int step = 0; step < A.run_steps; ++step) { solve_instance<L>(A, ric, cold, b, lane, step); __syncwarp(); }
+    for (int step = 0; step < A.run_steps; ++step) { solve_instance<L, KEEP>(A, ric, cold, b, lane, step); __syncwarp(); }
     __syncwarp();
     int fin = 0;
     if (lane == 0) { __threadfence(); fin = atomicAdd(A.done, 1); }      // this instance's outputs are visible before the count

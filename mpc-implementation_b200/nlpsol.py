@@ -60,19 +60,22 @@ def _spec_from(problem, opts: Optional[dict]) -> Dict[str, Any]:
 
 
 class _Sol(dict):
-    """Result dict of a solve.  sol['lam_p'] -- the sixth key of CasADi's result dict, which no reference script reads -- is
-    computed on first access (one small launch, nmpc_lam_p) instead of on every call."""
+    """Result dict of a solve.  The keys in `lazy` are computed on first access instead of on every call: sol['lam_p'] -- the
+    sixth key of CasADi's result dict, which no reference script reads -- (one small launch, nmpc_lam_p), and with want_jac
+    sol['jac_x_p'] / sol['jac_x_w'] (nmpc_sensitivity)."""
 
-    def __init__(self, items, lam_p_fn=None):
+    def __init__(self, items, lam_p_fn=None, lazy=None):
         super().__init__(items)
-        self._lam_p_fn = lam_p_fn
+        self._lazy = dict(lazy or {})
         if lam_p_fn is not None:
-            super().__setitem__("lam_p", None)
+            self._lazy["lam_p"] = lam_p_fn
+        for k in self._lazy:
+            super().__setitem__(k, None)
 
     def __getitem__(self, k):
-        if k == "lam_p" and self._lam_p_fn is not None:
-            super().__setitem__("lam_p", self._lam_p_fn())
-            self._lam_p_fn = None
+        fn = self._lazy.pop(k, None)
+        if fn is not None:
+            super().__setitem__(k, fn())
         return super().__getitem__(k)
 
     def get(self, k, default=None):
@@ -107,6 +110,7 @@ class Solver:
         self._warm = None
         self._sched = None
         self._held: Dict[str, Any] = {}      # tensors of the last call's per-call settings (_setting)
+        self._solves = 0                     # solve calls so far: the handle's kept barrier data belongs to the last one
         self._create(max_batch)
 
     # -- handle management ---------------------------------------------------------------------
@@ -169,7 +173,7 @@ class Solver:
     # -- the call --------------------------------------------------------------------------------
     def __call__(self, x0=None, p=None, lbx=None, ubx=None, lbg=None, ubg=None, obstacles=None,
                  want_g: bool = True, want_lam: bool = True, order=None, weights=None, target_traj=None,
-                 blocking: bool = True, lam_x0=None, lam_g0=None):
+                 blocking: bool = True, lam_x0=None, lam_g0=None, want_jac: bool = False):
         """lam_x0 [B, n_w], lam_g0 [B, n_g]: CasADi's multiplier guesses.  Like IPOPT they are ignored unless the solver was
         built with opts = {'ipopt': {'warm_start_init_point': 'yes', ...}} (no reference script does: non-reference fast mode,
         nmpc_set_warm_start); a NaN in lam_x0[b, 0] cold-starts instance b.
@@ -179,7 +183,12 @@ class Solver:
         in the reference).
         blocking=False (host buffers only): enqueue the copies and the solve and return at once; the outputs are
         page-locked arrays owned by this solver that become valid after `solver.wait()` and are reused by the next
-        call.  Pass page-locked inputs (torch pin_memory) for the copies to overlap."""
+        call.  Pass page-locked inputs (torch pin_memory) for the copies to overlap.
+        want_jac (blocking calls): the result also has sol['jac_x_p'] [B, n_w, n_p] = dx*/dp (CasADi's jac:x:p) and, for model 0,
+        sol['jac_x_w'] [B, n_w, 2] = dx*/d(w1, w2), computed on first access (nmpc_sensitivity; the solve keeps its barrier data,
+        NMPC_KEEP_BARRIER, and its results do not change).  They must be read before the next solve on this solver.  Rows of
+        instances that did not converge, or whose reduced Hessian is not positive definite (no sensitivity exists), are NaN.
+        The theta_t column is 0, and so are the target columns with target_traj.  want_jac implies want_lam."""
         if p is None:
             raise ValueError("solver: p is required")
         if any(v is None for v in (lbx, ubx, lbg, ubg)):
@@ -189,7 +198,8 @@ class Solver:
             dev = f"cuda:{self.device}"
             t = lambda a, n: None if a is None else torch.as_tensor(np.asarray(a, dtype=np.float64), device=dev).reshape(-1, n)
             out = self(x0=t(x0, self.n_w), p=t(p, self.n_p), lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg, obstacles=obstacles, want_g=want_g,
-                       want_lam=want_lam, order=order, weights=weights, target_traj=target_traj, lam_x0=lam_x0, lam_g0=lam_g0)
+                       want_lam=want_lam, order=order, weights=weights, target_traj=target_traj, lam_x0=lam_x0, lam_g0=lam_g0,
+                       want_jac=want_jac)
             torch.cuda.synchronize()
             self._stats = {k: v.cpu().numpy() for k, v in self._stats.items()}
             return {k: (None if v is None else v.cpu().numpy()) for k, v in out.items()}
@@ -201,9 +211,12 @@ class Solver:
                 self.set_warm_start(torch.as_tensor(lam_x0, dtype=torch.float64, device=p.device).reshape(B, self.n_w),
                                     torch.as_tensor(lam_g0, dtype=torch.float64, device=p.device).reshape(B, self.n_g))
                 stack.callback(self.set_warm_start, None, None)
+            jac = (weights, target_traj) if want_jac else None
             if _is_cuda_tensor(p):
-                return self._call_device(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, order)
-            return self._call_host(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking)
+                return self._call_device(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, order, jac)
+            if jac is not None and not blocking:
+                raise ValueError("solver: want_jac needs a blocking call")
+            return self._call_host(x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking, jac)
 
     def wait(self):
         """Complete a blocking=False call (nmpc_synchronize)."""
@@ -308,8 +321,9 @@ class Solver:
         o, flags = self._obst(obstacles, B)
         return dev_bounds, torch.from_numpy(o).to(f"cuda:{self.device}"), flags
 
-    def _call_host(self, x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking=True):
+    def _call_host(self, x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, blocking=True, jac=None):
         L = _ffi.lib()
+        want_lam = want_lam or jac is not None
         single = np.asarray(p).ndim == 1 or (np.asarray(p).ndim == 2 and np.asarray(p).shape[1] == 1)
         p = self._host(p, self.n_p, "p")
         B = p.shape[0]
@@ -329,7 +343,8 @@ class Solver:
         fn = L.nmpc_solve_host if blocking else L.nmpc_solve_host_async
         if not blocking:
             self._keep = (p, x0, lbx, ubx, lbg, ubg, obs)      # inputs stay alive until wait()
-        _ffi.check(fn(self._h, B, ptr(p), ptr(x0), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags,
+        self._solves += 1
+        _ffi.check(fn(self._h, B, ptr(p), ptr(x0), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags | (_ffi.NMPC_KEEP_BARRIER if jac else 0),
                       ptr(x), ptr(f), ptr(g), ptr(lam_x), ptr(lam_g), ptr(status), ptr(iters)),
                    "nmpc_solve_host")
         self._stats = dict(return_status=status, iter_count=iters)      # success is derived in stats(): valid after wait()
@@ -345,10 +360,12 @@ class Solver:
         out = dict(x=x, f=f, g=g, lam_x=lam_x, lam_g=lam_g)
         if single:
             out = {k: (v[0] if v is not None else None) for k, v in out.items()}
-        return _Sol(out, lam_p_host if (want_lam and blocking) else None)
+        lazy = self._jac_keys(B, single, True, x, p, lam_g, obs, flags, status, *jac) if jac is not None else None
+        return _Sol(out, lam_p_host if (want_lam and blocking) else None, lazy)
 
-    def _call_device(self, x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, order=None):
+    def _call_device(self, x0, p, lbx, ubx, lbg, ubg, obstacles, want_g, want_lam, order=None, jac=None):
         L = _ffi.lib()
+        want_lam = want_lam or jac is not None
         dev = p.device
         single = p.dim() == 1
         p = p.to(torch.float64).reshape(-1, self.n_p).contiguous()
@@ -369,7 +386,8 @@ class Solver:
             if order.numel() != B:
                 raise ValueError("solver: order must be a permutation of range(B)")
             _ffi.check(L.nmpc_set_order(self._h, order.data_ptr()), "nmpc_set_order")
-        _ffi.check(L.nmpc_solve(self._h, B, ptr(p), ptr(x0), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags,
+        self._solves += 1
+        _ffi.check(L.nmpc_solve(self._h, B, ptr(p), ptr(x0), ptr(lbx), ptr(ubx), ptr(lbg), ptr(ubg), ptr(obs), flags | (_ffi.NMPC_KEEP_BARRIER if jac else 0),
                                 ptr(x), ptr(f), ptr(g), ptr(lam_x), ptr(lam_g), ptr(status), ptr(iters), stream),
                    "nmpc_solve")
         def lam_p_dev():      # CasADi's result dict also carries lam_p (nobody in the reference reads it): on first access
@@ -383,7 +401,44 @@ class Solver:
         out = dict(x=x, f=f, g=g, lam_x=lam_x, lam_g=lam_g)
         if single:
             out = {k: (v[0] if v is not None else None) for k, v in out.items()}
-        return _Sol(out, lam_p_dev if want_lam else None)
+        lazy = self._jac_keys(B, single, False, x, p, lam_g, obs, flags, status, *jac) if jac is not None else None
+        return _Sol(out, lam_p_dev if want_lam else None, lazy)
+
+    def _jac_keys(self, B, single, host, x, p, lam_g, obs, flags, status, weights, target_traj):
+        """The lazy result keys jac_x_p (and jac_x_w for model 0) of the solve just launched: one nmpc_sensitivity launch on
+        first access of either, with the solve's own weights / target trajectory.  NaN rows where the solve did not converge or
+        no sensitivity exists (sens_status 1).  host: numpy inputs, numpy results."""
+        L = _ffi.lib()
+        solve_no, memo = self._solves, {}
+
+        def compute():
+            if not memo:
+                if self._solves != solve_no:
+                    raise RuntimeError("solver: jac_x_p / jac_x_w must be read before the next solve on this solver "
+                                       "(the sensitivity needs that solve's barrier data, which the next solve replaces)")
+                dev = torch.device(f"cuda:{self.device}")
+                up = lambda a: a if _is_cuda_tensor(a) else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+                xd, pd, ld, od, sd = up(x), up(p), up(lam_g), up(obs), up(status)
+                jp = torch.empty((B, self.n_w, self.n_p), dtype=torch.float64, device=dev)
+                jw = None if self.model else torch.empty((B, self.n_w, 2), dtype=torch.float64, device=dev)
+                ss = torch.empty(B, dtype=torch.int32, device=dev)
+                ptr = lambda t: None if t is None else t.data_ptr()
+                with torch.cuda.device(dev), self._settings(B, weights, target_traj):
+                    _ffi.check(L.nmpc_sensitivity(self._h, B, ptr(xd), ptr(pd), ptr(ld), ptr(od) if od.numel() else None, flags,
+                                                  ptr(jp), ptr(jw), ptr(ss), torch.cuda.current_stream(dev).cuda_stream),
+                               "nmpc_sensitivity")
+                bad = (sd != 0) | (ss != 0)
+                for t in (jp, jw):
+                    if t is not None:
+                        t[bad] = float("nan")
+                for k, t in (("jac_x_p", jp), ("jac_x_w", jw)):
+                    if t is not None and host:
+                        t = t.cpu().numpy()
+                    memo[k] = t[0] if (single and t is not None) else t
+            return memo
+
+        keys = ("jac_x_p",) if self.model else ("jac_x_p", "jac_x_w")
+        return {k: (lambda k=k: compute()[k]) for k in keys}
 
     def stats(self) -> Dict[str, Any]:
         """Per-instance outcome of the last call (CasADi: solver.stats()); after a blocking=False call, valid once
@@ -469,6 +524,7 @@ class Solver:
         x = torch.empty((B, self.n_w), dtype=torch.float64, device=p.device) if want_x else None
         f = torch.empty(B, dtype=torch.float64, device=p.device)
         ptr = lambda t: None if t is None else t.data_ptr()
+        self._solves += 1
         with self._settings(B, weights, target_traj, obstacles, obstacle_vel):
             _ffi.check(getattr(_ffi.lib(), entry)(self._h, B, *lead, ptr(p), ptr(u_warm), *map(ptr, bounds), ptr(obs), flags,
                                                   ptr(target_vw), ptr(x), ptr(f), ptr(fov_centre), ptr(err_accum), *map(ptr, logs),
@@ -528,6 +584,28 @@ class Solver:
                                target_vw.data_ptr(), None if fov_centre is None else fov_centre.data_ptr(),
                                None if err_accum is None else err_accum.data_ptr(), stream),
                    "nmpc_step")
+
+
+if torch is not None:
+    class SolveFunction(torch.autograd.Function):
+        """x* = solver(p=p, weights=weights, **kw)['x'] as a differentiable torch operation: SolveFunction.apply(solver, p, weights, kw)
+        with p [B, n_p] and weights [B, 2] (or None: the solver's own) CUDA float64 tensors and kw the other keywords of the call.
+        backward returns grad_p = jac_x_p^T grad_x and grad_weights = jac_x_w^T grad_x (want_jac; computed in the forward pass when
+        a gradient is needed).  Instances that did not converge, or have no sensitivity, have NaN rows and so NaN gradients."""
+
+        @staticmethod
+        def forward(ctx, solver, p, weights, kw):
+            need = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+            sol = solver(p=p, weights=weights, want_jac=need, **kw)
+            ctx.jac = (sol["jac_x_p"], sol.get("jac_x_w") if weights is not None else None) if need else (None, None)
+            return sol["x"]
+
+        @staticmethod
+        def backward(ctx, grad_x):
+            jp, jw = ctx.jac
+            gp = torch.einsum("...wp,...w->...p", jp, grad_x) if ctx.needs_input_grad[1] else None
+            gw = torch.einsum("...wk,...w->...k", jw, grad_x) if (ctx.needs_input_grad[2] and jw is not None) else None
+            return None, gp, gw, None
 
 
 def nlpsol(name: str, plugin: str, problem, opts: Optional[dict] = None, device: int = 0, max_batch: int = 1,
