@@ -175,6 +175,13 @@ int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, 
  * for the keeping solve, and the next solve on the handle waits for the launch (they share the handle's Riccati scratch). */
 int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g, const double* obst,
                      uint32_t flags, double* dx_dp, double* dx_dw, int32_t* sens_status, void* cuda_stream);
+/* The obstacle columns of the same sensitivity: dx_dobst [B][n_w][n_obs][3] = dx/d(cx_j, cy_j, r_j) of every obstacle row j,
+ * r_j = r_uav + r_obs as in the obstacle table.  The other arguments, the conditions and the stream ordering are those of
+ * nmpc_sensitivity: obst / flags must be the positions the solve used (one shared table or NMPC_OBS_PER_INSTANCE), and with a
+ * shared table each instance's columns are its own x* with respect to the shared entries.  sens_status as for nmpc_sensitivity
+ * (the same factorisation: the same value).  Also refused for a problem without obstacle rows (n_obs = 0). */
+int nmpc_sensitivity_obstacles(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g,
+                               const double* obst, uint32_t flags, double* dx_dobst, int32_t* sens_status, void* cuda_stream);
 /* The barrier data nmpc_sensitivity uses: sig_x [B][n_w], sig_g [B][n_g] (device pointers, either may be NULL) <- the Sigma_x and
  * Sigma_g kept by the last solve, B its batch size.  Lets a caller check the sensitivity system or form other right-hand sides.
  * Refused when the last solve did not keep them.  (An addition to the sensitivity call: the tests build the sensitivity system

@@ -43,7 +43,7 @@ class NmpcStats(C.Structure):
                 ("trial_passes", C.c_int64)]
 
 
-EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_sensitivity", "nmpc_barrier_data", "nmpc_step",
+EXPORTS = ["nmpc_create", "nmpc_destroy", "nmpc_solve", "nmpc_solve_host", "nmpc_solve_host_async", "nmpc_synchronize", "nmpc_query", "nmpc_solve_and_step", "nmpc_run_closed_loop", "nmpc_eval", "nmpc_lam_p", "nmpc_sensitivity", "nmpc_sensitivity_obstacles", "nmpc_barrier_data", "nmpc_step",
            "nmpc_get_stats", "nmpc_set_debug_log", "nmpc_set_order", "nmpc_set_weights", "nmpc_set_target_trajectory", "nmpc_set_obstacle_motion", "nmpc_set_schedule", "nmpc_set_warm_start", "nmpc_measure_fp64_peak", "nmpc_n_w", "nmpc_n_g", "nmpc_n_p",
            "nmpc_last_error", "nmpc_version"]
 
@@ -83,6 +83,8 @@ def lib():
     if hasattr(L, "nmpc_sensitivity"):
         L.nmpc_sensitivity.argtypes = [vp, C.c_int32, vp, vp, vp, vp, C.c_uint32, vp, vp, vp, vp]
         L.nmpc_barrier_data.argtypes = [vp, vp, vp, vp]
+    if hasattr(L, "nmpc_sensitivity_obstacles"):
+        L.nmpc_sensitivity_obstacles.argtypes = [vp, C.c_int32, vp, vp, vp, vp, C.c_uint32, vp, vp, vp]
     L.nmpc_get_stats.argtypes = [vp, C.POINTER(NmpcStats)]
     L.nmpc_set_debug_log.argtypes = [vp, vp, C.c_int32]
     L.nmpc_set_order.argtypes = [vp, vp]

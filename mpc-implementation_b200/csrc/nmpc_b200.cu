@@ -281,10 +281,11 @@ struct nmpc_handle {
 // The refusals several entry points share, each naming `fn`, the public function the caller called.  Those in `which` are
 // checked in this order; an entry point that makes them at different places of its own order calls this once per place.
 enum : unsigned { NULL_HANDLE = 1u, NO_OBSTACLES = 2u, PREDICT_WITHOUT_VW = 4u, PREDICT_WITH_TRAJECTORY = 8u, KEEP_WITHOUT_OUTPUTS = 16u,
-                  NOT_KEPT = 32u, KEPT_OTHER_B = 64u, WEIGHTS_OF_MODEL_1 = 128u };
+                  NOT_KEPT = 32u, KEPT_OTHER_B = 64u, WEIGHTS_OF_MODEL_1 = 128u, NO_OBSTACLE_ROWS = 256u };
 static int refused(const nmpc_handle* h, const char* fn, unsigned which, const double* obst = nullptr, uint32_t flags = 0, int32_t B = 0,
                    const double* dx_dw = nullptr) {
   if ((which & NULL_HANDLE) && !h) return fail(std::string(fn) + ": null handle");
+  if ((which & NO_OBSTACLE_ROWS) && h->pr.n_obs == 0) return fail(std::string(fn) + ": this problem has no obstacle rows (n_obs = 0)");
   if ((which & NO_OBSTACLES) && h->pr.n_obs > 0 && !obst) return fail(std::string(fn) + ": obstacle table required");
   if ((which & PREDICT_WITHOUT_VW) && (flags & NMPC_PREDICT_TARGET))
     return fail(std::string(fn) + ": NMPC_PREDICT_TARGET needs the target's (v, omega) of the step: use nmpc_solve_and_step or nmpc_run_closed_loop");
@@ -634,14 +635,15 @@ int nmpc_lam_p(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, 
   return launch_eval(h, "nmpc_lam_p", A, flags, !x_sol || !p || !lam_g || !lam_p, cuda_stream);
 }
 
-int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g, const double* obst,
-                     uint32_t flags, double* dx_dp, double* dx_dw, int32_t* sens_status, void* cuda_stream) {
-  const char* fn = "nmpc_sensitivity";
+// One launch of the sensitivity kernel for the entry point `fn`: the p and weight columns (dx_dp, required, and dx_dw) or,
+// with `obstacles`, the obstacle columns (dx_do, required).
+static int launch_sens(nmpc_handle* h, const char* fn, bool obstacles, int32_t B, const double* x_sol, const double* p, const double* lam_g,
+                       const double* obst, uint32_t flags, double* dx_dp, double* dx_dw, double* dx_do, int32_t* sens_status, void* cuda_stream) {
   const std::string f(fn);
-  if (refused(h, fn, NULL_HANDLE)) return 1;
+  if (refused(h, fn, NULL_HANDLE | (obstacles ? NO_OBSTACLE_ROWS : 0u))) return 1;
   if (B <= 0) return 0;
   if (refused(h, fn, NOT_KEPT | KEPT_OTHER_B | WEIGHTS_OF_MODEL_1 | PREDICT_WITHOUT_VW, nullptr, flags, B, dx_dw)) return 1;
-  if (!x_sol || !p || !lam_g || !dx_dp) return fail(f + ": null required pointer");
+  if (!x_sol || !p || !lam_g || !(obstacles ? dx_do : dx_dp)) return fail(f + ": null required pointer");
   if (refused(h, fn, NO_OBSTACLES, obst)) return 1;
   CK(cudaSetDevice(h->device));
   // x_sol enters as the start point x0 (ph_load puts it where the solve keeps its iterate) and as x
@@ -651,7 +653,7 @@ int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const doubl
   A.weights = h->weights; A.tgt = h->tgt;
   A.sig_x = h->d_sigx; A.sig_g = h->d_sigg;
   A.ric = h->d_ric; A.ric_stride = h->ric_stride; A.ricmap = h->d_ricmap;
-  A.dx_dp = dx_dp; A.dx_dw = dx_dw; A.sens_status = sens_status;
+  A.dx_dp = dx_dp; A.dx_dw = dx_dw; A.sens_status = sens_status; A.dx_do = dx_do;
   const cudaStream_t s = (cudaStream_t)cuda_stream;
   if (h->keep_stream != s) CK(cudaStreamWaitEvent(s, h->ev_keep, 0));      // the kept Sigmas are complete
   const int slots = h->max_blocks * h->warps_per_block;      // the Riccati scratch holds one slot per resident warp of the solve
@@ -660,6 +662,16 @@ int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const doubl
   h->sens_pending = 1; h->sens_stream = s;
   h->last_stream = s; h->launches = 1;
   return 0;
+}
+
+int nmpc_sensitivity(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g, const double* obst,
+                     uint32_t flags, double* dx_dp, double* dx_dw, int32_t* sens_status, void* cuda_stream) {
+  return launch_sens(h, "nmpc_sensitivity", false, B, x_sol, p, lam_g, obst, flags, dx_dp, dx_dw, nullptr, sens_status, cuda_stream);
+}
+
+int nmpc_sensitivity_obstacles(nmpc_handle* h, int32_t B, const double* x_sol, const double* p, const double* lam_g,
+                               const double* obst, uint32_t flags, double* dx_dobst, int32_t* sens_status, void* cuda_stream) {
+  return launch_sens(h, "nmpc_sensitivity_obstacles", true, B, x_sol, p, lam_g, obst, flags, nullptr, nullptr, dx_dobst, sens_status, cuda_stream);
 }
 
 int nmpc_barrier_data(nmpc_handle* h, double* sig_x, double* sig_g, void* cuda_stream) {

@@ -1,4 +1,5 @@
-// nmpc_sens.cuh -- solution sensitivities of converged solves (nmpc_sensitivity): dw*/dp and dw*/d(w1, w2).
+// nmpc_sens.cuh -- solution sensitivities of converged solves (nmpc_sensitivity, nmpc_sensitivity_obstacles): dw*/dp,
+// dw*/d(w1, w2) and dw*/d(cx, cy, r) of every obstacle.
 //
 // At the final iterate of a solve that kept its barrier data (NMPC_KEEP_BARRIER: Sigma_x, Sigma_g from ph_output) the
 // sensitivity is the implicit-function derivative of the barrier KKT system at delta_w = 0 (DESIGN.md section 1):
@@ -10,6 +11,9 @@
 //   target columns   linear terms -d2 l_k / dX d(x, y) of stages 1..N-1 (the cost depends on (x - x_t, y - y_t) only), dx_0 = 0;
 //                    exactly 0 with a per-stage target trajectory, as lam_p; theta_t never enters the NLP: exactly 0
 //   weight columns   linear terms grad_X dist_k and grad_X fov_k of each stage cost (model 0)
+//   obstacle columns linear terms y d(grad_X g)/dth + J^T Sigma_g dg/dth of the obstacle's row g = r - ||(x, y) - c|| on stages
+//                    1..N (the terminal stage included: its rows depend on w), dx_0 = 0
+// Each family runs only when its output is given; all share the one factorisation.
 // A non-positive pivot means the reduced Hessian is not positive definite at delta_w = 0 and the sensitivity is undefined:
 // NaN columns and sens_status 1.
 #pragma once
@@ -107,10 +111,12 @@ __device__ __noinline__ void sens_instance(const SolveArgs& A, double* ric, int 
   const bool ok = riccati_factor<L>(T, ric, A.ricmap, 0.0, 0.0, lane);
   __syncwarp();
   if (lane == 0 && A.sens_status) A.sens_status[b] = ok ? 0 : 1;
-  const int ncol = NPA + ((L::MODEL || !A.dx_dw) ? 0 : 2);
+  // column j: p for j < NPA, (w1, w2) for j < NPA + 2, then (cx, cy, r) of each obstacle; a family runs when its output is given
+  constexpr int NO = 3 * L::NOBS, JO = NPA + 2;
   const double2 tg = stage_target<L>(A, lane);
 #pragma unroll 1
-  for (int j = 0; j < ncol; ++j) {
+  for (int j = 0; j < JO + NO; ++j) {
+    if (!(j < NPA ? A.dx_dp : (j < JO ? (L::MODEL ? nullptr : A.dx_dw) : A.dx_do))) continue;
     const bool zero = j == NPA - 1 || (j >= NXP && j < NPA && A.tgt != nullptr);
     if (ok && !zero) {
       if (j < NXP) {
@@ -121,7 +127,7 @@ __device__ __noinline__ void sens_instance(const SolveArgs& A, double* ric, int 
         double q[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) q[i] = 0.0;
-        if (hasu && lane >= 1) {
+        if (hasu && lane >= 1 && j < JO) {
           if (j < NPA) {
             const int c = j - NXP;      // d/dx_t = -d/dx, d/dy_t = -d/dy
 #pragma unroll
@@ -131,6 +137,19 @@ __device__ __noinline__ void sens_instance(const SolveArgs& A, double* ric, int 
             stage_cost_d2(with_weights(pr, j == NPA ? 1.0 : 0.0, j == NPA ? 0.0 : 1.0), st.X, tg.x, tg.y, g1, H1);
 #pragma unroll
             for (int v = 0; v < 6; ++v) q[cost_state(v)] = g1[v];
+          }
+        }
+        if (act && lane >= 1 && j >= JO) {      // row g = r - D of obstacle jn on stages 1..N (the terminal one included)
+          const int jn = (j - JO) / 3, t = j - JO - 3 * jn;
+          double nx, ny, iD;
+          obs_value<L>(st.X, jn, nx, ny, iD);
+          const size_t ro = (size_t)b * R * S + lane * R + L::NB + jn;
+          const double w = A.sig_g[ro], y = A.lam_g[ro];
+          if (t == 2) { q[0] = -w * nx; q[1] = -w * ny; }     // J^T Sigma_g dg/dr = -Sigma_g n
+          else {      // y d(-n)/dc_t = y (e_t - n_t n) / D,  J^T Sigma_g dg/dc_t = -Sigma_g n_t n
+            const double m = t ? ny : nx, c = y * iD;
+            q[0] = c * ((t ? 0.0 : 1.0) - m * nx) - w * m * nx;
+            q[1] = c * ((t ? 1.0 : 0.0) - m * ny) - w * m * ny;
           }
         }
         if (act) {
@@ -143,8 +162,9 @@ __device__ __noinline__ void sens_instance(const SolveArgs& A, double* ric, int 
       }
     }
     if (hasu) {
-      double* col = j < NPA ? A.dx_dp + (size_t)b * nw * NPA + j : A.dx_dw + (size_t)b * nw * 2 + (j - NPA);
-      const int ld = j < NPA ? NPA : 2;
+      double* col = j < NPA ? A.dx_dp + (size_t)b * nw * NPA + j
+                            : (j < JO ? A.dx_dw + (size_t)b * nw * 2 + (j - NPA) : A.dx_do + (size_t)b * nw * NO + (j - JO));
+      const int ld = j < NPA ? NPA : (j < JO ? 2 : NO);
 #pragma unroll
       for (int i = 0; i < NUA; ++i) col[(size_t)(NUA * lane + i) * ld] = !ok ? CUDART_NAN : (zero ? 0.0 : LV(LV_DU + i));
     }

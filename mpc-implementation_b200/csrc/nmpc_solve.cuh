@@ -94,6 +94,7 @@ struct SolveArgs {
   // sig_g [B][n_g] the same for the row slacks.  The sensitivity kernel (nmpc_sens.cuh) reads them, with x / lam_g as inputs.
   double *sig_x, *sig_g;
   double *dx_dp, *dx_dw; int32_t* sens_status;     // nmpc_sensitivity: [B][n_w][n_p], [B][n_w][2] (may be NULL), [B]
+  double* dx_do;                     // nmpc_sensitivity_obstacles: [B][n_w][3 n_obs], column 3 j + (0, 1, 2) = (cx_j, cy_j, r_j)
 };
 constexpr int NSTAT = 9;
 constexpr int DBG_COLS = 10;

@@ -186,7 +186,9 @@ class Solver:
         call.  Pass page-locked inputs (torch pin_memory) for the copies to overlap.
         want_jac (blocking calls): the result also has sol['jac_x_p'] [B, n_w, n_p] = dx*/dp (CasADi's jac:x:p) and, for model 0,
         sol['jac_x_w'] [B, n_w, 2] = dx*/d(w1, w2), computed on first access (nmpc_sensitivity; the solve keeps its barrier data,
-        NMPC_KEEP_BARRIER, and its results do not change).  They must be read before the next solve on this solver.  Rows of
+        NMPC_KEEP_BARRIER, and its results do not change).  With obstacle rows there is also sol['jac_x_obst'] [B, n_w, n_obs, 3]
+        = dx*/d(cx, cy, r_uav + r_obs) of each obstacle of the call's table (shared or per instance), computed by its own launch on
+        first access (nmpc_sensitivity_obstacles).  They must be read before the next solve on this solver.  Rows of
         instances that did not converge, or whose reduced Hessian is not positive definite (no sensitivity exists), are NaN.
         The theta_t column is 0, and so are the target columns with target_traj.  want_jac implies want_lam."""
         if p is None:
@@ -405,40 +407,48 @@ class Solver:
         return _Sol(out, lam_p_dev if want_lam else None, lazy)
 
     def _jac_keys(self, B, single, host, x, p, lam_g, obs, flags, status, weights, target_traj):
-        """The lazy result keys jac_x_p (and jac_x_w for model 0) of the solve just launched: one nmpc_sensitivity launch on
-        first access of either, with the solve's own weights / target trajectory.  NaN rows where the solve did not converge or
-        no sensitivity exists (sens_status 1).  host: numpy inputs, numpy results."""
+        """The lazy result keys of the solve just launched, with the solve's own weights / target trajectory / obstacles: jac_x_p
+        (and jac_x_w for model 0) from one nmpc_sensitivity launch on first access of either, and with obstacle rows jac_x_obst
+        from its own nmpc_sensitivity_obstacles launch.  NaN rows where the solve did not converge or no sensitivity exists
+        (sens_status 1).  host: numpy inputs, numpy results."""
         L = _ffi.lib()
-        solve_no, memo = self._solves, {}
+        solve_no = self._solves
 
-        def compute():
-            if not memo:
-                if self._solves != solve_no:
-                    raise RuntimeError("solver: jac_x_p / jac_x_w must be read before the next solve on this solver "
-                                       "(the sensitivity needs that solve's barrier data, which the next solve replaces)")
-                dev = torch.device(f"cuda:{self.device}")
-                up = lambda a: a if _is_cuda_tensor(a) else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
-                xd, pd, ld, od, sd = up(x), up(p), up(lam_g), up(obs), up(status)
-                jp = torch.empty((B, self.n_w, self.n_p), dtype=torch.float64, device=dev)
-                jw = None if self.model else torch.empty((B, self.n_w, 2), dtype=torch.float64, device=dev)
-                ss = torch.empty(B, dtype=torch.int32, device=dev)
-                ptr = lambda t: None if t is None else t.data_ptr()
-                with torch.cuda.device(dev), self._settings(B, weights, target_traj):
-                    _ffi.check(L.nmpc_sensitivity(self._h, B, ptr(xd), ptr(pd), ptr(ld), ptr(od) if od.numel() else None, flags,
-                                                  ptr(jp), ptr(jw), ptr(ss), torch.cuda.current_stream(dev).cuda_stream),
-                               "nmpc_sensitivity")
-                bad = (sd != 0) | (ss != 0)
-                for t in (jp, jw):
-                    if t is not None:
+        def family(fn, shapes):
+            """shapes: key -> shape of each output pointer of `fn`, in order (None: pass NULL, no key)."""
+            memo = {}
+
+            def compute():
+                if not memo:
+                    if self._solves != solve_no:
+                        raise RuntimeError(f"solver: {' / '.join(k for k, s in shapes.items() if s)} must be read before the next "
+                                           "solve on this solver (the sensitivity needs that solve's barrier data, which the next "
+                                           "solve replaces)")
+                    dev = torch.device(f"cuda:{self.device}")
+                    up = lambda a: a if _is_cuda_tensor(a) else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+                    xd, pd, ld, od, sd = up(x), up(p), up(lam_g), up(obs), up(status)
+                    outs = {k: None if s is None else torch.empty(s, dtype=torch.float64, device=dev) for k, s in shapes.items()}
+                    ss = torch.empty(B, dtype=torch.int32, device=dev)
+                    ptr = lambda t: None if t is None else t.data_ptr()
+                    with torch.cuda.device(dev), self._settings(B, weights, target_traj):
+                        _ffi.check(getattr(L, fn)(self._h, B, ptr(xd), ptr(pd), ptr(ld), ptr(od) if od.numel() else None, flags,
+                                                  *(ptr(t) for t in outs.values()), ptr(ss), torch.cuda.current_stream(dev).cuda_stream),
+                                   fn)
+                    bad = (sd != 0) | (ss != 0)
+                    for k, t in outs.items():
+                        if t is None:
+                            continue
                         t[bad] = float("nan")
-                for k, t in (("jac_x_p", jp), ("jac_x_w", jw)):
-                    if t is not None and host:
-                        t = t.cpu().numpy()
-                    memo[k] = t[0] if (single and t is not None) else t
-            return memo
+                        if host:
+                            t = t.cpu().numpy()
+                        memo[k] = t[0] if single else t
+                return memo
+            return {k: (lambda k=k: compute()[k]) for k, s in shapes.items() if s}
 
-        keys = ("jac_x_p",) if self.model else ("jac_x_p", "jac_x_w")
-        return {k: (lambda k=k: compute()[k]) for k in keys}
+        keys = family("nmpc_sensitivity", {"jac_x_p": (B, self.n_w, self.n_p), "jac_x_w": None if self.model else (B, self.n_w, 2)})
+        if self.n_obs:
+            keys.update(family("nmpc_sensitivity_obstacles", {"jac_x_obst": (B, self.n_w, self.n_obs, 3)}))
+        return keys
 
     def stats(self) -> Dict[str, Any]:
         """Per-instance outcome of the last call (CasADi: solver.stats()); after a blocking=False call, valid once
@@ -591,13 +601,31 @@ if torch is not None:
         """x* = solver(p=p, weights=weights, **kw)['x'] as a differentiable torch operation: SolveFunction.apply(solver, p, weights, kw)
         with p [B, n_p] and weights [B, 2] (or None: the solver's own) CUDA float64 tensors and kw the other keywords of the call.
         backward returns grad_p = jac_x_p^T grad_x and grad_weights = jac_x_w^T grad_x (want_jac; computed in the forward pass when
-        a gradient is needed).  Instances that did not converge, or have no sensitivity, have NaN rows and so NaN gradients."""
+        a gradient is needed).  Instances that did not converge, or have no sensitivity, have NaN rows and so NaN gradients.
+
+        SolveFunction.apply(solver, p, weights, kw, obstacles) also differentiates with respect to the obstacle table, a CUDA
+        float64 tensor of (cx, cy, r_uav + r_obs) rows (then not in kw): grad_obstacles = jac_x_obst^T grad_x.
+          [B, n_obs, 3], one table per instance: per instance, NaN rows for instances without a sensitivity, as for p.
+          [n_obs, 3], shared by the batch: the sum over the instances of their contributions, where an instance whose grad_x row is
+            exactly zero contributes exactly zero, even with NaN columns -- so a non-converged instance left out of the loss does
+            not make the shared gradient NaN.  One that enters the loss with NaN columns still does."""
 
         @staticmethod
-        def forward(ctx, solver, p, weights, kw):
-            need = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-            sol = solver(p=p, weights=weights, want_jac=need, **kw)
-            ctx.jac = (sol["jac_x_p"], sol.get("jac_x_w") if weights is not None else None) if need else (None, None)
+        def forward(ctx, solver, p, weights, kw, obstacles=None):
+            if obstacles is not None:
+                if "obstacles" in kw:
+                    raise ValueError("SolveFunction: obstacles given both as an argument and in kw")
+                if not (_is_cuda_tensor(obstacles) and obstacles.dtype == torch.float64):
+                    raise ValueError("SolveFunction: obstacles must be a CUDA float64 tensor, [n_obs, 3] or [B, n_obs, 3]")
+                kw = dict(kw, obstacles=obstacles)
+            need_po = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+            need_o = len(ctx.needs_input_grad) > 4 and ctx.needs_input_grad[4]
+            sol = solver(p=p, weights=weights, want_jac=need_po or need_o, **kw)
+            ctx.jac = (sol["jac_x_p"], sol.get("jac_x_w") if weights is not None else None) if need_po else (None, None)
+            ctx.jac_o = sol["jac_x_obst"] if need_o else None
+            # the solver's shape rule: 3 n_obs entries are one table shared by the batch
+            ctx.shared = need_o and solver._obs_flag(obstacles.numel(), sol["x"].numel() // solver.n_w) == 0
+            ctx.obs_shape = None if obstacles is None else obstacles.shape
             return sol["x"]
 
         @staticmethod
@@ -605,7 +633,17 @@ if torch is not None:
             jp, jw = ctx.jac
             gp = torch.einsum("...wp,...w->...p", jp, grad_x) if ctx.needs_input_grad[1] else None
             gw = torch.einsum("...wk,...w->...k", jw, grad_x) if (ctx.needs_input_grad[2] and jw is not None) else None
-            return None, gp, gw, None
+            go = None
+            if ctx.jac_o is not None:
+                if ctx.shared:
+                    jo = ctx.jac_o.reshape(-1, *ctx.jac_o.shape[-3:])
+                    gx = grad_x.reshape(jo.shape[0], -1)
+                    used = (gx != 0).any(dim=1)      # instances outside the loss contribute exactly zero, NaN columns or not
+                    go = torch.einsum("bwoc,bw->oc", jo[used], gx[used])
+                else:
+                    go = torch.einsum("...woc,...w->...oc", ctx.jac_o, grad_x)
+                go = go.reshape(ctx.obs_shape)
+            return (None, gp, gw, None, go)[:len(ctx.needs_input_grad)]
 
 
 def nlpsol(name: str, plugin: str, problem, opts: Optional[dict] = None, device: int = 0, max_batch: int = 1,
